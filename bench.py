@@ -3,13 +3,17 @@
 (BASELINE.json configs[1]): per GPU a batch of 64 synthetic MV-TOD-shaped scenes, V=73 views of
 480x640, N=100k points, Q=21 objects, C=768, production flags of tools/preprocess_data.py:177-185.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
 
 One "step" = one pass of the hot path over one batch. `value` = scenes/s with inputs resident in
 HBM; `e2e` = the same metric through the reference-shaped call MultiviewFeatureFusion.fuse() with
 host numpy inputs (pinned staging + H2D + D2H inside the timed region). `--impl reference` times
 the CPU restatement of the reference's own torch/numpy path (oracle/fusion_ref.py; the reference is
-pure Python and /root/reference does not exist on the GPU box) on the host cores.
+pure Python and is not part of this repository) on the host cores.
+
+`--dump-outputs DIR` writes what the last timed step computed (rank 0) as DIR/<name>.npy, float32 or
+float64, under 64 MB in all; see dump_outputs(). The inputs are generated from fixed seeds, so two
+builds run with the same arguments can be compared output for output.
 """
 from __future__ import annotations
 
@@ -20,6 +24,7 @@ import subprocess
 import sys
 import threading
 import time
+import zlib
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
@@ -30,10 +35,18 @@ import torch  # noqa: E402
 WORKLOAD = "mvtod_object_fusion_sim_max_batch64_V73_N100k_Q21_C768"
 
 
+def positive_int(s):
+    v = int(s)
+    if v < 1:
+        raise argparse.ArgumentTypeError("must be >= 1")
+    return v
+
+
 def parse():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=10)
+    ap.add_argument("--steps", type=positive_int, default=10,
+                    help="timed steps of the headline, one-stream, full-output, uint8-map and e2e loops")
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--scenes", type=int, default=64, help="scenes per GPU per step")
@@ -49,6 +62,8 @@ def parse():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--no-extras", action="store_true", help="skip the supplementary configs 4/5 (pixel-level fusion, grounding)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the outputs of the last timed step as DIR/<name>.npy (rank 0)")
     return ap.parse_args()
 
 
@@ -193,7 +208,7 @@ def workload_config(args, world):
 
 def run_reference(args):
     """The reference's own CPU path (oracle/fusion_ref.py, the pinned restatement of utils/feature_fusion.py:272-343 -
-    the reference is pure Python and /root/reference does not travel) on rank 0's host cores: one scene of the
+    the reference is pure Python and is not part of this repository) on rank 0's host cores: one scene of the
     workload per step, in the fastest of the thread modes of cpu_modes()."""
     rank = int(os.environ.get("RANK", "0"))
     if rank != 0:
@@ -239,6 +254,54 @@ def algorithmic_bytes(b, mask_elem=1):
     wmean = b.total_rows * dim * fe + sum(q * v * 4 + q * dim * 4 for q, v in zip(b.n_queries, b.n_views))
     score_flops = 2 * b.total_rows * dim * max(b.n_queries)
     return {"project_visibility": vis, "seg_histogram": seg, "segmented_wmean": wmean, "view_score_flops": score_flops}
+
+
+def _fit(name, a, cap, dtype=np.float32):
+    """`a` (a CUDA tensor) as a host array of `dtype`: in full if it has at most `cap` elements, otherwise flattened and
+    sampled at sorted indices drawn from a generator seeded by the name and the size (the same for equal sizes)."""
+    flat = a.reshape(-1)
+    if flat.numel() > cap:
+        seed = (zlib.crc32(name.encode()), flat.numel())
+        idx = np.unique(np.random.default_rng(seed).integers(0, flat.numel(), size=cap))
+        a = flat[torch.from_numpy(idx).to(flat.device)]
+    return a.cpu().numpy().astype(dtype)
+
+
+def dump_outputs(out_dir, b, res, comp):
+    """The results of one step as a caller of the device-resident path receives them: fused object features (sum Q, C),
+    view weights (wobj layout), per-view status flags, the keep flag of every point, kept points per scene, and the
+    compacted (V, N') uint8 visibility masks as per-(scene, view) visible counts plus a seeded sample of their elements.
+    Counts and status flags are written as float64 (exact for any count). Each array is capped (_fit) so that all of them
+    stay under 64 MB whatever the batch size.
+    An object seen in no view has an all-NaN feature row, as in the reference; it is written as `object_seen` = 0 and a
+    row of zeros. Any other non-finite value is written as it is and reported on stderr."""
+    fused = res["fused"]
+    unseen = torch.isnan(fused).all(1)
+    fused = fused.masked_fill(unseen[:, None], 0.0)
+    _, kept_off, _, out_off, cmask, _ = comp
+    kept = kept_off.cpu().numpy()
+    out = out_off.cpu().numpy()
+    cmask = cmask[:int(out[-1])]
+    counts = [cmask[int(out[s]):int(out[s + 1])].view(v, int(kept[s + 1] - kept[s])).sum(1, dtype=torch.int64)
+              for s, v in enumerate(b.n_views)]
+    arrays = {
+        "fused_features": _fit("fused_features", fused, 1 << 21),
+        "object_seen": _fit("object_seen", ~unseen, 1 << 17),
+        "view_weights": _fit("view_weights", res["weight_obj"], 1 << 20),
+        "view_status": _fit("view_status", res["view_status"][:b.total_views], 1 << 17, np.float64),
+        "any_visible": _fit("any_visible", res["any_visible"], 1 << 23),
+        "kept_points_per_scene": np.diff(kept).astype(np.float64),
+        "visible_points_per_view": _fit("visible_points_per_view", torch.cat(counts), 1 << 17, np.float64),
+        "visibility_mask_sample": _fit("visibility_mask_sample", cmask, 1 << 21),
+    }
+    total = sum(a.nbytes for a in arrays.values())
+    assert total <= 64_000_000, total
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+    bad = {name: int((~np.isfinite(a)).sum()) for name, a in arrays.items() if not np.isfinite(a).all()}
+    if bad:
+        sys.stderr.write("bench.py: non-finite values in the dumped outputs (count per array): %s\n" % bad)
 
 
 def run_ours(args):
@@ -310,6 +373,8 @@ def run_ours(args):
     if world > 1:
         dist.barrier()
     clocks = sampler.stop() if rank == 0 else None
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, batch, res, comp)
     ms = torch.tensor([start.elapsed_time(end)], device=dev)
     if world > 1:
         dist.all_reduce(ms, op=dist.ReduceOp.MAX)
@@ -373,13 +438,13 @@ def run_ours(args):
             eng.profile = {}
             a0, a1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
             a0.record()
-            for _ in range(5):
+            for _ in range(args.steps):
                 keep_a = step()
             a1.record()
             torch.cuda.synchronize()
             pa = eng.profile_ms()
             roofline["one_stream"] = {
-                "ms_per_step": a0.elapsed_time(a1) / 5,
+                "ms_per_step": a0.elapsed_time(a1) / args.steps,
                 "kernels": {k: {"ms": pa[k], "gbs": alg[k] / (pa[k] * 1e-3) / 1e9, "frac": alg[k] / (pa[k] * 1e-3) / 1e9 / hbm_peak}
                             for k in ("project_visibility", "seg_histogram") if k in pa and pa[k] > 0}}
             del keep_a
@@ -530,7 +595,7 @@ def run_ours(args):
         torch.cuda.synchronize()
         if world > 1:
             dist.barrier()
-        n_e2e = max(2, min(args.steps, 10))
+        n_e2e = args.steps
         up0 = M._staging.bytes_uploaded
         t0 = time.perf_counter()
         for _ in range(n_e2e):
@@ -823,6 +888,8 @@ def other_configs(dev, eng):
 def main():
     args = parse()
     if args.impl == "reference":
+        if args.dump_outputs:
+            raise SystemExit("--dump-outputs writes the outputs of --impl ours")
         run_reference(args)
     else:
         if not torch.cuda.is_available():

@@ -47,16 +47,26 @@ def test_library_targets_sm100a_with_tensor_core_and_tma_instructions():
     assert "UBLKCP.S.G" in ring and "SYNCS.ARRIVE.TRANS64" in ring and "SYNCS.PHASECHK.TRANS64.TRYWAIT" in ring
 
 
+_NO_GPU_SCRIPT = r"""
+import sys
+sys.path.insert(0, {root!r})
+import numpy as np, pytest, torch
+assert not torch.cuda.is_available()
+from dropclip_b200.engine import FusionEngine
+from dropclip_b200.feature_fusion import MultiviewFeatureFusion
+with pytest.raises(RuntimeError):
+    FusionEngine("cuda")
+M = MultiviewFeatureFusion({{"fx": 1.0, "fy": 1.0, "cx": 0.0, "cy": 0.0}}, use_similarity=False, device="cpu")
+with pytest.raises(RuntimeError):
+    M.get_visibility_mask(np.zeros((3, 3)), [np.zeros((480, 640), np.float32)], [np.eye(4, dtype=np.float32)])
+"""
+
+
 def test_no_cpu_fallback_without_gpu():
-    if torch.cuda.is_available():
-        pytest.skip("GPU present")
-    from dropclip_b200.engine import FusionEngine
-    from dropclip_b200.feature_fusion import MultiviewFeatureFusion
-    with pytest.raises(RuntimeError):
-        FusionEngine("cuda")
-    M = MultiviewFeatureFusion({"fx": 1.0, "fy": 1.0, "cx": 0.0, "cy": 0.0}, use_similarity=False, device="cpu")
-    with pytest.raises(RuntimeError):
-        M.get_visibility_mask(np.zeros((3, 3)), [np.zeros((480, 640), np.float32)], [np.eye(4, dtype=np.float32)])
+    """Runs in a child process with every CUDA device hidden, so that it checks the same on a machine that has a GPU."""
+    r = subprocess.run([sys.executable, "-c", _NO_GPU_SCRIPT.format(root=ROOT)], env=dict(os.environ, CUDA_VISIBLE_DEVICES=""),
+                       capture_output=True, text=True, timeout=300)
+    assert r.returncode == 0, r.stdout + r.stderr
 
 
 def test_product_package_never_imports_the_oracle():

@@ -192,6 +192,41 @@ def test_sparse_quantize_restatement_properties():
         assert vl[j] == (labs[0] if labs.size == 1 else 0)
 
 
+def test_restatement_against_reference_golden():
+    """The live comparison below against the reference's stored values (tests/golden/live_restatement.npz): masks and
+    kept points bit for bit; features and weights to the fp32 GEMM's thread-count ulps, as in the other golden tests."""
+    from tests.make_golden_live import SCENE, restatement_scene, scene_digest
+    z = gio.load("live_restatement.npz")
+    sc = restatement_scene()
+    assert scene_digest(sc) == str(z["inputs_sha"]), "small_scene() no longer generates the stored inputs"
+    H, W = SCENE["height"], SCENE["width"]
+    K = fusion_ref.intrinsic_matrix(sc.intrinsic)
+    (of, ow, ov), (op, _, _) = fusion_ref.fuse_object_level(
+        sc.points, sc.colors, sc.labels, sc.depths, sc.seg_masks, sc.camera_poses, sc.mv_features,
+        sc.query_embeddings, K, H, W, return_obj=True)
+    assert op.shape[0] == int(z["n_kept"][0]) and np.array_equal(op, z["points"])
+    assert np.array_equal(ov.numpy(), gio.unpack(z["vis"], op.shape[0]))
+    np.testing.assert_allclose(ow.numpy(), z["weight"], rtol=1e-6, atol=0)
+    np.testing.assert_allclose(of.numpy(), z["feat"], rtol=1e-5, atol=1e-7, equal_nan=True)
+    cm = c_oracle.visibility_mask(sc.points, sc.depths, sc.camera_poses, K)
+    assert np.array_equal(cm, gio.unpack(z["vis_full"], sc.n_points))
+
+
+def test_c_visibility_with_fp64_poses_against_reference_golden():
+    """The C oracle on fp64 poses and on their fp32 roundings against the reference's masks for the same inputs
+    (tests/golden/live_fp64_poses.npz), bit for bit."""
+    from tests.make_golden_live import fp64_pose_digest
+    z = gio.load("live_fp64_poses.npz")
+    sc, poses64, pts = gio.fp64_pose_case()
+    assert fp64_pose_digest(sc, poses64, pts) == str(z["inputs_sha"]), "fp64_pose_case() no longer generates the stored inputs"
+    poses32 = [p.astype(np.float32) for p in poses64]
+    K = fusion_ref.intrinsic_matrix(sc.intrinsic)
+    ref64, ref32 = gio.unpack(z["vis64"], pts.shape[0]), gio.unpack(z["vis32"], pts.shape[0])
+    assert np.array_equal(c_oracle.visibility_mask(pts, sc.depths, poses64, K), ref64)
+    assert np.array_equal(c_oracle.visibility_mask(pts, sc.depths, poses32, K), ref32)
+    assert (ref64 != ref32).sum() > 100, "the case must distinguish fp64 poses from their fp32 roundings"
+
+
 @pytest.mark.needs_reference
 def test_restatement_against_live_reference():
     from dropclip_b200.scenes import small_scene

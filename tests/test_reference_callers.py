@@ -5,6 +5,8 @@ imports (`models.similarity`, `utils.misc`) after `dropclip_b200.install.install
 branches (center_crop / subsample_step / transform_coords, utils/projections.py:118-145) against outputs of the
 unmodified reference; (iv) sparse_collate (data/dataset_blender.py:450-461)."""
 import inspect
+import json
+import os
 import sys
 import types
 
@@ -17,6 +19,19 @@ from tests import golden_io as gio
 
 def _params(fn):
     return [(n, p.default, p.kind) for n, p in inspect.signature(fn).parameters.items()]
+
+
+def test_signatures_equal_the_reference_golden():
+    """The live comparison below against the reference's signatures stored in tests/golden/reference_signatures.json
+    (tests/make_golden_live.py): every mirrored callable, static or not, defaults included."""
+    from tests.make_golden_live import our_modules, signatures
+    want = json.load(open(os.path.join(gio.GOLDEN, "reference_signatures.json")))
+    got = json.loads(json.dumps(signatures(*our_modules(), ours=True)))  # tuples -> lists, as stored
+    assert sorted(got) == sorted(want)
+    for key in want:
+        assert got[key] == want[key], key
+    import dropclip_b200.similarity as oms
+    assert str(inspect.signature(oms.ClipSimilarity.__init__).parameters["device"].default) == "cuda"
 
 
 @pytest.mark.needs_reference
