@@ -44,7 +44,7 @@ def main():
                               "points_per_s": n / (ms * 1e-3), "useful_tflops": flops / (ms * 1e-3) / 1e12,
                               "issued_tflops": flops * terms / (ms * 1e-3) / 1e12, "alg_GBps": alg_bytes / (ms * 1e-3) / 1e9,
                               "frac_hbm": alg_bytes / (ms * 1e-3) / 1e9 / peaks.get("hbm_gbs", 6650.0),
-                              "frac_tensor_useful": flops / (ms * 1e-3) / 1e12 / peaks.get("bf16_tflops", 1590.0), "two_pass": bool(os.environ.get("DC_GROUND_TWO_PASS"))}))
+                              "frac_tensor_useful": flops / (ms * 1e-3) / 1e12 / peaks.get("bf16_tflops", 1590.0)}))
 
 if __name__ == "__main__":
     main()

@@ -1,5 +1,5 @@
-"""Headline step under the four combinations of {one stream, two streams} x {register-staged, bulk-copy ring}
-instance-histogram kernel. Checks that both histogram kernels return identical tables first.
+"""Headline step on one stream (register-staged instance-histogram kernel) and on two streams (bulk-copy ring kernel
+beside the visibility filter), alternated. Checks first that both histogram kernels return identical tables.
 
     python benchmarks/overlap_probe.py [scenes] [unique]
 """
@@ -20,15 +20,14 @@ uniq = [make_scene(1234 + i, n_views=73, n_points=100_000, n_objects=21, device=
 batch = batch_from_device([uniq[i % n_unique] for i in range(n_scenes)], dev, seg_dtype=torch.int64)
 torch.cuda.synchronize()
 
-os.environ["DC_SEG_MODE"] = "ldg"
+eng.overlap = False
 ref = [t.clone() for t in eng.seg_tables(batch)]
-os.environ["DC_SEG_MODE"] = "ring"
+eng.overlap = True
 got = eng.seg_tables(batch)
 torch.cuda.synchronize()
-os.environ.pop("DC_SEG_MODE")
 for name, a, b in zip(("counts", "outside", "row_object", "object_row", "status"), ref, got):
     assert torch.equal(a, b), f"ring histogram differs from the register-staged kernel: {name}"
-print("ring == ldg tables: ok")
+print("ring == register-staged tables: ok")
 
 
 def step():
@@ -39,16 +38,8 @@ def step():
 
 
 base = None
-configs = [(0, "", 0, "", 0), (1, "", 0, "", 0), (1, "ring", 3, 72, 12), (1, "ring", 3, 58, 12), (1, "ring", 4, 72, 8), (1, "ring", 2, 58, 16), (1, "ring", 2, 72, 16), (0, "", 0, "", 0), (1, "", 0, "", 0)]
-if len(sys.argv) > 3:
-    configs = [tuple(int(x) if x.lstrip("-").isdigit() else x for x in c.split(",")) for c in sys.argv[3:]]
-for overlap, mode, stages, carve, warps in configs:
-    eng.overlap = bool(overlap)
-    for key, val in (("DC_SEG_MODE", mode), ("DC_SEG_STAGES", stages), ("DC_CARVEOUT_PCT", carve), ("DC_SEG_WARPS", warps)):
-        if val in ("", 0):
-            os.environ.pop(key, None)  # library defaults
-        else:
-            os.environ[key] = str(val)
+for overlap in (False, True, False, True):
+    eng.overlap = overlap
     keep = None
     for _ in range(3):
         keep = step()
@@ -70,5 +61,5 @@ for overlap, mode, stages, carve, warps in configs:
     if base is None:
         base = sig
     assert sig == base, (sig, base)
-    print(f"overlap={overlap} seg={mode}{stages or ''} warps={warps} carve={carve}: {a.elapsed_time(b) / 10:.3f} ms/step (host enqueue {host_ms:.2f} ms/step)  "
+    print(f"overlap={overlap}: {a.elapsed_time(b) / 10:.3f} ms/step (host enqueue {host_ms:.2f} ms/step)  "
           + "  ".join(f"{k}={v:.3f}" for k, v in prof.items()), flush=True)

@@ -3,7 +3,6 @@
 // Reference: utils/feature_fusion.py:311-313 (feat_v_norm @ query.T), models/similarity.py:28-101
 // (vis_feats @ text.T, paired softmax, min-max, threshold), engine/distil.py:244-246.
 #include <algorithm>
-#include <stdlib.h>
 #include <mutex>
 
 #include "gemm.cuh"
@@ -741,19 +740,6 @@ int launch_bn(int bn, const void* a_hi, const void* a_lo, int64_t a_rows, const 
 
 int pick_bn(int n) { return n <= 32 ? 32 : n <= 64 ? 64 : n <= 128 ? 128 : 256; }
 
-// grounding GEMM with the in-place fp16 row normalisation of A fused in (p.norm_rows): k = 256 * chunks
-template <int kNormChunks>
-int launch_bn_norm(int bn, const void* a_hi, int64_t a_rows, const void* b_hi, const void* b_lo, int64_t b_rows,
-                   const Params& p, const EpiGround& epi, int max_tiles, cudaStream_t st) {
-  switch (bn) {
-    case 32: return dc::gemm::launch<32, EpiGround, kNormChunks>(a_hi, nullptr, a_rows, b_hi, b_lo, b_rows, p, epi, max_tiles, st);
-    case 64: return dc::gemm::launch<64, EpiGround, kNormChunks>(a_hi, nullptr, a_rows, b_hi, b_lo, b_rows, p, epi, max_tiles, st);
-    case 128: return dc::gemm::launch<128, EpiGround, kNormChunks>(a_hi, nullptr, a_rows, b_hi, b_lo, b_rows, p, epi, max_tiles, st);
-    case 256: return dc::gemm::launch<256, EpiGround, kNormChunks>(a_hi, nullptr, a_rows, b_hi, b_lo, b_rows, p, epi, max_tiles, st);
-  }
-  return dc::fail(DC_ERR_UNSUPPORTED, "unsupported GEMM N tile %d", bn);
-}
-
 size_t align_up(size_t x, size_t a) { return (x + a - 1) / a * a; }
 
 struct ScoreWorkspace {
@@ -907,14 +893,12 @@ int dc_ground(const void* x_hi, const void* x_lo, int64_t n_points, const void* 
   DC_CHECK_ARG(n_points < (1ll << 31), "dc_ground: too many points for one call");
   DC_CHECK_ARG(!normalize_fp16_rows || !x_lo, "dc_ground: normalize_fp16_rows is for fp16 features (x_lo must be NULL)");
   if (n_points <= 0) return DC_OK;
-  // fp16 features to be normalised in place (models/similarity.py:77): fused into the first GEMM launch when the row
-  // width allows (four extra warps normalise the rows of the coming tiles while the tensor pipe works, so the features
-  // cross HBM once in each direction instead of being re-read by the GEMM), else a separate pass first
-  // (measured on B200, 200k x 256 x 768: the fused kernel is bit-identical but not faster than the two passes - its
-  // normaliser warps are latency-bound, profiles/r02_ground_fused.md - so it is opt-in: DC_GROUND_FUSED=1)
-  const bool fuse_norm = normalize_fp16_rows && (dim == 512 || dim == 768 || dim == 1024) && ((uintptr_t)x_hi & 15) == 0 &&
-                         getenv("DC_GROUND_FUSED") && !getenv("DC_GROUND_TWO_PASS");
-  if (normalize_fp16_rows && !fuse_norm) {
+  // fp16 features to be normalised in place (models/similarity.py:77): a separate pass before the GEMM. Each row is a
+  // dependent chain (sum of squares, shuffle reduction, sqrt, quotient) that the pass hides behind 64 resident warps per
+  // SM, at the HBM rate. Next to the GEMM's operand ring only a few warps fit, and normalising there cost more than the
+  // GEMM re-reading the rows.
+  // Fused-normaliser experiment (bit-identical, 0.232 vs 0.177 ms on B200): profiles/r02_ground.md.
+  if (normalize_fp16_rows) {
     const int rc = launch_row_normalize(const_cast<void*>(x_hi), DC_F16, n_points, dim, 1, true, nullptr, nullptr, dc::as_stream(stream));
     if (rc) return rc;
   }
@@ -931,7 +915,7 @@ int dc_ground(const void* x_hi, const void* x_lo, int64_t n_points, const void* 
     const int bn = pick_bn(cols);
     Params p{nullptr, nullptr, n_points, cols, dim, n_terms};
     // after the separate normalisation pass the rows written last are still in L2 (126 MB): walk the tiles backwards
-    p.reverse = (normalize_fp16_rows && !fuse_norm && c0 == 0 && !getenv("DC_GROUND_FORWARD")) ? 1 : 0;
+    p.reverse = (normalize_fp16_rows && c0 == 0) ? 1 : 0;
     EpiGround epi{};
     epi.mode = mode;
     epi.n_prompts = cols;
@@ -947,15 +931,7 @@ int dc_ground(const void* x_hi, const void* x_lo, int64_t n_points, const void* 
     epi.argmax_idx = argmax_idx;
     const char* th = (const char*)t_hi + (size_t)c0 * dim * 2;
     const char* tl = t_lo ? (const char*)t_lo + (size_t)c0 * dim * 2 : th;
-    int rc;
-    if (fuse_norm && c0 == 0) {
-      p.norm_rows = reinterpret_cast<__half*>(const_cast<void*>(x_hi));
-      rc = dim == 512 ? launch_bn_norm<2>(bn, x_hi, n_points, th, tl, cols, p, epi, max_tiles, dc::as_stream(stream))
-         : dim == 768 ? launch_bn_norm<3>(bn, x_hi, n_points, th, tl, cols, p, epi, max_tiles, dc::as_stream(stream))
-                      : launch_bn_norm<4>(bn, x_hi, n_points, th, tl, cols, p, epi, max_tiles, dc::as_stream(stream));
-    } else {
-      rc = launch_bn(bn, x_hi, x_lo, n_points, th, tl, cols, p, epi, max_tiles, dc::as_stream(stream));
-    }
+    const int rc = launch_bn(bn, x_hi, x_lo, n_points, th, tl, cols, p, epi, max_tiles, dc::as_stream(stream));
     if (rc) return rc;
   }
   return DC_OK;

@@ -29,20 +29,6 @@ constexpr int kUmmaK = 16;
 constexpr int kThreads = 320;
 constexpr int kEpilogueWarps = 8;
 constexpr int kEpilogueWarp0 = 2;
-// fused row normalisation (grounding, fp16 features): four more warps turn the raw rows of the NEXT tiles into unit rows
-// in global memory (in place, quirk q15 of models/similarity.py:77) while the tensor pipe works on the current tile
-// Warp layout of the fused kernel (640 threads, five warpgroups, registers re-split with setmaxnreg):
-//   WG0  warp 0 TMA producer, warp 1 TMEM allocator + MMA issuer, warps 2-3 idle      (40 registers)
-//   WG1-2 warps 4-11 epilogue                                                           (128 registers)
-//   WG3-4 warps 12-19 normalisers                                                       (88 registers)
-constexpr int kFusedEpilogueWarp0 = 4;
-constexpr int kNormWarp0 = 12;
-constexpr int kNormWarps = 8;
-constexpr int kNormThreads = kNormWarps * 32;
-constexpr int kNormRowsPerWarp = 128 / kNormWarps;  // rows of a tile owned by one normaliser warp
-constexpr int kNormChunkRows = 2;   // rows per bulk copy (one row pair)
-constexpr int kNormBufs = 3;        // staging buffers per normaliser warp (two copies in flight)
-constexpr int kFusedThreads = (kNormWarp0 + kNormWarps) * 32;
 
 struct Tile {
   int a_row;   // first row of the A tile
@@ -58,32 +44,23 @@ struct Params {
   int n_cols;             // valid columns (dense tiling)
   int k;                  // inner dimension (multiple of 64)
   int n_terms;            // 1: hi.hi   2: + hi.lo   3: + lo.hi
-  __half* norm_rows;      // fused normalisation: the fp16 A matrix itself ([m_total, k], dense tiling), else nullptr
   int reverse;            // dense tiling: walk the row tiles last to first (the rows a preceding pass wrote last are still in L2)
 };
 
-// kNormChunks: 0 = plain GEMM; else k == 256 * kNormChunks and four extra warps normalise the A rows in place
-template <int BN, int kNormChunks = 0>
+template <int BN>
 struct Config {
   static constexpr int kStageBytesA = kBlockM * kBlockK * 2;
   static constexpr int kStageBytesB = BN * kBlockK * 2;
   static constexpr int kStageBytes = kStageBytesA + kStageBytesB;
-  static constexpr int kNormRowBytes = kNormChunks * 512;                            // 256 fp16 per chunk
-  static constexpr int kNormBufBytes = kNormChunkRows * kNormRowBytes;               // one bulk copy
-  static constexpr int kNormBytes = kNormWarps * kNormBufs * kNormBufBytes;          // 72 KB at k = 768
   static constexpr int kBarrierBytes = 512;
   static constexpr int kScratchBytes = kBlockM * 8 * 4;                              // epilogue scratch
-  static constexpr int kBudget = 227 * 1024 - 1024 - kBarrierBytes - kScratchBytes - kNormBytes;
-  static constexpr int kStagesPlain = (BN >= 256) ? 4 : (BN >= 128 ? 6 : 8);
-  static constexpr int kStagesFit = kBudget / kStageBytes;
-  static constexpr int kStages = (kNormChunks == 0 || kStagesFit >= kStagesPlain) ? kStagesPlain : kStagesFit;
-  static constexpr int kThreadsTotal = kNormChunks ? kFusedThreads : kThreads;
+  static constexpr int kStages = (BN >= 256) ? 4 : (BN >= 128 ? 6 : 8);
   static constexpr int kTmemCols = (2 * BN < 32) ? 32 : 2 * BN;  // two accumulator buffers
-  static constexpr int kSmemBytes = kStages * kStageBytes + 1024 /*align slack*/ + kBarrierBytes + kScratchBytes + kNormBytes;
+  static constexpr int kSmemBytes = kStages * kStageBytes + 1024 /*align slack*/ + kBarrierBytes + kScratchBytes;
   static_assert(BN % 16 == 0 && BN >= 16 && BN <= 256, "invalid UMMA N");
   static_assert((kTmemCols & (kTmemCols - 1)) == 0 && kTmemCols <= 512, "TMEM columns must be a power of two");
-  static_assert(kStages >= 2, "not enough shared memory for the operand ring");
-  static_assert((2 * kStages + 4) * 8 + 8 + (kNormWarps * kNormBufs + 4) * 8 <= kBarrierBytes, "barrier region too small");
+  static_assert(kSmemBytes <= 227 * 1024, "not enough shared memory for the operand ring");
+  static_assert((2 * kStages + 4) * 8 + 8 <= kBarrierBytes, "barrier region too small");
 };
 
 __device__ __forceinline__ Tile fetch_tile(const Params& p, int t) {
@@ -103,201 +80,11 @@ __device__ __forceinline__ Tile fetch_tile(const Params& p, int t) {
 //   void finish(const Tile&, int row_in_tile, int half, int n_halves, float* scratch);
 //        // after the last chunk; `scratch` = kBlockM * 8 floats of shared memory for combining the two
 //        // column halves of a row (all epilogue threads of the active groups call finish together)
-// ---- fused normaliser helpers
-__device__ __forceinline__ void bulk_load(void* smem_dst, const void* gmem_src, uint32_t bytes, uint64_t* bar) {
-  asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];"
-               ::"r"(umma::smem_u32(smem_dst)), "l"(gmem_src), "r"(bytes), "r"(umma::smem_u32(bar)) : "memory");
-}
-__device__ __forceinline__ double warp_sum_f64_(double v) {
-#pragma unroll
-  for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
-  return v;
-}
-
-// One normaliser warp. Tile t of this CTA: the warp owns rows [16 w, 16 w + 16) of the tile, fetched a row pair at a time
-// by bulk copies into its own staging buffers (two copies in flight), normalised with torch's fp16 semantics (norm and
-// quotient rounded to fp16, bit-identical to row_normalize_vec_kernel) and written back in place with 16-byte stores.
-// When the warp's rows of a tile are out, it publishes them to the async proxy and arrives on tile_ready; the TMA
-// producer loads the A tile (now an L2 hit) only after all normaliser warps have arrived.
-template <int kNormChunks>
-__device__ __forceinline__ void normaliser_warp(const Params& p, int nw, int lane, int n_tiles, uint8_t* bufs, uint64_t* nfull,
-                                                uint64_t* tile_ready, uint64_t* tile_free) {
-  constexpr int kRowBytes = kNormChunks * 512;
-  constexpr int kBufBytes = kNormChunkRows * kRowBytes;
-  constexpr int kRowVec = kRowBytes / 16;
-  uint8_t* my_bufs = bufs + (size_t)nw * kNormBufs * kBufBytes;
-  uint64_t* my_full = nfull + nw * kNormBufs;
-  const int64_t m_total = p.m_total;
-  auto warp_rows = [&](int t) -> int {  // rows of tile t owned by this warp
-    const int64_t left = m_total - (int64_t)t * kBlockM - nw * kNormRowsPerWarp;
-    return left <= 0 ? 0 : (left < kNormRowsPerWarp ? (int)left : kNormRowsPerWarp);
-  };
-  // issue side: (tile, chunk) iterator running two chunks ahead of the consumer
-  int it = blockIdx.x, ic = 0, ib = 0;
-  auto issue = [&]() {
-    while (it < n_tiles && ic * kNormChunkRows >= warp_rows(it)) { it += gridDim.x; ic = 0; }
-    if (it >= n_tiles) return;
-    const int rows = min(kNormChunkRows, warp_rows(it) - ic * kNormChunkRows);
-    if (lane == 0) {
-      const uint32_t bytes = (uint32_t)rows * kRowBytes;
-      umma::mbar_expect_tx(my_full + ib, bytes);
-      const uint8_t* src = reinterpret_cast<const uint8_t*>(p.norm_rows) +
-                           ((int64_t)it * kBlockM + nw * kNormRowsPerWarp + ic * kNormChunkRows) * kRowBytes;
-      bulk_load(my_bufs + ib * kBufBytes, src, bytes, my_full + ib);
-    }
-    ++ic;
-    if (++ib == kNormBufs) ib = 0;
-  };
-  issue();
-  issue();
-  int cb = 0;
-  uint32_t full_phase = 0;  // bit b = parity to wait for on buffer b
-  int local_tile = 0;
-  for (int t = blockIdx.x; t < n_tiles; t += gridDim.x, ++local_tile) {
-    const int slot = local_tile & 1;
-    umma::mbar_wait(tile_free + slot, (((uint32_t)local_tile >> 1) & 1u) ^ 1u);  // at most two tiles ahead of the TMA producer
-    const int rows = warp_rows(t);
-#pragma unroll 1
-    for (int c = 0; c * kNormChunkRows < rows; ++c) {
-      const int n = min(kNormChunkRows, rows - c * kNormChunkRows);  // 2, or 1 at a ragged end
-      umma::mbar_wait(my_full + cb, (full_phase >> cb) & 1u);
-      full_phase ^= 1u << cb;
-      const int4* src = reinterpret_cast<const int4*>(my_bufs + cb * kBufBytes);
-      int4* dst = reinterpret_cast<int4*>(reinterpret_cast<uint8_t*>(p.norm_rows) +
-                                          ((int64_t)t * kBlockM + nw * kNormRowsPerWarp + c * kNormChunkRows) * kRowBytes);
-      // The two rows go through the steps together: the latency of one row's dependent chain (accumulation, shuffle
-      // reduction, sqrt) is covered by the other row. Arithmetic is two-wide (fma.rn.f32x2) on the half2 pairs.
-      int4 raw[2][kNormChunks];
-#pragma unroll
-      for (int r = 0; r < 2; ++r) {
-        const int rr = (r < n) ? r : 0;  // a missing second row repeats the first (never stored)
-#pragma unroll
-        for (int k = 0; k < kNormChunks; ++k) raw[r][k] = src[rr * kRowVec + k * 32 + lane];
-      }
-      // Norm = fp16(sqrt(sum x^2)), CORRECTLY rounded (row_normalize_vec_kernel accumulates in fp64). Here the squares
-      // (exact in fp32: 11-bit significands) are summed in fp32 - every partial sum is positive, so the split chains +
-      // 5 shuffle rounds + sqrt stay within 20 eps = 1.2e-6 of the exact norm - and the fp16 rounding of both ends of
-      // that interval is compared: equal (99 % of the rows) means it IS the rounding of the exact norm; otherwise the
-      // row pair is re-summed in fp64.
-      float2 sf[2][2];
-#pragma unroll
-      for (int r = 0; r < 2; ++r) {
-        sf[r][0] = sf[r][1] = make_float2(0.f, 0.f);
-#pragma unroll
-        for (int k = 0; k < kNormChunks; ++k) {
-          const __half2* h2 = reinterpret_cast<const __half2*>(&raw[r][k]);
-#pragma unroll
-          for (int j = 0; j < 4; ++j) {
-            const float2 f = __half22float2(h2[j]);
-            sf[r][j & 1] = __ffma2_rn(f, f, sf[r][j & 1]);
-          }
-        }
-        const float2 s2 = __fadd2_rn(sf[r][0], sf[r][1]);
-        sf[r][0].x = s2.x + s2.y;
-      }
-#pragma unroll
-      for (int o = 16; o > 0; o >>= 1) {
-#pragma unroll
-        for (int r = 0; r < 2; ++r) sf[r][0].x += __shfl_xor_sync(0xffffffffu, sf[r][0].x, o);
-      }
-      float nrm[2];
-      bool exact = true;
-#pragma unroll
-      for (int r = 0; r < 2; ++r) {
-        const float n32 = sqrtf(sf[r][0].x);
-        const __half lo = __float2half_rn(n32 * (1.0f - 1.5e-6f)), hi = __float2half_rn(n32 * (1.0f + 1.5e-6f));
-        nrm[r] = __half2float(lo);
-        // overflow to inf, NaN, zero or tiny sums: the fp64 path decides
-        exact &= (__half_as_ushort(lo) == __half_as_ushort(hi)) && n32 < 60000.f && sf[r][0].x > 1e-12f;
-      }
-      if (!exact) {
-#pragma unroll 1
-        for (int r = 0; r < 2; ++r) {
-          double s0 = 0.0, s1 = 0.0;
-#pragma unroll 1
-          for (int k = 0; k < kNormChunks; ++k) {
-            const __half2* h2 = reinterpret_cast<const __half2*>(&raw[r][k]);
-#pragma unroll
-            for (int j = 0; j < 4; ++j) {
-              const float2 f = __half22float2(h2[j]);
-              s0 = fma((double)f.x, (double)f.x, s0);
-              s1 = fma((double)f.y, (double)f.y, s1);
-            }
-          }
-          nrm[r] = __half2float(__double2half(sqrt(warp_sum_f64_(s0 + s1))));
-        }
-      }
-      float rinv[2];
-#pragma unroll
-      for (int r = 0; r < 2; ++r) {
-        rinv[r] = 1.0f / nrm[r];
-#pragma unroll
-        for (int k = 0; k < kNormChunks; ++k)  // the fp16 words stay the live form of the rows (the converted floats of the
-          asm volatile("" : "+r"(raw[r][k].x), "+r"(raw[r][k].y), "+r"(raw[r][k].z), "+r"(raw[r][k].w));  // sum phase are not kept)
-      }
-      // x / nrm, correctly rounded (what the IEEE division of row_normalize_vec_kernel / torch returns): with the
-      // correctly rounded reciprocal r, q = x * r, the exact remainder x - q * nrm and one fma give RN(x / nrm)
-      // (Markstein; nrm is an fp16 value, so its significand is never all ones). A zero, infinite or NaN norm takes
-      // the plain division (inf / NaN results exactly like torch) - decided once per row pair, outside the element loops.
-      const bool sane = nrm[0] > 0.f && nrm[0] < INFINITY && nrm[1] > 0.f && nrm[1] < INFINITY;
-      if (sane) {
-#pragma unroll
-        for (int r = 0; r < 2; ++r) {
-          const float2 rv = make_float2(rinv[r], rinv[r]), nn = make_float2(-nrm[r], -nrm[r]);
-#pragma unroll
-          for (int k = 0; k < kNormChunks; ++k) {
-            const __half2* h2 = reinterpret_cast<const __half2*>(&raw[r][k]);
-            int4 packed;
-            __half2* o2 = reinterpret_cast<__half2*>(&packed);
-#pragma unroll
-            for (int j = 0; j < 4; ++j) {
-              const float2 f = __half22float2(h2[j]);
-              const float2 q0 = __fmul2_rn(f, rv);
-              const float2 q1 = __ffma2_rn(__ffma2_rn(q0, nn, f), rv, q0);
-              o2[j] = __floats2half2_rn(q1.x, q1.y);
-            }
-            // the quotient carries the sign of x ((+0) + (-0) = +0 in the last fma would lose the sign of a -0 entry)
-            packed.x = (packed.x & 0x7fff7fff) | (raw[r][k].x & 0x80008000);
-            packed.y = (packed.y & 0x7fff7fff) | (raw[r][k].y & 0x80008000);
-            packed.z = (packed.z & 0x7fff7fff) | (raw[r][k].z & 0x80008000);
-            packed.w = (packed.w & 0x7fff7fff) | (raw[r][k].w & 0x80008000);
-            if (r < n) dst[r * kRowVec + k * 32 + lane] = packed;
-          }
-        }
-      } else {
-#pragma unroll 1
-        for (int r = 0; r < 2; ++r) {
-#pragma unroll 1
-          for (int k = 0; k < kNormChunks; ++k) {
-            const __half2* h2 = reinterpret_cast<const __half2*>(&raw[r][k]);
-            int4 packed;
-            __half2* o2 = reinterpret_cast<__half2*>(&packed);
-#pragma unroll
-            for (int j = 0; j < 4; ++j) {
-              const float2 f = __half22float2(h2[j]);
-              o2[j] = __floats2half2_rn(f.x / nrm[r], f.y / nrm[r]);
-            }
-            if (r < n) dst[r * kRowVec + k * 32 + lane] = packed;
-          }
-        }
-      }
-      __syncwarp();  // every lane is done reading the buffer before the next bulk copy overwrites it
-      issue();
-      if (++cb == kNormBufs) cb = 0;
-    }
-    // publish this warp's rows of the tile: device-scope visibility, then generic -> async proxy, then the arrival
-    __threadfence();
-    asm volatile("fence.proxy.async;" ::: "memory");
-    __syncwarp();
-    if (lane == 0) umma::mbar_arrive(tile_ready + slot);
-  }
-}
-
-template <int BN, class Epi, int kNormChunks = 0>
-__global__ void __launch_bounds__(Config<BN, kNormChunks>::kThreadsTotal, 1)
+template <int BN, class Epi>
+__global__ void __launch_bounds__(kThreads, 1)
 gemm_kernel(const __grid_constant__ CUtensorMap tm_a_hi, const __grid_constant__ CUtensorMap tm_a_lo,
             const __grid_constant__ CUtensorMap tm_b_hi, const __grid_constant__ CUtensorMap tm_b_lo, Params p, Epi epi) {
-  using Cfg = Config<BN, kNormChunks>;
+  using Cfg = Config<BN>;
   extern __shared__ uint8_t smem_raw[];
   const uint32_t raw_addr = umma::smem_u32(smem_raw);
   uint8_t* smem = smem_raw + ((1024u - (raw_addr & 1023u)) & 1023u);  // SWIZZLE_128B tiles need 1024-B alignment
@@ -309,15 +96,10 @@ gemm_kernel(const __grid_constant__ CUtensorMap tm_a_hi, const __grid_constant__
   uint64_t* tmem_full = bars + 2 * Cfg::kStages;   // [2]
   uint64_t* tmem_empty = tmem_full + 2;            // [2]
   uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(tmem_empty + 2);
-  uint64_t* norm_full = tmem_empty + 3;                                // [kNormWarps * kNormBufs]
-  uint64_t* tile_ready = norm_full + kNormWarps * kNormBufs;           // [2] normalisers -> TMA producer
-  uint64_t* tile_free = tile_ready + 2;                                // [2] TMA producer -> normalisers
   float* epi_scratch = reinterpret_cast<float*>(smem + Cfg::kStages * Cfg::kStageBytes + Cfg::kBarrierBytes);  // [kBlockM * 8]
-  uint8_t* norm_bufs = smem + Cfg::kStages * Cfg::kStageBytes + Cfg::kBarrierBytes + Cfg::kScratchBytes;
 
   const int warp = threadIdx.x >> 5;
   const int lane = threadIdx.x & 31;
-  constexpr int kEpi0 = kNormChunks ? kFusedEpilogueWarp0 : kEpilogueWarp0;
   const int n_tiles = p.tiles ? __ldg(p.tile_count) : (int)ceil_div<int64_t>(p.m_total, kBlockM);
   const int k_blocks = p.k / kBlockK;
 
@@ -334,13 +116,6 @@ gemm_kernel(const __grid_constant__ CUtensorMap tm_a_hi, const __grid_constant__
       umma::mbar_init(tmem_full + a, 1);
       umma::mbar_init(tmem_empty + a, (BN >= 64) ? 8 : 4);  // one arrival per active epilogue warp
     }
-    if (kNormChunks) {
-      for (int b = 0; b < kNormWarps * kNormBufs; ++b) umma::mbar_init(norm_full + b, 1);
-      for (int a = 0; a < 2; ++a) {
-        umma::mbar_init(tile_ready + a, kNormWarps);
-        umma::mbar_init(tile_free + a, 1);
-      }
-    }
     umma::fence_barrier_init();
   }
   if (warp == 1) {
@@ -352,24 +127,13 @@ gemm_kernel(const __grid_constant__ CUtensorMap tm_a_hi, const __grid_constant__
   umma::fence_after_sync();
   const uint32_t tmem_base = *tmem_slot;
 
-  // Fused kernel: 640 threads start with 96 registers each; the producer group and the normalisers hand registers to
-  // the epilogue (56 * 128 + 2 * 8 * 128 = 9216 released, 2 * 32 * 128 = 8192 taken). Each setmaxnreg sits at the head of
-  // its role's code so that the register allocation of that code follows it.
-  if (kNormChunks && warp < 4) asm volatile("setmaxnreg.dec.sync.aligned.u32 40;");
-
   if (warp == 0) {
     // ===================== TMA producer =====================
     if (lane == 0) {
       int stage = 0;
       uint32_t phase = 0;
-      int local_tile = 0;
-      for (int t = blockIdx.x; t < n_tiles; t += gridDim.x, ++local_tile) {
+      for (int t = blockIdx.x; t < n_tiles; t += gridDim.x) {
         const Tile tile = fetch_tile(p, t);
-        if (kNormChunks) {  // the tile's rows must have been normalised (and published to the async proxy) first
-          const int slot = local_tile & 1;
-          umma::mbar_wait(tile_ready + slot, ((uint32_t)local_tile >> 1) & 1u);
-          umma::mbar_arrive(tile_free + slot);
-        }
         for (int term = 0; term < p.n_terms; ++term) {
           const CUtensorMap* ta = (term == 2) ? &tm_a_lo : &tm_a_hi;
           const CUtensorMap* tb = (term == 1) ? &tm_b_lo : &tm_b_hi;
@@ -413,18 +177,13 @@ gemm_kernel(const __grid_constant__ CUtensorMap tm_a_hi, const __grid_constant__
         if (++acc == 2) { acc = 0; acc_phase ^= 1; }
       }
     }
-  } else if (kNormChunks && warp >= kNormWarp0) {
-    // ===================== normaliser warps =====================
-    asm volatile("setmaxnreg.dec.sync.aligned.u32 88;");
-    normaliser_warp<kNormChunks ? kNormChunks : 1>(p, warp - kNormWarp0, lane, n_tiles, norm_bufs, norm_full, tile_ready, tile_free);
-  } else if (warp >= kEpi0) {
+  } else if (warp >= kEpilogueWarp0) {
     // ===================== epilogue warps =====================
-    if (kNormChunks) asm volatile("setmaxnreg.inc.sync.aligned.u32 128;");
     constexpr int kHalves = (BN >= 64) ? 2 : 1;
     constexpr int kHalfCols = BN / kHalves;
     constexpr int kChunks = kHalfCols / 32;
     const int quarter = warp & 3;  // TMEM lane quarter this warp may access
-    const int half = (warp - kEpi0) >> 2;
+    const int half = (warp - kEpilogueWarp0) >> 2;
     const int row_in_tile = quarter * 32 + lane;
     if (half < kHalves) {
       int acc = 0;
@@ -479,21 +238,21 @@ gemm_kernel(const __grid_constant__ CUtensorMap tm_a_hi, const __grid_constant__
 // dependency on libcuda.
 int encode_plane_map(CUtensorMap* out, const void* base, int64_t rows, int k, int box_rows);
 
-template <int BN, class Epi, int kNormChunks = 0>
+template <int BN, class Epi>
 int launch(const void* a_hi, const void* a_lo, int64_t a_rows, const void* b_hi, const void* b_lo, int64_t b_rows,
            const Params& p, const Epi& epi, int max_tiles, cudaStream_t st) {
-  using Cfg = Config<BN, kNormChunks>;
+  using Cfg = Config<BN>;
   CUtensorMap ta_hi, ta_lo, tb_hi, tb_lo;
   int rc;
   if ((rc = encode_plane_map(&ta_hi, a_hi, a_rows, p.k, kBlockM))) return rc;
   if ((rc = encode_plane_map(&ta_lo, a_lo ? a_lo : a_hi, a_rows, p.k, kBlockM))) return rc;
   if ((rc = encode_plane_map(&tb_hi, b_hi, b_rows, p.k, BN))) return rc;
   if ((rc = encode_plane_map(&tb_lo, b_lo ? b_lo : b_hi, b_rows, p.k, BN))) return rc;
-  auto kern = gemm_kernel<BN, Epi, kNormChunks>;
+  auto kern = gemm_kernel<BN, Epi>;
   DC_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, Cfg::kSmemBytes));
   int grid = max_tiles < sm_count() ? max_tiles : sm_count();
   if (grid < 1) grid = 1;
-  kern<<<grid, Cfg::kThreadsTotal, Cfg::kSmemBytes, st>>>(ta_hi, ta_lo, tb_hi, tb_lo, p, epi);
+  kern<<<grid, kThreads, Cfg::kSmemBytes, st>>>(ta_hi, ta_lo, tb_hi, tb_lo, p, epi);
   DC_LAUNCH_CHECK();
   return DC_OK;
 }

@@ -13,7 +13,6 @@
 // Bicubic weights follow ATen's upsample_bicubic2d (align_corners=False, A=-0.75, source index
 // scale*(dst+0.5)-0.5 un-clamped, taps clamped to the border).
 #include <algorithm>
-#include <stdlib.h>
 
 #include "common.cuh"
 #include "umma.cuh"
@@ -1479,7 +1478,7 @@ int dc_pixel_fuse_mma(const double* points, const int64_t* point_off, const int6
   // regions: the rows one region adds to should fit well inside the 126 MB L2 (~24 MB per region), while every scene keeps
   // enough points per region for full tiles
   int n_regions = 1;
-  if (rank && !getenv("DC_PIXEL_ONE_REGION")) {
+  if (rank) {
     const int64_t row_bytes = (int64_t)dim * 4;
     const int64_t want = dc::ceil_div<int64_t>(max_points_per_scene * n_scenes * row_bytes, (int64_t)24 << 20);
     n_regions = (int)std::max<int64_t>(1, std::min<int64_t>(std::min<int64_t>(want, mma::kMaxRegions), max_points_per_scene / 2048));

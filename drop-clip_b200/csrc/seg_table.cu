@@ -145,7 +145,13 @@ __global__ void __launch_bounds__(kThreads) seg_histogram_kernel(const T* __rest
 // Counting is the same run-length scheme as above. A lane owns 64 contiguous bytes = eight neighbouring pixels:
 // "all eight equal" is an XOR/OR tree on the ALU, then one 64-bit compare against the current run.
 constexpr int kUnit = 2048;  // bytes per warp unit: 32 lanes x 64 B
-constexpr int kRingDepthDefault = 2;
+// 12 warps x 2 slots x 2 KB = 48 KB of ring, beside two filter CTAs in the shared carve-out (common.cuh).
+// Alone: 6.7 TB/s (3 slots: 7.2, 8 warps: 5.8); the two-stream step: 2.75-2.78 ms with 2 slots, 2.80-2.85 with 3
+// (B200, profiles/r02_seg_ring.md).
+constexpr int kRingWarps = 12;
+constexpr int kRingMinCtas = 3;
+constexpr int kRingThreads = kRingWarps * 32;
+constexpr int kRingDepth = 2;
 
 __device__ __forceinline__ void bulk_load_evict_first(void* smem_dst, const void* gmem_src, uint32_t bytes, uint64_t* bar,
                                                       uint64_t policy) {
@@ -185,13 +191,11 @@ __device__ __forceinline__ unsigned or_xor(unsigned acc, unsigned x, unsigned re
 constexpr int kTicketSlots = 64;
 __device__ unsigned g_ring_tickets[kTicketSlots];
 
-template <int kRingWarps, int kMinCtas>
-__global__ void __launch_bounds__(kRingWarps * 32, kMinCtas)
+__global__ void __launch_bounds__(kRingThreads, kRingMinCtas)
 seg_histogram_ring_kernel(const long long* __restrict__ seg, int64_t bytes_per_view, int units_per_view, int total_views,
-                          int nbins, int depth, int flags, unsigned* __restrict__ ticket, uint32_t* __restrict__ counts,
+                          int nbins, int depth, unsigned* __restrict__ ticket, uint32_t* __restrict__ counts,
                           unsigned long long* __restrict__ outside_out) {
   using namespace dc::umma;
-  constexpr int kRingThreads = kRingWarps * 32;
   extern __shared__ __align__(128) unsigned char s_ring[];  // [warps][depth][2 KB], histogram, full[warps][depth], views[2]
   const size_t ring_bytes = (size_t)kRingWarps * depth * kUnit;
   unsigned* s_hist = reinterpret_cast<unsigned*>(s_ring + ring_bytes);
@@ -230,11 +234,7 @@ seg_histogram_ring_kernel(const long long* __restrict__ seg, int64_t bytes_per_v
   auto issue = [&]() {
     const uint32_t bytes = (uint32_t)(pj == units_per_view - 1 ? last_bytes : kUnit);
     mbar_expect_tx(full + pslot, bytes);
-    if (flags & 2)
-      asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];"
-                   ::"r"(smem_u32(my_ring + pslot * kUnit)), "l"(psrc), "r"(bytes), "r"(smem_u32(full + pslot)) : "memory");
-    else
-      bulk_load_evict_first(my_ring + pslot * kUnit, psrc, bytes, full + pslot, policy);
+    bulk_load_evict_first(my_ring + pslot * kUnit, psrc, bytes, full + pslot, policy);
     pslot = (pslot == depth - 1) ? 0 : pslot + 1;
     pj += kRingWarps;
     psrc += kRingWarps * kUnit;
@@ -267,52 +267,45 @@ seg_histogram_ring_kernel(const long long* __restrict__ seg, int64_t bytes_per_v
     if (v >= total_views) break;
     unsigned long long* outside = outside_out + 4 * (int64_t)v;
     for (int it = 0; it < n_it; ++it) {
-      if (flags & 4)
-        mbar_wait(full + slot, parity);
-      else
-        mbar_wait_suspended(full + slot, parity);
+      mbar_wait_suspended(full + slot, parity);
       if (!(ends_partial && it == n_it - 1)) {
         int4 r[4];
 #pragma unroll
         for (int k = 0; k < 4; ++k) r[k] = *reinterpret_cast<const int4*>(slot_ptr + off[k]);
-        if (flags & 1) {
-          run.cnt += (unsigned)(r[0].x ^ r[1].y ^ r[2].z ^ r[3].w) & 1u;
-        } else {
-          const unsigned lo0 = (unsigned)r[0].x, hi0 = (unsigned)r[0].y;
-          unsigned dl = (unsigned)r[0].z ^ lo0, dh = (unsigned)r[0].w ^ hi0;
+        const unsigned lo0 = (unsigned)r[0].x, hi0 = (unsigned)r[0].y;
+        unsigned dl = (unsigned)r[0].z ^ lo0, dh = (unsigned)r[0].w ^ hi0;
 #pragma unroll
-          for (int k = 1; k < 4; ++k) {
-            dl = or_xor(or_xor(dl, (unsigned)r[k].x, lo0), (unsigned)r[k].z, lo0);
-            dh = or_xor(or_xor(dh, (unsigned)r[k].y, hi0), (unsigned)r[k].w, hi0);
-          }
-          if ((dl | dh) == 0) {  // eight equal ids
-            const long long id = (long long)(((unsigned long long)hi0 << 32) | lo0);
-            if (id != run.cur) {
-              flush_run(run, s_hist, outside, nbins);
-              run.cur = id;
-              run.cnt = 0;
-            }
-            run.cnt += 8;
-          } else {
-            // an object boundary inside the lane's eight pixels. The other lanes of the warp wait for this path, so it
-            // is kept short and free of dependent chains: close the run, then one shared-memory atomic per pixel.
+        for (int k = 1; k < 4; ++k) {
+          dl = or_xor(or_xor(dl, (unsigned)r[k].x, lo0), (unsigned)r[k].z, lo0);
+          dh = or_xor(or_xor(dh, (unsigned)r[k].y, hi0), (unsigned)r[k].w, hi0);
+        }
+        if ((dl | dh) == 0) {  // eight equal ids
+          const long long id = (long long)(((unsigned long long)hi0 << 32) | lo0);
+          if (id != run.cur) {
             flush_run(run, s_hist, outside, nbins);
-            run.cur = -1;
+            run.cur = id;
             run.cnt = 0;
-            const unsigned hi_any = (unsigned)r[0].y | (unsigned)r[0].w | (unsigned)r[1].y | (unsigned)r[1].w | (unsigned)r[2].y |
-                                    (unsigned)r[2].w | (unsigned)r[3].y | (unsigned)r[3].w;
-            const unsigned lo_max = max(max(max((unsigned)r[0].x, (unsigned)r[0].z), max((unsigned)r[1].x, (unsigned)r[1].z)),
-                                        max(max((unsigned)r[2].x, (unsigned)r[2].z), max((unsigned)r[3].x, (unsigned)r[3].z)));
-            if (hi_any == 0 && lo_max < (unsigned)nbins) {
+          }
+          run.cnt += 8;
+        } else {
+          // an object boundary inside the lane's eight pixels. The other lanes of the warp wait for this path, so it
+          // is kept short and free of dependent chains: close the run, then one shared-memory atomic per pixel.
+          flush_run(run, s_hist, outside, nbins);
+          run.cur = -1;
+          run.cnt = 0;
+          const unsigned hi_any = (unsigned)r[0].y | (unsigned)r[0].w | (unsigned)r[1].y | (unsigned)r[1].w | (unsigned)r[2].y |
+                                  (unsigned)r[2].w | (unsigned)r[3].y | (unsigned)r[3].w;
+          const unsigned lo_max = max(max(max((unsigned)r[0].x, (unsigned)r[0].z), max((unsigned)r[1].x, (unsigned)r[1].z)),
+                                      max(max((unsigned)r[2].x, (unsigned)r[2].z), max((unsigned)r[3].x, (unsigned)r[3].z)));
+          if (hi_any == 0 && lo_max < (unsigned)nbins) {
 #pragma unroll
-              for (int k = 0; k < 4; ++k) {
-                atomicAdd(s_hist + (unsigned)r[k].x, 1u);
-                atomicAdd(s_hist + (unsigned)r[k].z, 1u);
-              }
-            } else {  // ids outside the histogram (negative background, id >= nbins): the general path
-#pragma unroll
-              for (int k = 0; k < 4; ++k) consume_vector<long long>(r[k], run, s_hist, outside, nbins);
+            for (int k = 0; k < 4; ++k) {
+              atomicAdd(s_hist + (unsigned)r[k].x, 1u);
+              atomicAdd(s_hist + (unsigned)r[k].z, 1u);
             }
+          } else {  // ids outside the histogram (negative background, id >= nbins): the general path
+#pragma unroll
+            for (int k = 0; k < 4; ++k) consume_vector<long long>(r[k], run, s_hist, outside, nbins);
           }
         }
       } else {  // partial last unit of the view
@@ -350,17 +343,15 @@ seg_histogram_ring_kernel(const long long* __restrict__ seg, int64_t bytes_per_v
   }
 }
 
-inline bool ring_fits(int64_t bytes_per_view, int warps, int depth) {
-  return dc::ceil_div<int64_t>(bytes_per_view, kUnit) >= (int64_t)4 * warps * depth;
+inline bool ring_fits(int64_t bytes_per_view) {
+  return dc::ceil_div<int64_t>(bytes_per_view, kUnit) >= (int64_t)4 * kRingWarps * kRingDepth;
 }
 
-template <int kRingWarps, int kMinCtas>
-int launch_ring(const void* seg, int64_t bytes_per_view, int64_t total_views, int nbins, int depth, int flags, int carve,
-                uint32_t* counts, uint64_t* outside, cudaStream_t st) {
-  auto kernel = seg_histogram_ring_kernel<kRingWarps, kMinCtas>;
+int launch_ring(const void* seg, int64_t bytes_per_view, int64_t total_views, int nbins, uint32_t* counts, uint64_t* outside,
+                cudaStream_t st) {
   const int upv = (int)dc::ceil_div<int64_t>(bytes_per_view, kUnit);
-  const size_t smem = (size_t)kRingWarps * depth * kUnit + ((sizeof(unsigned) * nbins + 15) & ~(size_t)15) +
-                      (size_t)kRingWarps * depth * sizeof(uint64_t) + 16;
+  const size_t smem = (size_t)kRingWarps * kRingDepth * kUnit + ((sizeof(unsigned) * nbins + 15) & ~(size_t)15) +
+                      (size_t)kRingWarps * kRingDepth * sizeof(uint64_t) + 16;
   // a zeroed ticket counter per launch; launches in flight at the same time use different slots
   static std::atomic<unsigned> next_slot{0};
   static unsigned* tickets_of_device[dc::FuncAttrCache::kMaxDevices] = {nullptr};
@@ -374,12 +365,13 @@ int launch_ring(const void* seg, int64_t bytes_per_view, int64_t total_views, in
   unsigned* ticket = tickets + next_slot.fetch_add(1) % kTicketSlots;
   DC_CUDA(cudaMemsetAsync(ticket, 0, sizeof(unsigned), st));
   static dc::FuncAttrCache smem_attr, carve_attr;
-  DC_CUDA(smem_attr.set(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+  DC_CUDA(smem_attr.set(seg_histogram_ring_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
   // the SM's shared-memory carve-out is fixed while CTAs are resident: ask for one under which the filter's CTAs fit beside
-  DC_CUDA(carve_attr.set(kernel, cudaFuncAttributePreferredSharedMemoryCarveout, carve));
+  const int carve = dc::stream_overlap() ? dc::kOverlapCarveoutPct : cudaSharedmemCarveoutDefault;
+  DC_CUDA(carve_attr.set(seg_histogram_ring_kernel, cudaFuncAttributePreferredSharedMemoryCarveout, carve));
   const int grid = (int)std::min<int64_t>(dc::sm_count(), total_views);
-  kernel<<<grid, kRingWarps * 32, smem, st>>>((const long long*)seg, bytes_per_view, upv, (int)total_views, nbins, depth, flags, ticket,
-                                              counts, (unsigned long long*)outside);
+  seg_histogram_ring_kernel<<<grid, kRingThreads, smem, st>>>((const long long*)seg, bytes_per_view, upv, (int)total_views, nbins,
+                                                             kRingDepth, ticket, counts, (unsigned long long*)outside);
   DC_LAUNCH_CHECK();
   return DC_OK;
 }
@@ -455,26 +447,13 @@ extern "C" int dc_seg_histogram(const void* seg, int seg_dtype, int64_t total_vi
   DC_CUDA(cudaMemsetAsync(outside, 0, sizeof(uint64_t) * 4 * (size_t)total_views, st));
   // int64 maps with 16-byte aligned views, enough of them to give every SM a few MB: the ring kernel (bulk copies)
   const int64_t bytes_per_view = pixels_per_view * esize;
-  const char* mode = getenv("DC_SEG_MODE");  // "ldg" / "ring": force one kernel (benchmarks/ring_probe.py)
+  // DC_SEG_MODE=ring forces the ring kernel wherever its preconditions hold, so that tests reach it at small sizes. It is
+  // the library's only environment switch: every other launch decision follows from the arguments and the overlap mode.
+  const char* mode = getenv("DC_SEG_MODE");
   const bool forced = mode && strcmp(mode, "ring") == 0;
-  const bool want_ring = forced || (!mode && dc::stream_overlap() && total_views * bytes_per_view >= (int64_t)dc::sm_count() * (4 << 20));
-  int depth = kRingDepthDefault, warps = 12;
-  if (const char* e = getenv("DC_SEG_STAGES")) depth = max(2, min(12, atoi(e)));
-  if (const char* e = getenv("DC_SEG_WARPS")) warps = atoi(e) == 16 ? 16 : atoi(e) == 8 ? 8 : 12;
-  const bool ring_ok = want_ring && seg_dtype == DC_I64 && (uintptr_t)seg % 16 == 0 && bytes_per_view % 16 == 0 &&
-                       ring_fits(bytes_per_view, warps, depth);
-  if (ring_ok) {
-    // 12 warps x 2 slots x 2 KB = 48 KB of ring, beside two filter CTAs in the shared carve-out (common.cuh).
-    // Alone: 6.7 TB/s (3 slots: 7.2, 8 warps: 5.8); the two-stream step: 2.75-2.78 ms with 2 slots, 2.80-2.85 with 3.
-    int carve = dc::stream_overlap() ? dc::kOverlapCarveoutPct : cudaSharedmemCarveoutDefault;
-    if (const char* e = getenv("DC_CARVEOUT_PCT")) carve = atoi(e);
-    // measurement switches of benchmarks/ring_probe.py (1: copy only - WRONG counts -, 2: no L2 policy, 4: spin-wait):
-    // honoured only together with DC_SEG_MODE=ring, never on the default path
-    const int flags = forced && getenv("DC_SEG_FLAGS") ? atoi(getenv("DC_SEG_FLAGS")) : 0;
-    if (warps == 16) return launch_ring<16, 3>(seg, bytes_per_view, total_views, nbins, depth, flags, carve, counts, outside, st);
-    if (warps == 8) return launch_ring<8, 4>(seg, bytes_per_view, total_views, nbins, depth, flags, carve, counts, outside, st);
-    return launch_ring<12, 3>(seg, bytes_per_view, total_views, nbins, depth, flags, carve, counts, outside, st);
-  }
+  const bool want_ring = forced || (dc::stream_overlap() && total_views * bytes_per_view >= (int64_t)dc::sm_count() * (4 << 20));
+  if (want_ring && seg_dtype == DC_I64 && (uintptr_t)seg % 16 == 0 && bytes_per_view % 16 == 0 && ring_fits(bytes_per_view))
+    return launch_ring(seg, bytes_per_view, total_views, nbins, counts, outside, st);
   // CTAs of ~512 KB: enough of them per view to fill the machine a few times over when there are few views, and small
   // enough that the last wave does not leave SMs idle when there are many (4672 views of 2.4 MB: one CTA per view
   // ran at 6.9 TB/s, four at 7.3 TB/s)

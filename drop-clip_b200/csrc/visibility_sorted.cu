@@ -872,11 +872,8 @@ int dc_project_visibility_sorted(const double* points, const int64_t* point_off,
   if (smem > 48 * 1024) DC_CUDA(smem_attr.set(visibility_filter_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
   // two-stream mode: the instance-histogram ring kernel of the object branch (csrc/seg_table.cu) shares the SMs with this
   // kernel, and an SM cannot change its shared-memory carve-out while CTAs are resident: both ask for the same one
-  {
-    int carve = dc::stream_overlap() ? dc::kOverlapCarveoutPct : cudaSharedmemCarveoutDefault;
-    if (const char* e = getenv("DC_CARVEOUT_PCT")) carve = atoi(e);
-    DC_CUDA(carve_attr.set(visibility_filter_kernel, cudaFuncAttributePreferredSharedMemoryCarveout, carve));
-  }
+  DC_CUDA(carve_attr.set(visibility_filter_kernel, cudaFuncAttributePreferredSharedMemoryCarveout,
+                         dc::stream_overlap() ? dc::kOverlapCarveoutPct : cudaSharedmemCarveoutDefault));
   // The per-view constants live in the constant bank (uniform operands instead of 24 shared-memory
   // wavefronts per view and warp), refreshed per group of scenes by a device-to-device copy in
   // stream order. A group is at most one full wave of CTAs.

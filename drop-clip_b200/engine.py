@@ -307,7 +307,7 @@ class PinnedStaging:
         ranks = max(1, int(os.environ.get("LOCAL_WORLD_SIZE", "1") or 1))
         return max(1, min(16, cores // ranks))
 
-    def upload_list(self, arrays, dtype: torch.dtype, item_shape, group_bytes: int = int(os.environ.get("DC_UPLOAD_GROUP_MB", "32")) << 20,
+    def upload_list(self, arrays, dtype: torch.dtype, item_shape, group_bytes: int = 32 << 20,
                     narrow_to_u8: bool = False):
         """Stacks a list of equally-shaped host arrays straight into one pinned buffer and uploads it
         group by group, so the H2D copy of group g overlaps the host copy of group g+1. Contiguous
@@ -449,7 +449,7 @@ class FusionEngine:
         self.device = torch.device(device)
         self.launches = 0  # kernels launched by this engine (bench.py's gpu_launches)
         # object-level similarity weights below this are re-evaluated in fp64 (dc_view_weights); inf = every row
-        self.refine_below = float(os.environ.get("DC_REFINE_BELOW", "0.02"))
+        self.refine_below = 0.02
         self.profile: Optional[Dict[str, list]] = None  # name -> [(start_event, end_event)] when enabled
         # object branch and visibility branch of fuse_object_level on two streams (DC_OVERLAP=0: one stream)
         self._side: Dict[Optional[int], "torch.cuda.Stream"] = {}
@@ -766,7 +766,7 @@ class FusionEngine:
         key = torch.device(device).index
         if key not in self._side:
             # high priority: the object branch ends in a chain of small kernels that should not queue behind filter CTAs
-            self._side[key] = torch.cuda.Stream(device=device, priority=int(os.environ.get("DC_SIDE_PRIORITY", "-1")))
+            self._side[key] = torch.cuda.Stream(device=device, priority=-1)
             self._events[key] = (torch.cuda.Event(), torch.cuda.Event())
         return self._side[key]
 
@@ -861,7 +861,7 @@ class FusionEngine:
             x_hi, x_lo = planes[0], planes[1]
             check(self.lib.dc_row_normalize(ptr(feats), code, n, dim, int(normalize), ptr(x_hi), ptr(x_lo), current_stream()))
         else:
-            x_hi, x_lo = feats, None  # fp16 rows are normalised in place inside dc_ground (fused into the GEMM kernel)
+            x_hi, x_lo = feats, None  # fp16 rows are normalised in place by dc_ground (a separate pass before the GEMM)
         t32 = text.to(torch.float32).contiguous()
         tplanes = torch.empty((2, p, dim), dtype=torch.float16, device=dev)
         t_lo = tplanes[1] if text.dtype == torch.float32 else None

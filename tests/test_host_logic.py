@@ -77,6 +77,24 @@ def test_product_package_never_imports_the_oracle():
             assert not re.search(r"^\s*(from|import)\s+oracle\b", src, flags=re.M), fn
 
 
+def test_environment_reaches_only_the_known_switches():
+    """Launch sequences and results follow from the arguments: the library's only environment read is the DC_SEG_MODE
+    test seam, and the package reads DC_OVERLAP (INTEGRATION.md) and DC_PIXEL_PATH (the pixel path's A/B seam)."""
+    csrc = os.path.join(ROOT, "drop-clip_b200", "csrc")
+    reads = []
+    for fn in sorted(os.listdir(csrc)):
+        if ".cu" in fn:
+            reads += re.findall(r"\bgetenv\s*\(\s*([^)]*)\)", open(os.path.join(csrc, fn)).read())
+    assert reads == ['"DC_SEG_MODE"'], reads
+    pkg = os.path.join(ROOT, "drop-clip_b200")
+    names = set()
+    for fn in os.listdir(pkg):
+        if fn.endswith(".py"):
+            src = open(os.path.join(pkg, fn)).read()
+            names |= set(re.findall(r"\b(?:os\.environ(?:\.get)?\s*[\[(]|os\.getenv\s*\()\s*[\"'](\w+)[\"']", src))
+    assert {n for n in names if n.startswith("DC_")} == {"DC_OVERLAP", "DC_PIXEL_PATH"}, names
+
+
 def test_batch_offsets_layout():
     from dropclip_b200.engine import SceneBatch
     off = SceneBatch.offsets_for([5, 0, 7], [2, 3, 1], [4, 4, 2], [3, 3, 1, 1, 1, 2])
