@@ -712,9 +712,14 @@ __global__ void init_minmax_kernel(float* m) {
   if (threadIdx.x == 0) { m[0] = INFINITY; m[1] = -INFINITY; m[2] = INFINITY; m[3] = -INFINITY; }
 }
 
+// blockIdx.y selects one of several rows of n values, each with its own 4 extrema (dc_predict_queries); a single-row
+// launch has gridDim.y == 1
 __global__ void __launch_bounds__(256) minmax_threshold_kernel(float* __restrict__ v, int64_t n, const float* __restrict__ mm,
                                                                int use_raw, float thr, int pred_from_thr,
                                                                uint8_t* __restrict__ pred) {
+  v += (int64_t)blockIdx.y * n;
+  mm += 4 * blockIdx.y;
+  if (pred) pred += (int64_t)blockIdx.y * n;
   const float mn = mm[0], mx = mm[1];
   const bool differ = use_raw ? (mm[3] != mm[2]) : (mx != mn);
   const float range = mx - mn;
@@ -725,6 +730,95 @@ __global__ void __launch_bounds__(256) minmax_threshold_kernel(float* __restrict
     if (pred_from_thr) pred[i] = x > thr ? 1 : 0;
   }
 }
+
+__global__ void init_query_minmax_kernel(float* m, int n_slots) {
+  for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < 4 * n_slots; i += gridDim.x * blockDim.x)
+    m[i] = (i & 1) ? -INFINITY : INFINITY;
+}
+
+// atomic_min_f / atomic_max_f skipped when a plain read already shows a value at least as extreme: the stored extremum
+// only moves outwards, so a value that does not beat a stale read cannot beat the current one (most warps, once the
+// extrema settle). NaN compares false and still takes the atomic, as in the epilogues.
+__device__ __forceinline__ void atomic_min_f_if(float* a, float v) {
+  if (!(v >= *(volatile float*)a)) atomic_min_f(a, v);
+}
+__device__ __forceinline__ void atomic_max_f_if(float* a, float v) {
+  if (!(v <= *(volatile float*)a)) atomic_max_f(a, v);
+}
+
+// Per-query scores from the raw similarity matrix S [n_points, n_prompts] (dc_predict_queries). Query q has the
+// positive column pos[q] and the negative columns neg_cols[neg_off[q] .. neg_off[q+1]) (m of them):
+//   RAW    (m == 0): v = S[n, pos]
+//   PAIRED (m >= 1): v = 1 / (m + sum_j exp((S[n, j] - S[n, pos]) / T)), NaN -> 0   (EpiGround's arithmetic)
+//   ARGMAX (m >= 1): v = S[n, pos] - mean_j S[n, j], pred = S[n, pos] >= max_j S[n, j] (the positive wins ties)
+// out v [n_queries, n_points]; minmax [4 * q]: min/max of v, min/max of S over {pos} + negatives.
+// A block stages `tile_rows` rows of S in shared memory (coalesced: the rows are contiguous in S; the row stride in
+// shared memory is odd, so 32 lanes reading one column of 32 rows hit 32 banks). Thread t owns row t % tile_rows for
+// the queries q0 + t / tile_rows, q0 + t / tile_rows + groups, ... of the block's query chunk; a warp holds 32 rows of
+// one query, so the stores of v are coalesced and the extrema reduce with shuffles. Consecutive blocks share a tile
+// (blockIdx.x = tile * n_chunks + chunk): the chunks re-read it from L2.
+template <int kMode>
+__global__ void __launch_bounds__(256) query_scores_kernel(const float* __restrict__ S, int64_t n_points, int n_prompts,
+                                                           const int* __restrict__ pos, const int* __restrict__ neg_off,
+                                                           const int* __restrict__ neg_cols, int n_queries, int tile_rows,
+                                                           int q_per_chunk, int n_chunks, float inv_temp, float* __restrict__ v,
+                                                           uint8_t* __restrict__ pred, float* __restrict__ minmax) {
+  extern __shared__ float s_tile[];
+  const int ld = n_prompts | 1;
+  const int64_t row0 = (int64_t)(blockIdx.x / n_chunks) * tile_rows;
+  const int chunk = blockIdx.x % n_chunks;
+  const int rows = (int)min((int64_t)tile_rows, n_points - row0);
+  const float* src = S + row0 * n_prompts;
+  for (int i = threadIdx.x; i < rows * n_prompts; i += blockDim.x) {
+    const int r = i / n_prompts;
+    s_tile[r * ld + (i - r * n_prompts)] = src[i];
+  }
+  __syncthreads();
+  const int r = threadIdx.x % tile_rows;
+  const int groups = blockDim.x / tile_rows;
+  const bool have = r < rows;
+  const float* srow = s_tile + r * ld;
+  const int64_t n = row0 + r;
+  const float scale = inv_temp * 1.4426950408889634f;  // log2(e) / T
+  const int q_end = min(n_queries, (chunk + 1) * q_per_chunk);
+  for (int q = chunk * q_per_chunk + threadIdx.x / tile_rows; q < q_end; q += groups) {  // warp-uniform
+    const float sp = have ? srow[__ldg(pos + q)] : 0.f;
+    const int j0 = __ldg(neg_off + q), j1 = __ldg(neg_off + q + 1);
+    float raw_min = sp, raw_max = sp, acc[4] = {0.f, 0.f, 0.f, 0.f}, neg_max = -INFINITY;
+    const float bias = -sp * scale;
+    for (int j = j0; j < j1; ++j) {
+      const float s = srow[__ldg(neg_cols + j)];
+      raw_min = fminf(raw_min, s);
+      raw_max = fmaxf(raw_max, s);
+      if (kMode == DC_GROUND_PAIRED) acc[(j - j0) & 3] += ex2_approx(fmaf(s, scale, bias));
+      else { acc[(j - j0) & 3] += s; neg_max = fmaxf(neg_max, s); }
+    }
+    const float sum = (acc[0] + acc[1]) + (acc[2] + acc[3]);
+    const float m = (float)(j1 - j0);
+    float o = sp;
+    if (kMode == DC_GROUND_PAIRED) {
+      o = 1.f / (m + sum);
+      if (o != o) o = 0.f;  // nan_to_num
+    } else if (kMode == DC_GROUND_ARGMAX) {
+      o = sp - sum / m;
+    }
+    if (have) {
+      v[(int64_t)q * n_points + n] = o;
+      if (kMode == DC_GROUND_ARGMAX) pred[(int64_t)q * n_points + n] = (sp >= neg_max) ? 1 : 0;
+    }
+    float a = have ? o : INFINITY, b = have ? o : -INFINITY, c = have ? raw_min : INFINITY, d = have ? raw_max : -INFINITY;
+    a = dc::warp_min(a); b = dc::warp_max(b); c = dc::warp_min(c); d = dc::warp_max(d);
+    if ((threadIdx.x & 31) == 0) {
+      float* mm = minmax + 4 * q;
+      if (a != INFINITY) atomic_min_f_if(mm + 0, a);
+      if (b != -INFINITY) atomic_max_f_if(mm + 1, b);
+      if (c != INFINITY) atomic_min_f_if(mm + 2, c);
+      if (d != -INFINITY) atomic_max_f_if(mm + 3, d);
+    }
+  }
+}
+
+constexpr int kQueryMaxPrompts = 1536;  // dc_predict_queries: 32 staged rows of S, 32 * 1537 * 4 = 197 KB of shared memory
 
 template <class Epi>
 int launch_bn(int bn, const void* a_hi, const void* a_lo, int64_t a_rows, const void* b_hi, const void* b_lo, int64_t b_rows,
@@ -987,6 +1081,142 @@ int dc_predict(void* feats, int feat_dtype, int64_t n_points, const void* text, 
   // the arg-max prediction the epilogue wrote
   return dc_minmax_threshold(out, n_points, minmax, mode == DC_GROUND_ARGMAX ? 1 : 0, threshold,
                              mode == DC_GROUND_ARGMAX ? 0 : 1, pred, stream);
+}
+
+}  // extern "C"
+
+namespace {
+
+struct QueryWorkspace {
+  size_t minmax, csr, t_planes, x_planes, sims, total;
+};
+
+QueryWorkspace query_layout(int64_t n_points, int n_prompts, int n_queries, int64_t n_neg_total, int dim, int feat_dtype,
+                            int text_dtype) {
+  QueryWorkspace w{};
+  size_t off = 0;
+  w.minmax = off; off += align_up(sizeof(float) * 4 * ((size_t)n_queries + 1), 256);  // + the GEMM's unused extrema
+  w.csr = off; off += align_up(sizeof(int) * (2 * (size_t)n_queries + 1 + (size_t)n_neg_total), 256);
+  w.t_planes = off; if (text_dtype == DC_F32) off += 2 * align_up((size_t)n_prompts * dim * 2, 256);
+  w.x_planes = off; if (feat_dtype == DC_F32) off += 2 * align_up((size_t)(n_points > 0 ? n_points : 1) * dim * 2, 256);
+  w.sims = off; off += align_up((size_t)(n_points > 0 ? n_points : 1) * n_prompts * sizeof(float), 256);
+  w.total = off;
+  return w;
+}
+
+}  // namespace
+
+extern "C" {
+
+size_t dc_predict_queries_workspace(int64_t n_points, int n_prompts, int n_queries, int64_t n_neg_total, int dim,
+                                    int feat_dtype, int text_dtype) {
+  return query_layout(n_points, n_prompts, n_queries, n_neg_total, dim, feat_dtype, text_dtype).total;
+}
+
+int dc_predict_queries(void* feats, int feat_dtype, int64_t n_points, const void* text, int text_dtype, int n_prompts,
+                       int dim, const int32_t* pos, const int32_t* neg_off, const int32_t* neg_cols, int n_queries, int mode,
+                       float softmax_temp, int normalize, float threshold, float* out, uint8_t* pred, void* workspace,
+                       size_t workspace_bytes, dc_stream_t stream) {
+  DC_CHECK_ARG(text && pos && neg_off && workspace, "dc_predict_queries: null pointer argument");
+  DC_CHECK_ARG(n_points <= 0 || (feats && out && pred), "dc_predict_queries: null pointer argument");  // empty tensors have none
+  DC_CHECK_ARG(feat_dtype == DC_F16 || feat_dtype == DC_F32, "dc_predict_queries: features must be fp16 or fp32");
+  DC_CHECK_ARG(text_dtype == DC_F16 || text_dtype == DC_F32, "dc_predict_queries: prompt embeddings must be fp16 or fp32");
+  DC_CHECK_ARG(mode == DC_GROUND_RAW || mode == DC_GROUND_PAIRED || mode == DC_GROUND_ARGMAX, "dc_predict_queries: bad mode");
+  DC_CHECK_ARG(n_queries >= 1 && n_queries <= 65535, "dc_predict_queries: 1..65535 queries (got %d)", n_queries);
+  DC_CHECK_ARG(n_prompts >= 1 && n_prompts <= kQueryMaxPrompts, "dc_predict_queries: 1..%d prompts (got %d)", kQueryMaxPrompts,
+               n_prompts);
+  DC_CHECK_ARG(dim > 0 && dim % 64 == 0, "dc_predict_queries: feature dim must be a multiple of 64 (got %d)", dim);
+  DC_CHECK_ARG(n_points < (1ll << 31), "dc_predict_queries: too many points for one call");
+  DC_CHECK_ARG(((uintptr_t)workspace & 255) == 0, "dc_predict_queries: workspace must be 256-byte aligned");
+  // the column table lives in host memory: checked here, then copied into the workspace
+  DC_CHECK_ARG(neg_off[0] == 0, "dc_predict_queries: neg_off[0] must be 0");
+  for (int q = 0; q < n_queries; ++q) {
+    const int m = neg_off[q + 1] - neg_off[q];
+    DC_CHECK_ARG(pos[q] >= 0 && pos[q] < n_prompts, "dc_predict_queries: query %d: positive column %d outside [0, %d)", q,
+                 pos[q], n_prompts);
+    DC_CHECK_ARG(m >= 0, "dc_predict_queries: neg_off must not decrease (query %d)", q);
+    DC_CHECK_ARG(mode != DC_GROUND_RAW || m == 0, "dc_predict_queries: raw mode is the no-negatives case (query %d has %d)", q, m);
+    DC_CHECK_ARG(mode == DC_GROUND_RAW || m >= 1, "dc_predict_queries: paired/argmax need a negative for every query (query %d)", q);
+  }
+  const int64_t n_neg = neg_off[n_queries];
+  DC_CHECK_ARG(n_neg == 0 || neg_cols, "dc_predict_queries: null pointer argument");
+  for (int64_t j = 0; j < n_neg; ++j)
+    DC_CHECK_ARG(neg_cols[j] >= 0 && neg_cols[j] < n_prompts, "dc_predict_queries: negative column %d outside [0, %d)",
+                 neg_cols[j], n_prompts);
+  const QueryWorkspace w = query_layout(n_points, n_prompts, n_queries, n_neg, dim, feat_dtype, text_dtype);
+  if (workspace_bytes < w.total)
+    return dc::fail(DC_ERR_WORKSPACE, "dc_predict_queries: workspace %zu < %zu", workspace_bytes, w.total);
+  cudaStream_t st = dc::as_stream(stream);
+  uint8_t* ws = static_cast<uint8_t*>(workspace);
+  float* minmax = reinterpret_cast<float*>(ws + w.minmax);
+  init_query_minmax_kernel<<<1, 256, 0, st>>>(minmax, n_queries + 1);
+  DC_LAUNCH_CHECK();
+  if (n_points <= 0) return DC_OK;
+  int* d_pos = reinterpret_cast<int*>(ws + w.csr);
+  int* d_off = d_pos + n_queries;
+  int* d_cols = d_off + n_queries + 1;
+  DC_CUDA(cudaMemcpyAsync(d_pos, pos, sizeof(int) * n_queries, cudaMemcpyHostToDevice, st));
+  DC_CUDA(cudaMemcpyAsync(d_off, neg_off, sizeof(int) * (n_queries + 1), cudaMemcpyHostToDevice, st));
+  if (n_neg) DC_CUDA(cudaMemcpyAsync(d_cols, neg_cols, sizeof(int) * n_neg, cudaMemcpyHostToDevice, st));
+  // prologue of dc_predict: operand planes of fp32 prompts and fp32 features (normalised in place when asked); fp16
+  // features are normalised in place by dc_ground
+  int rc;
+  const void *t_hi = text, *t_lo = nullptr;
+  if (text_dtype == DC_F32) {
+    const size_t pb = align_up((size_t)n_prompts * dim * 2, 256);
+    if ((rc = launch_row_normalize(const_cast<void*>(text), DC_F32, n_prompts, dim, 0, false, ws + w.t_planes,
+                                   ws + w.t_planes + pb, st)))
+      return rc;
+    t_hi = ws + w.t_planes;
+    t_lo = ws + w.t_planes + pb;
+  }
+  const void *x_hi = feats, *x_lo = nullptr;
+  if (feat_dtype == DC_F32) {
+    const size_t xb = align_up((size_t)n_points * dim * 2, 256);
+    if ((rc = launch_row_normalize(feats, DC_F32, n_points, dim, normalize, true, ws + w.x_planes, ws + w.x_planes + xb, st)))
+      return rc;
+    x_hi = ws + w.x_planes;
+    x_lo = ws + w.x_planes + xb;
+  }
+  // S = X . T^T once, every distinct prompt a column
+  float* sims = reinterpret_cast<float*>(ws + w.sims);
+  if ((rc = dc_ground(x_hi, x_lo, n_points, t_hi, t_lo, n_prompts, dim, DC_GROUND_RAW, softmax_temp,
+                      (feat_dtype == DC_F16 && normalize) ? 1 : 0, sims, n_prompts, nullptr, nullptr,
+                      minmax + 4 * n_queries, nullptr, 0, stream)))
+    return rc;
+  // rows of S per block: as many as fit 48 KB of shared memory, 32 to 256
+  const int ld = n_prompts | 1;
+  int tile_rows = 256;
+  while (tile_rows > 32 && (size_t)tile_rows * ld * sizeof(float) > 48 * 1024) tile_rows >>= 1;
+  const size_t smem = (size_t)tile_rows * ld * sizeof(float);
+  const int64_t n_tiles = dc::ceil_div<int64_t>(n_points, tile_rows);
+  // few tiles (small scenes): split the queries over more blocks, up to 4 blocks per SM in all
+  const int want_chunks = (int)std::min<int64_t>(n_queries, dc::ceil_div<int64_t>(4 * (int64_t)dc::sm_count(), n_tiles));
+  const int q_per_chunk = (n_queries + want_chunks - 1) / want_chunks;
+  const int n_chunks = (n_queries + q_per_chunk - 1) / q_per_chunk;
+  DC_CHECK_ARG(n_tiles * n_chunks < (1ll << 31), "dc_predict_queries: too many blocks");
+  const float inv_temp = 1.0f / softmax_temp;
+  // the attribute belongs to the (function, device) pair: set for the device in use whenever a tile needs > 48 KB
+  const void* fn = mode == DC_GROUND_PAIRED ? (const void*)query_scores_kernel<DC_GROUND_PAIRED>
+                 : mode == DC_GROUND_ARGMAX ? (const void*)query_scores_kernel<DC_GROUND_ARGMAX>
+                                            : (const void*)query_scores_kernel<DC_GROUND_RAW>;
+  if (smem > 48 * 1024) DC_CUDA(cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+  const unsigned grid = (unsigned)(n_tiles * n_chunks);
+#define DC_QUERY_SCORES(M)                                                                                              \
+  query_scores_kernel<M><<<grid, 256, smem, st>>>(sims, n_points, n_prompts, d_pos, d_off, d_cols, n_queries, tile_rows, \
+                                                  q_per_chunk, n_chunks, inv_temp, out, pred, minmax)
+  if (mode == DC_GROUND_PAIRED) DC_QUERY_SCORES(DC_GROUND_PAIRED);
+  else if (mode == DC_GROUND_ARGMAX) DC_QUERY_SCORES(DC_GROUND_ARGMAX);
+  else DC_QUERY_SCORES(DC_GROUND_RAW);
+#undef DC_QUERY_SCORES
+  DC_LAUNCH_CHECK();
+  // per-query min-max (+ threshold), every query in one launch (blockIdx.y = query)
+  const int64_t blocks = dc::ceil_div<int64_t>(n_points, 256);
+  const int64_t per_query = std::max<int64_t>(1, dc::ceil_div<int64_t>((int64_t)dc::sm_count() * 8, n_queries));
+  minmax_threshold_kernel<<<dim3((unsigned)std::min(blocks, per_query), (unsigned)n_queries), 256, 0, st>>>(
+      out, n_points, minmax, mode == DC_GROUND_ARGMAX ? 1 : 0, threshold, mode == DC_GROUND_ARGMAX ? 0 : 1, pred);
+  DC_LAUNCH_CHECK();
+  return DC_OK;
 }
 
 int dc_minmax_threshold(float* values, int64_t n, const float* minmax, int use_raw_extrema_for_test, float threshold,

@@ -57,6 +57,28 @@ def _labels_as_int64(labels) -> np.ndarray:
     return arr.astype(np.int64)
 
 
+def query_csr(pos, neg_lists, n_prompts: int):
+    """Host column table of FusionEngine.predict_queries: (pos int32 [Q], neg_off int32 [Q+1], neg_cols int32) from
+    query q's positive row pos[q] and negative rows neg_lists[q] (neg_lists None: no query has negatives). Every index
+    must lie in [0, n_prompts): IndexError otherwise, before anything reaches the device."""
+    pos_a = np.asarray(list(pos), dtype=np.int64).reshape(-1)
+    q = pos_a.size
+    if neg_lists is None:
+        neg_lists = [()] * q
+    neg_lists = [np.asarray(list(x), dtype=np.int64).reshape(-1) for x in neg_lists]
+    if len(neg_lists) != q:
+        raise ValueError(f"{q} positive columns but {len(neg_lists)} negative lists")
+    cols = np.concatenate(neg_lists) if q else np.zeros(0, dtype=np.int64)
+    for what, a in (("positive", pos_a), ("negative", cols)):
+        bad = (a < 0) | (a >= n_prompts)
+        if bad.any():
+            raise IndexError(f"{what} prompt index {int(a[bad][0])} outside [0, {n_prompts})")
+    off = _prefix([x.size for x in neg_lists])
+    if off[-1] >= 2 ** 31:
+        raise ValueError("too many negative columns for one call")
+    return pos_a.astype(np.int32), off.astype(np.int32), cols.astype(np.int32)
+
+
 def intrinsic_matrix(intr: Dict[str, float]) -> np.ndarray:
     """utils/feature_fusion.py:35-40, always promoted to fp64 (K @ fp64 points is fp64 anyway)."""
     return np.asarray([[intr["fx"], 0, intr["cx"]], [0, intr["fy"], intr["cy"]], [0, 0, 1]], dtype=np.float64)
@@ -908,6 +930,43 @@ class FusionEngine:
                                   None, ctypes.c_void_p(ws.data_ptr() + shift), ws_bytes, current_stream()))
         self.launches += 3 + int(tcode == _lib.DC_F32) + int(fcode == _lib.DC_F32 or bool(normalize)) + (p + 255) // 256 - 1
         return out, pred
+
+    def predict_queries(self, feats: torch.Tensor, text: torch.Tensor, pos, neg_lists, mode: int, softmax_temp: float,
+                        normalize: bool, threshold: float):
+        """`predict` for Qq queries over one prompt table in one library call: the (N, P) similarity matrix is computed
+        once and every query is scored from its own columns. text (P,C) already normalised rows; pos[q] is query q's
+        positive row, neg_lists[q] its negative rows (None: no negatives, RAW). Row q of the result equals
+        predict(feats, text[[pos[q]] + neg_lists[q]], ...). Returns (score (Qq,N) fp32, pred (Qq,N) uint8)."""
+        n_prompts = int(text.shape[0])
+        pos_a, off, cols = query_csr(pos, neg_lists, n_prompts)
+        if (mode == _lib.DC_GROUND_RAW) != (cols.size == 0) or (mode != _lib.DC_GROUND_RAW and (np.diff(off) == 0).any()):
+            raise ValueError("raw mode takes no negatives; paired and argmax need negatives for every query")
+        n, dim = feats.shape
+        q = int(pos_a.size)
+        dev = feats.device
+        if q == 0:
+            return torch.empty((0, n), dtype=torch.float32, device=dev), torch.empty((0, n), dtype=torch.uint8, device=dev)
+        text = text.contiguous()
+        if text.dtype not in (torch.float16, torch.float32):
+            text = text.float()
+        fcode, tcode = _lib.torch_dtype_code(feats.dtype), _lib.torch_dtype_code(text.dtype)
+        ws_bytes = self.lib.dc_predict_queries_workspace(n, n_prompts, q, int(cols.size), dim, fcode, tcode)
+        res = torch.empty(max(q * n, 1) * 5 + 256, dtype=torch.uint8, device=dev)  # score fp32 + pred u8 in one allocation
+        ws = torch.empty(ws_bytes + 256, dtype=torch.uint8, device=dev)
+        shift = (-ws.data_ptr()) % 256
+        score = res[:4 * q * n].view(torch.float32).view(q, n)
+        pred = res[4 * max(q * n, 1):4 * max(q * n, 1) + q * n].view(q, n)
+        c_i32 = lambda a: a.ctypes.data_as(ctypes.c_void_p)  # noqa: E731
+        check(self.lib.dc_predict_queries(
+            ptr(feats), fcode, n, ptr(text), tcode, n_prompts, dim, c_i32(pos_a), c_i32(off), c_i32(cols) if cols.size else None,
+            q, mode, float(softmax_temp), int(bool(normalize)), float(threshold), ctypes.c_void_p(res.data_ptr()),
+            ctypes.c_void_p(res.data_ptr() + 4 * max(q * n, 1)), ctypes.c_void_p(ws.data_ptr() + shift), ws_bytes,
+            current_stream()))
+        if n > 0:
+            self.launches += 4 + int(tcode == _lib.DC_F32) + int(fcode == _lib.DC_F32 or bool(normalize)) + (n_prompts + 255) // 256 - 1
+        else:
+            self.launches += 1
+        return score, pred
 
     def minmax_threshold(self, values, minmax, use_raw: bool, threshold: float, want_pred: bool):
         pred = torch.empty(values.numel(), dtype=torch.uint8, device=values.device) if want_pred else None

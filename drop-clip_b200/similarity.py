@@ -19,6 +19,34 @@ from .engine import FusionEngine
 DEVICE = torch.device("cuda")  # the reference's expression always evaluates to 'cuda' (quirk q20)
 
 
+def query_columns(queries, qneg, generic):
+    """The prompt table of ClipSimilarity.predict_queries: (texts, pos, neg_lists). `texts` holds every distinct text
+    once (queries first, in order of appearance); query q's positive prompt is texts[pos[q]] and its negatives are
+    texts[j] for j in neg_lists[q], in the order predict(vis_feats, queries[q], qneg_q) would encode them:
+      qneg == "scene": qneg_q = [x for x in queries if x != queries[q]] (the reference's evaluation loops), `generic`
+                       when that is empty;
+      qneg a list:     the same negatives for every query, `generic` for [];
+      qneg None:       no negatives, neg_lists is None."""
+    texts, col = [], {}
+
+    def column(t):
+        if t not in col:
+            col[t] = len(texts)
+            texts.append(t)
+        return col[t]
+
+    pos = [column(t) for t in queries]
+    if qneg is None:
+        return texts, pos, None
+    if isinstance(qneg, str) and qneg == "scene":
+        per_query = [[x for x in queries if x != t] or list(generic) for t in queries]
+    else:
+        assert isinstance(qneg, list), "qneg argument should be list or None"
+        shared = list(qneg) if len(qneg) else list(generic)
+        per_query = [shared] * len(queries)
+    return texts, pos, [[column(x) for x in negs] for negs in per_query]
+
+
 
 def _load_clip(model_name, device):
     """The reference imports its vendored CLIP (`models.features.clip`); use it when importable."""
@@ -122,6 +150,40 @@ class ClipSimilarity(object):
                 raise IndexError("too many indices for tensor of dimension 1")  # reference behaviour (q18)
             out, pred = eng.predict(vis_feats, text, _lib.DC_GROUND_ARGMAX, self.SOFTMAX_TEMP, bool(norm_vis_feat), threshold)
             return pred.view(torch.bool), out
+
+    @torch.no_grad()
+    def predict_queries(self, vis_feats, queries, qneg="scene", norm_vis_feat=None, method=None, threshold=None):
+        """`predict` for every text query of a scene in one library call. Returns (pred (Qq,N) bool, sims (Qq,N) fp32):
+        row q is predict(vis_feats.clone(), queries[q], qneg_q, norm_vis_feat, method, threshold) flattened to (N,), with
+        qneg_q = every other query text for qneg == "scene" (the reference's evaluation loops, tools/validate_upper_bound.py
+        :200-218; the generic negatives when there is none), the same list for every query when qneg is a list, no
+        negatives for None. Every distinct text is encoded once, the features are normalised in place once and
+        multiplied with the prompt rows once. None where predict returns None."""
+        method = method or self.method
+        threshold = threshold or self.threshold
+        norm_vis_feat = norm_vis_feat or self.norm_vis_feat
+        self._check_feats(vis_feats)
+        queries = list(queries)
+        texts, pos, negs = query_columns(queries, qneg, self.NEGATIVE_PROMPT_GENERIC)
+        if negs is None:
+            mode = _lib.DC_GROUND_RAW
+        elif method == "paired":
+            mode = _lib.DC_GROUND_PAIRED
+        elif method == "argmax":
+            mode = _lib.DC_GROUND_ARGMAX
+        else:
+            return None  # predict falls off the end of its if/elif chain
+        n = vis_feats.shape[0]
+        if mode == _lib.DC_GROUND_ARGMAX and n == 1 and queries:
+            raise IndexError("too many indices for tensor of dimension 1")  # predict's behaviour (q18)
+        if not queries:
+            return (torch.empty((0, n), dtype=torch.bool, device=vis_feats.device),
+                    torch.empty((0, n), dtype=torch.float32, device=vis_feats.device))
+        text = self.model.encode_text(self._tok(texts).to(self.device))
+        text /= text.norm(dim=-1, keepdim=True)
+        score, pred = self._eng().predict_queries(vis_feats, text.to(vis_feats.device), pos, negs, mode, self.SOFTMAX_TEMP,
+                                                  bool(norm_vis_feat), threshold)
+        return pred.view(torch.bool), score
 
 
 # ---------------------------------------------------------------------- a18

@@ -368,6 +368,25 @@ DC_API size_t dc_predict_workspace(int64_t n_points, int n_prompts, int dim, int
 DC_API int dc_predict(void* feats, int feat_dtype, int64_t n_points, const void* text, int text_dtype, int n_prompts, int dim,
                int mode, float softmax_temp, int normalize, float threshold, float* out, uint8_t* pred,
                float** minmax_out, void* workspace, size_t workspace_bytes, dc_stream_t stream);
+/* ClipSimilarity.predict for every text query of a scene in ONE call: the features are normalised (when `normalize`)
+ * and multiplied with the prompt rows once, S = X . T^T [n_points, n_prompts] (dc_ground, RAW), then each query is scored
+ * from its own columns of S, with its own min-max and threshold. Row q of the result equals dc_predict on the prompt rows
+ * [pos[q], neg_cols[neg_off[q]], ..., neg_cols[neg_off[q+1] - 1]].
+ *   feats [n_points, dim] fp16/fp32 (normalised in place when `normalize`), text [n_prompts, dim] fp16/fp32 rows already
+ *   L2-normalised, each distinct prompt once; n_prompts <= 1536. feats, out and pred may be NULL when n_points == 0.
+ *   pos [n_queries], neg_off [n_queries + 1], neg_cols [neg_off[n_queries]] int32 in HOST memory: query q's positive
+ *   column and its negative columns (CSR; repeats allowed). Checked on the host (every column in [0, n_prompts); RAW:
+ *   no query has negatives; PAIRED / ARGMAX: every query has one at least) and copied into the workspace by
+ *   cudaMemcpyAsync, so pageable arrays may be reused when the call returns.
+ *   out [n_queries, n_points] fp32 = the min-max normalised scores, pred [n_queries, n_points] uint8 (score > threshold,
+ *   or argmax == 0).
+ *   workspace: 256-byte aligned, dc_predict_queries_workspace() bytes (S alone is 4 * n_points * n_prompts). */
+DC_API size_t dc_predict_queries_workspace(int64_t n_points, int n_prompts, int n_queries, int64_t n_neg_total, int dim,
+                                           int feat_dtype, int text_dtype);
+DC_API int dc_predict_queries(void* feats, int feat_dtype, int64_t n_points, const void* text, int text_dtype, int n_prompts,
+                              int dim, const int32_t* pos, const int32_t* neg_off, const int32_t* neg_cols, int n_queries,
+                              int mode, float softmax_temp, int normalize, float threshold, float* out, uint8_t* pred,
+                              void* workspace, size_t workspace_bytes, dc_stream_t stream);
 
 /* Global min-max normalisation + threshold (models/similarity.py:83-88, :95-98):
  * values <- (v - min)/(max - min) (or v / max when the raw extrema coincide), pred = values > thr
