@@ -69,6 +69,9 @@ SIGNATURES = {
     "dc_predict_queries_workspace": (c_size_t, [c_int64, c_int, c_int, c_int64, c_int, c_int, c_int]),
     "dc_predict_queries": (c_int, [P, c_int, c_int64, P, c_int, c_int, c_int, P, P, P, c_int, c_int, c_float, c_int, c_float, P,
                                    P, P, c_size_t, P]),
+    "dc_predict_many_workspace": (c_size_t, [c_int, P, P, P, c_int64, c_int, c_int, c_int]),
+    "dc_predict_many": (c_int, [P, c_int, P, c_int, c_int, c_int, P, P, P, P, P, P, c_int, c_float, c_int, c_float, P, P, P,
+                                c_size_t, P]),
     "dc_minmax_threshold": (c_int, [P, c_int64, P, c_int, c_float, c_int, P, P]),
     "dc_backproject": (c_int, [P, c_int, c_int, c_int, P, c_int, c_int, P, P, P]),
     "dc_points_to_pixels": (c_int, [P, c_int64, P, P, P]),

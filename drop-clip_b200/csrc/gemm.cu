@@ -3,7 +3,9 @@
 // Reference: utils/feature_fusion.py:311-313 (feat_v_norm @ query.T), models/similarity.py:28-101
 // (vis_feats @ text.T, paired softmax, min-max, threshold), engine/distil.py:244-246.
 #include <algorithm>
+#include <cstring>
 #include <mutex>
+#include <vector>
 
 #include "gemm.cuh"
 
@@ -712,14 +714,20 @@ __global__ void init_minmax_kernel(float* m) {
   if (threadIdx.x == 0) { m[0] = INFINITY; m[1] = -INFINITY; m[2] = INFINITY; m[3] = -INFINITY; }
 }
 
-// blockIdx.y selects one of several rows of n values, each with its own 4 extrema (dc_predict_queries); a single-row
-// launch has gridDim.y == 1
+// A single-row launch (gridDim.y == 1, no row table) normalises v [n] with the extrema mm [4]. With `row_off`, blockIdx.y
+// selects query row y = v [row_off[y], row_off[y + 1]) with its own extrema mm [4 * y] (dc_predict_queries,
+// dc_predict_many); `n` is then unused.
 __global__ void __launch_bounds__(256) minmax_threshold_kernel(float* __restrict__ v, int64_t n, const float* __restrict__ mm,
                                                                int use_raw, float thr, int pred_from_thr,
-                                                               uint8_t* __restrict__ pred) {
-  v += (int64_t)blockIdx.y * n;
-  mm += 4 * blockIdx.y;
-  if (pred) pred += (int64_t)blockIdx.y * n;
+                                                               uint8_t* __restrict__ pred,
+                                                               const int64_t* __restrict__ row_off = nullptr) {
+  if (row_off) {
+    const int64_t o = row_off[blockIdx.y];
+    n = row_off[blockIdx.y + 1] - o;
+    v += o;
+    mm += 4 * blockIdx.y;
+    if (pred) pred += o;
+  }
   const float mn = mm[0], mx = mm[1];
   const bool differ = use_raw ? (mm[3] != mm[2]) : (mx != mn);
   const float range = mx - mn;
@@ -746,42 +754,63 @@ __device__ __forceinline__ void atomic_max_f_if(float* a, float v) {
   if (!(v <= *(volatile float*)a)) atomic_max_f(a, v);
 }
 
-// Per-query scores from the raw similarity matrix S [n_points, n_prompts] (dc_predict_queries). Query q has the
-// positive column pos[q] and the negative columns neg_cols[neg_off[q] .. neg_off[q+1]) (m of them):
+// One scene of the scoring tables (dc_predict_queries: one, dc_predict_many: one per scene of the batch).
+struct ScoreScene {
+  int64_t s_row;    // the scene's first row of S
+  int64_t out_off;  // start of the scene's [n_queries, n_points] block of v and pred
+  int n_points;
+  int n_prompts;    // the scene's columns of S: [0, n_prompts)
+  int q0;           // the scene's first query
+  int pad;
+};
+// One block of query_scores_kernel: rows [row0, row0 + rows) of scene `scene` (scene-local), queries [q0, q1).
+struct ScoreBlock {
+  int scene, row0, rows, q0, q1;
+};
+
+// Per-query scores from the raw similarity matrix S [rows, s_ld] (dc_predict_queries, dc_predict_many). Query q of
+// scene s has the positive column pos[q] and the negative columns neg_cols[neg_off[q] .. neg_off[q+1]) (m of them),
+// all in [0, P_s):
 //   RAW    (m == 0): v = S[n, pos]
 //   PAIRED (m >= 1): v = 1 / (m + sum_j exp((S[n, j] - S[n, pos]) / T)), NaN -> 0   (EpiGround's arithmetic)
 //   ARGMAX (m >= 1): v = S[n, pos] - mean_j S[n, j], pred = S[n, pos] >= max_j S[n, j] (the positive wins ties)
-// out v [n_queries, n_points]; minmax [4 * q]: min/max of v, min/max of S over {pos} + negatives.
-// A block stages `tile_rows` rows of S in shared memory (coalesced: the rows are contiguous in S; the row stride in
-// shared memory is odd, so 32 lanes reading one column of 32 rows hit 32 banks). Thread t owns row t % tile_rows for
-// the queries q0 + t / tile_rows, q0 + t / tile_rows + groups, ... of the block's query chunk; a warp holds 32 rows of
-// one query, so the stores of v are coalesced and the extrema reduce with shuffles. Consecutive blocks share a tile
-// (blockIdx.x = tile * n_chunks + chunk): the chunks re-read it from L2.
+// v: scene s's block [Q_s, N_s] at out_off; minmax [4 * q]: min/max of v, min/max of S over {pos} + negatives.
+// A block stages its rows of S (at most `tile_rows`) in shared memory (coalesced: each row's P_s columns are
+// contiguous in S; the row stride in shared memory is odd, so 32 lanes reading one column of 32 rows hit 32 banks).
+// Thread t owns row t % tile_rows for the queries q0 + t / tile_rows, q0 + t / tile_rows + groups, ... of the block;
+// a warp holds 32 rows of one query, so the stores of v are coalesced and the extrema reduce with shuffles. The
+// blocks of one row tile are listed consecutively: the query chunks after the first re-read the tile from L2.
 template <int kMode>
-__global__ void __launch_bounds__(256) query_scores_kernel(const float* __restrict__ S, int64_t n_points, int n_prompts,
+__global__ void __launch_bounds__(256) query_scores_kernel(const float* __restrict__ S, int s_ld,
+                                                           const ScoreBlock* __restrict__ blocks,
+                                                           const ScoreScene* __restrict__ scenes,
                                                            const int* __restrict__ pos, const int* __restrict__ neg_off,
-                                                           const int* __restrict__ neg_cols, int n_queries, int tile_rows,
-                                                           int q_per_chunk, int n_chunks, float inv_temp, float* __restrict__ v,
-                                                           uint8_t* __restrict__ pred, float* __restrict__ minmax) {
+                                                           const int* __restrict__ neg_cols, int tile_rows, float inv_temp,
+                                                           float* __restrict__ v, uint8_t* __restrict__ pred,
+                                                           float* __restrict__ minmax) {
   extern __shared__ float s_tile[];
+  const ScoreBlock blk = blocks[blockIdx.x];
+  const ScoreScene sc = scenes[blk.scene];
+  const int n_prompts = sc.n_prompts;
   const int ld = n_prompts | 1;
-  const int64_t row0 = (int64_t)(blockIdx.x / n_chunks) * tile_rows;
-  const int chunk = blockIdx.x % n_chunks;
-  const int rows = (int)min((int64_t)tile_rows, n_points - row0);
-  const float* src = S + row0 * n_prompts;
+  const int rows = blk.rows;
+  const float* src = S + (sc.s_row + blk.row0) * (int64_t)s_ld;
   for (int i = threadIdx.x; i < rows * n_prompts; i += blockDim.x) {
     const int r = i / n_prompts;
-    s_tile[r * ld + (i - r * n_prompts)] = src[i];
+    const int c = i - r * n_prompts;
+    s_tile[r * ld + c] = src[(int64_t)r * s_ld + c];
   }
   __syncthreads();
   const int r = threadIdx.x % tile_rows;
   const int groups = blockDim.x / tile_rows;
   const bool have = r < rows;
   const float* srow = s_tile + r * ld;
-  const int64_t n = row0 + r;
+  const int64_t n = blk.row0 + r;
   const float scale = inv_temp * 1.4426950408889634f;  // log2(e) / T
-  const int q_end = min(n_queries, (chunk + 1) * q_per_chunk);
-  for (int q = chunk * q_per_chunk + threadIdx.x / tile_rows; q < q_end; q += groups) {  // warp-uniform
+  v += sc.out_off - (int64_t)sc.q0 * sc.n_points;  // query q's row starts at q * n_points
+  if (kMode == DC_GROUND_ARGMAX) pred += sc.out_off - (int64_t)sc.q0 * sc.n_points;
+  const int64_t n_points = sc.n_points;
+  for (int q = blk.q0 + threadIdx.x / tile_rows; q < blk.q1; q += groups) {  // warp-uniform
     const float sp = have ? srow[__ldg(pos + q)] : 0.f;
     const int j0 = __ldg(neg_off + q), j1 = __ldg(neg_off + q + 1);
     float raw_min = sp, raw_max = sp, acc[4] = {0.f, 0.f, 0.f, 0.f}, neg_max = -INFINITY;
@@ -1087,21 +1116,205 @@ int dc_predict(void* feats, int feat_dtype, int64_t n_points, const void* text, 
 
 namespace {
 
-struct QueryWorkspace {
-  size_t minmax, csr, t_planes, x_planes, sims, total;
+// Host plan of the scoring pass of dc_predict_queries (one scene) and dc_predict_many (a batch): the workspace layout
+// and the device tables - query rows, column CSR, scenes, score blocks and (dc_predict_many) the GEMM's tile lists -
+// staged in one host buffer and copied into the workspace by one cudaMemcpyAsync. A scene without queries gets no
+// blocks, no tiles and no normalisation.
+struct ScorePlan {
+  size_t minmax, tables, t_planes, x_planes, sims, total;                          // workspace byte offsets
+  size_t t_qrow, t_pos, t_off, t_cols, t_scenes, t_blocks, t_counts, t_tiles, t_bytes;  // inside the table region
+  int n_queries = 0, minmax_slots = 0, max_prompts = 1, s_ld = 0, tile_rows = 0;  // max_prompts: over the scenes with queries
+  int64_t n_rows = 0, n_text_rows = 0, n_neg = 0, max_points = 0;  // max_points: over the scenes with queries
+  std::vector<int64_t> qrow_off;  // [n_queries + 1]: query q's row of v / pred
+  std::vector<ScoreScene> scenes;
+  std::vector<ScoreBlock> blocks;
+  std::vector<int4> tiles;                            // the column blocks' tile lists, one after the other
+  std::vector<int> tile_start, tile_count, tile_bn;   // per block of 256 prompt columns
 };
 
-QueryWorkspace query_layout(int64_t n_points, int n_prompts, int n_queries, int64_t n_neg_total, int dim, int feat_dtype,
-                            int text_dtype) {
-  QueryWorkspace w{};
+// tile_list: dc_predict_many's GEMM (explicit tiles, S row stride = the widest scene rounded up to 4); otherwise
+// dc_ground writes S [n_points, n_prompts] of the one scene densely. reverse: list the first column block's tiles last
+// to first (the rows normalised last are still in L2, as in dc_ground).
+ScorePlan score_plan(int n_scenes, const int64_t* point_off, const int32_t* prompt_off, const int32_t* query_off,
+                     int64_t n_neg, int dim, int feat_dtype, int text_dtype, bool tile_list, bool reverse) {
+  ScorePlan pl;
+  pl.n_rows = point_off[n_scenes];
+  pl.n_text_rows = prompt_off[n_scenes];
+  pl.n_queries = query_off[n_scenes];
+  pl.n_neg = n_neg;
+  int& max_prompts = pl.max_prompts;
+  int64_t out_off = 0;
+  for (int s = 0; s < n_scenes; ++s) {
+    const int64_t ns = point_off[s + 1] - point_off[s];
+    const int ps = prompt_off[s + 1] - prompt_off[s], qs = query_off[s + 1] - query_off[s];
+    pl.scenes.push_back(ScoreScene{point_off[s], out_off, (int)ns, ps, query_off[s], 0});
+    for (int q = 0; q < qs; ++q) pl.qrow_off.push_back(out_off + q * ns);
+    out_off += qs * ns;
+    if (qs > 0) {
+      max_prompts = std::max(max_prompts, ps);
+      pl.max_points = std::max(pl.max_points, ns);
+    }
+  }
+  pl.qrow_off.push_back(out_off);
+  pl.s_ld = tile_list ? (max_prompts + 3) / 4 * 4 : max_prompts;
+  // rows of S per block: as many as fit 48 KB of shared memory at the widest scene, 32 to 256
+  pl.tile_rows = 256;
+  while (pl.tile_rows > 32 && (size_t)pl.tile_rows * (max_prompts | 1) * sizeof(float) > 48 * 1024) pl.tile_rows >>= 1;
+  int64_t score_tiles = 0;
+  for (int s = 0; s < n_scenes; ++s)
+    if (query_off[s + 1] > query_off[s]) score_tiles += dc::ceil_div<int64_t>(point_off[s + 1] - point_off[s], pl.tile_rows);
+  // few row tiles (small scenes): split each scene's queries over more blocks, up to 4 blocks per SM in all
+  const int64_t want = score_tiles ? dc::ceil_div<int64_t>(4 * (int64_t)dc::sm_count(), score_tiles) : 1;
+  for (int s = 0; s < n_scenes; ++s) {
+    const int64_t ns = point_off[s + 1] - point_off[s];
+    const int qs = query_off[s + 1] - query_off[s], q0 = query_off[s];
+    if (qs == 0) continue;
+    const int q_per_chunk = (int)dc::ceil_div<int64_t>(qs, std::min<int64_t>(qs, want));
+    for (int64_t r0 = 0; r0 < ns; r0 += pl.tile_rows)
+      for (int c0 = 0; c0 < qs; c0 += q_per_chunk)
+        pl.blocks.push_back(ScoreBlock{s, (int)r0, (int)std::min<int64_t>(pl.tile_rows, ns - r0), q0 + c0,
+                                       q0 + std::min(qs, c0 + q_per_chunk)});
+  }
+  if (tile_list) {
+    for (int c0 = 0; c0 < max_prompts; c0 += 256) {
+      const int start = (int)pl.tiles.size();
+      int widest = 1;
+      for (int s = 0; s < n_scenes; ++s) {
+        const int ps = prompt_off[s + 1] - prompt_off[s];
+        if (query_off[s + 1] == query_off[s] || ps <= c0) continue;
+        const int cols = std::min(256, ps - c0);
+        widest = std::max(widest, cols);
+        for (int64_t r0 = point_off[s]; r0 < point_off[s + 1]; r0 += dc::gemm::kBlockM)
+          pl.tiles.push_back(make_int4((int)r0, prompt_off[s] + c0, (int)std::min<int64_t>(dc::gemm::kBlockM, point_off[s + 1] - r0),
+                                       cols));
+      }
+      if (reverse && c0 == 0) std::reverse(pl.tiles.begin() + start, pl.tiles.end());
+      pl.tile_start.push_back(start);
+      pl.tile_count.push_back((int)pl.tiles.size() - start);
+      pl.tile_bn.push_back(pick_bn(widest));
+    }
+  }
+  const size_t q = (size_t)pl.n_queries;
+  size_t t = 0;
+  pl.t_qrow = t; t += align_up(sizeof(int64_t) * (q + 1), 16);
+  pl.t_pos = t; t += align_up(sizeof(int) * q, 16);
+  pl.t_off = t; t += align_up(sizeof(int) * (q + 1), 16);
+  pl.t_cols = t; t += align_up(sizeof(int) * (size_t)n_neg, 16);
+  pl.t_scenes = t; t += align_up(sizeof(ScoreScene) * pl.scenes.size(), 16);
+  pl.t_blocks = t; t += align_up(sizeof(ScoreBlock) * pl.blocks.size(), 16);
+  pl.t_counts = t; t += align_up(sizeof(int) * pl.tile_count.size(), 16);
+  pl.t_tiles = t; t += sizeof(int4) * pl.tiles.size();
+  pl.t_bytes = t;
+  pl.minmax_slots = pl.n_queries + (tile_list ? 0 : 1);  // + dc_ground's extrema, unused
   size_t off = 0;
-  w.minmax = off; off += align_up(sizeof(float) * 4 * ((size_t)n_queries + 1), 256);  // + the GEMM's unused extrema
-  w.csr = off; off += align_up(sizeof(int) * (2 * (size_t)n_queries + 1 + (size_t)n_neg_total), 256);
-  w.t_planes = off; if (text_dtype == DC_F32) off += 2 * align_up((size_t)n_prompts * dim * 2, 256);
-  w.x_planes = off; if (feat_dtype == DC_F32) off += 2 * align_up((size_t)(n_points > 0 ? n_points : 1) * dim * 2, 256);
-  w.sims = off; off += align_up((size_t)(n_points > 0 ? n_points : 1) * n_prompts * sizeof(float), 256);
-  w.total = off;
-  return w;
+  pl.minmax = off; off += align_up(sizeof(float) * 4 * (size_t)pl.minmax_slots, 256);
+  pl.tables = off; off += align_up(t, 256);
+  pl.t_planes = off; if (text_dtype == DC_F32) off += 2 * align_up((size_t)pl.n_text_rows * dim * 2, 256);
+  pl.x_planes = off; if (feat_dtype == DC_F32) off += 2 * align_up((size_t)(pl.n_rows > 0 ? pl.n_rows : 1) * dim * 2, 256);
+  pl.sims = off; off += align_up((size_t)(pl.n_rows > 0 ? pl.n_rows : 1) * pl.s_ld * sizeof(float), 256);
+  pl.total = off;
+  return pl;
+}
+
+// The column tables live in host memory: query q of scene s has its positive and negative columns in [0, P_s).
+int check_columns(const char* fn, int n_scenes, const int32_t* prompt_off, const int32_t* query_off, const int32_t* pos,
+                  const int32_t* neg_off, const int32_t* neg_cols, int mode) {
+  DC_CHECK_ARG(neg_off[0] == 0, "%s: neg_off[0] must be 0", fn);
+  for (int s = 0; s < n_scenes; ++s) {
+    const int n_prompts = prompt_off[s + 1] - prompt_off[s];
+    for (int q = query_off[s]; q < query_off[s + 1]; ++q) {
+      const int m = neg_off[q + 1] - neg_off[q];
+      DC_CHECK_ARG(pos[q] >= 0 && pos[q] < n_prompts, "%s: query %d: positive column %d outside [0, %d)", fn, q, pos[q],
+                   n_prompts);
+      DC_CHECK_ARG(m >= 0, "%s: neg_off must not decrease (query %d)", fn, q);
+      DC_CHECK_ARG(mode != DC_GROUND_RAW || m == 0, "%s: raw mode is the no-negatives case (query %d has %d)", fn, q, m);
+      DC_CHECK_ARG(mode == DC_GROUND_RAW || m >= 1, "%s: paired/argmax need a negative for every query (query %d)", fn, q);
+    }
+  }
+  const int n_queries = query_off[n_scenes];
+  DC_CHECK_ARG(neg_off[n_queries] == 0 || neg_cols, "%s: null pointer argument", fn);
+  for (int s = 0; s < n_scenes; ++s) {
+    const int n_prompts = prompt_off[s + 1] - prompt_off[s];
+    for (int64_t j = neg_off[query_off[s]]; j < neg_off[query_off[s + 1]]; ++j)
+      DC_CHECK_ARG(neg_cols[j] >= 0 && neg_cols[j] < n_prompts, "%s: negative column %d outside [0, %d)", fn, neg_cols[j],
+                   n_prompts);
+  }
+  return DC_OK;
+}
+
+int stage_tables(const ScorePlan& pl, const int32_t* pos, const int32_t* neg_off, const int32_t* neg_cols, uint8_t* ws,
+                 cudaStream_t st) {
+  std::vector<uint8_t> h(pl.t_bytes);
+  auto put = [&](size_t at, const void* src, size_t bytes) {
+    if (bytes) memcpy(h.data() + at, src, bytes);
+  };
+  const size_t q = (size_t)pl.n_queries;
+  put(pl.t_qrow, pl.qrow_off.data(), sizeof(int64_t) * (q + 1));
+  put(pl.t_pos, pos, sizeof(int) * q);
+  put(pl.t_off, neg_off, sizeof(int) * (q + 1));
+  put(pl.t_cols, neg_cols, sizeof(int) * (size_t)pl.n_neg);
+  put(pl.t_scenes, pl.scenes.data(), sizeof(ScoreScene) * pl.scenes.size());
+  put(pl.t_blocks, pl.blocks.data(), sizeof(ScoreBlock) * pl.blocks.size());
+  put(pl.t_counts, pl.tile_count.data(), sizeof(int) * pl.tile_count.size());
+  put(pl.t_tiles, pl.tiles.data(), sizeof(int4) * pl.tiles.size());
+  // pageable source: cudaMemcpyAsync returns once it has staged the bytes, so `h` may go out of scope
+  DC_CUDA(cudaMemcpyAsync(ws + pl.tables, h.data(), pl.t_bytes, cudaMemcpyHostToDevice, st));
+  return DC_OK;
+}
+
+// Every query scored from its columns of S [n_rows, s_ld], then its min-max and threshold (one launch each).
+int score_queries(const ScorePlan& pl, uint8_t* ws, int mode, float softmax_temp, float threshold, float* out,
+                  uint8_t* pred, cudaStream_t st) {
+  if (pl.blocks.empty()) return DC_OK;
+  DC_CHECK_ARG(pl.blocks.size() < (1ull << 31), "too many score blocks for one launch");
+  const uint8_t* tb = ws + pl.tables;
+  const int64_t* qrow = reinterpret_cast<const int64_t*>(tb + pl.t_qrow);
+  const int* d_pos = reinterpret_cast<const int*>(tb + pl.t_pos);
+  const int* d_off = reinterpret_cast<const int*>(tb + pl.t_off);
+  const int* d_cols = reinterpret_cast<const int*>(tb + pl.t_cols);
+  const ScoreScene* scenes = reinterpret_cast<const ScoreScene*>(tb + pl.t_scenes);
+  const ScoreBlock* blocks = reinterpret_cast<const ScoreBlock*>(tb + pl.t_blocks);
+  const float* sims = reinterpret_cast<const float*>(ws + pl.sims);
+  float* minmax = reinterpret_cast<float*>(ws + pl.minmax);
+  const size_t smem = (size_t)pl.tile_rows * (pl.max_prompts | 1) * sizeof(float);
+  const float inv_temp = 1.0f / softmax_temp;
+  // the attribute belongs to the (function, device) pair: set for the device in use whenever a tile needs > 48 KB
+  const void* fn = mode == DC_GROUND_PAIRED ? (const void*)query_scores_kernel<DC_GROUND_PAIRED>
+                 : mode == DC_GROUND_ARGMAX ? (const void*)query_scores_kernel<DC_GROUND_ARGMAX>
+                                            : (const void*)query_scores_kernel<DC_GROUND_RAW>;
+  if (smem > 48 * 1024) DC_CUDA(cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+  const unsigned grid = (unsigned)pl.blocks.size();
+#define DC_QUERY_SCORES(M)                                                                                             \
+  query_scores_kernel<M><<<grid, 256, smem, st>>>(sims, pl.s_ld, blocks, scenes, d_pos, d_off, d_cols, pl.tile_rows, \
+                                                  inv_temp, out, pred, minmax)
+  if (mode == DC_GROUND_PAIRED) DC_QUERY_SCORES(DC_GROUND_PAIRED);
+  else if (mode == DC_GROUND_ARGMAX) DC_QUERY_SCORES(DC_GROUND_ARGMAX);
+  else DC_QUERY_SCORES(DC_GROUND_RAW);
+#undef DC_QUERY_SCORES
+  DC_LAUNCH_CHECK();
+  // per-query min-max (+ threshold), every query in one launch (blockIdx.y = query, its row from the table)
+  const int64_t blocks_x = dc::ceil_div<int64_t>(pl.max_points, 256);
+  const int64_t per_query = std::max<int64_t>(1, dc::ceil_div<int64_t>((int64_t)dc::sm_count() * 8, pl.n_queries));
+  minmax_threshold_kernel<<<dim3((unsigned)std::min(blocks_x, per_query), (unsigned)pl.n_queries), 256, 0, st>>>(
+      out, 0, minmax, mode == DC_GROUND_ARGMAX ? 1 : 0, threshold, mode == DC_GROUND_ARGMAX ? 0 : 1, pred, qrow);
+  DC_LAUNCH_CHECK();
+  return DC_OK;
+}
+
+// fp32 prompt rows: their fp16 hi/lo operand planes in the workspace; fp16 prompts are used as they are
+int prompt_planes(const ScorePlan& pl, const void* text, int text_dtype, int dim, uint8_t* ws, const void** t_hi,
+                  const void** t_lo, cudaStream_t st) {
+  *t_hi = text;
+  *t_lo = nullptr;
+  if (text_dtype != DC_F32) return DC_OK;
+  const size_t pb = align_up((size_t)pl.n_text_rows * dim * 2, 256);
+  int rc;
+  if ((rc = launch_row_normalize(const_cast<void*>(text), DC_F32, pl.n_text_rows, dim, 0, false, ws + pl.t_planes,
+                                 ws + pl.t_planes + pb, st)))
+    return rc;
+  *t_hi = ws + pl.t_planes;
+  *t_lo = ws + pl.t_planes + pb;
+  return DC_OK;
 }
 
 }  // namespace
@@ -1110,7 +1323,9 @@ extern "C" {
 
 size_t dc_predict_queries_workspace(int64_t n_points, int n_prompts, int n_queries, int64_t n_neg_total, int dim,
                                     int feat_dtype, int text_dtype) {
-  return query_layout(n_points, n_prompts, n_queries, n_neg_total, dim, feat_dtype, text_dtype).total;
+  const int64_t point_off[2] = {0, n_points > 0 ? n_points : 0};
+  const int32_t prompt_off[2] = {0, n_prompts}, query_off[2] = {0, n_queries};
+  return score_plan(1, point_off, prompt_off, query_off, n_neg_total, dim, feat_dtype, text_dtype, false, false).total;
 }
 
 int dc_predict_queries(void* feats, int feat_dtype, int64_t n_points, const void* text, int text_dtype, int n_prompts,
@@ -1128,95 +1343,138 @@ int dc_predict_queries(void* feats, int feat_dtype, int64_t n_points, const void
   DC_CHECK_ARG(dim > 0 && dim % 64 == 0, "dc_predict_queries: feature dim must be a multiple of 64 (got %d)", dim);
   DC_CHECK_ARG(n_points < (1ll << 31), "dc_predict_queries: too many points for one call");
   DC_CHECK_ARG(((uintptr_t)workspace & 255) == 0, "dc_predict_queries: workspace must be 256-byte aligned");
-  // the column table lives in host memory: checked here, then copied into the workspace
-  DC_CHECK_ARG(neg_off[0] == 0, "dc_predict_queries: neg_off[0] must be 0");
-  for (int q = 0; q < n_queries; ++q) {
-    const int m = neg_off[q + 1] - neg_off[q];
-    DC_CHECK_ARG(pos[q] >= 0 && pos[q] < n_prompts, "dc_predict_queries: query %d: positive column %d outside [0, %d)", q,
-                 pos[q], n_prompts);
-    DC_CHECK_ARG(m >= 0, "dc_predict_queries: neg_off must not decrease (query %d)", q);
-    DC_CHECK_ARG(mode != DC_GROUND_RAW || m == 0, "dc_predict_queries: raw mode is the no-negatives case (query %d has %d)", q, m);
-    DC_CHECK_ARG(mode == DC_GROUND_RAW || m >= 1, "dc_predict_queries: paired/argmax need a negative for every query (query %d)", q);
-  }
-  const int64_t n_neg = neg_off[n_queries];
-  DC_CHECK_ARG(n_neg == 0 || neg_cols, "dc_predict_queries: null pointer argument");
-  for (int64_t j = 0; j < n_neg; ++j)
-    DC_CHECK_ARG(neg_cols[j] >= 0 && neg_cols[j] < n_prompts, "dc_predict_queries: negative column %d outside [0, %d)",
-                 neg_cols[j], n_prompts);
-  const QueryWorkspace w = query_layout(n_points, n_prompts, n_queries, n_neg, dim, feat_dtype, text_dtype);
-  if (workspace_bytes < w.total)
-    return dc::fail(DC_ERR_WORKSPACE, "dc_predict_queries: workspace %zu < %zu", workspace_bytes, w.total);
+  const int64_t point_off[2] = {0, n_points > 0 ? n_points : 0};
+  const int32_t prompt_off[2] = {0, n_prompts}, query_off[2] = {0, n_queries};
+  int rc;
+  if ((rc = check_columns("dc_predict_queries", 1, prompt_off, query_off, pos, neg_off, neg_cols, mode))) return rc;
+  const ScorePlan pl = score_plan(1, point_off, prompt_off, query_off, neg_off[n_queries], dim, feat_dtype, text_dtype,
+                                  false, false);
+  if (workspace_bytes < pl.total)
+    return dc::fail(DC_ERR_WORKSPACE, "dc_predict_queries: workspace %zu < %zu", workspace_bytes, pl.total);
   cudaStream_t st = dc::as_stream(stream);
   uint8_t* ws = static_cast<uint8_t*>(workspace);
-  float* minmax = reinterpret_cast<float*>(ws + w.minmax);
-  init_query_minmax_kernel<<<1, 256, 0, st>>>(minmax, n_queries + 1);
+  float* minmax = reinterpret_cast<float*>(ws + pl.minmax);
+  init_query_minmax_kernel<<<1, 256, 0, st>>>(minmax, pl.minmax_slots);
   DC_LAUNCH_CHECK();
   if (n_points <= 0) return DC_OK;
-  int* d_pos = reinterpret_cast<int*>(ws + w.csr);
-  int* d_off = d_pos + n_queries;
-  int* d_cols = d_off + n_queries + 1;
-  DC_CUDA(cudaMemcpyAsync(d_pos, pos, sizeof(int) * n_queries, cudaMemcpyHostToDevice, st));
-  DC_CUDA(cudaMemcpyAsync(d_off, neg_off, sizeof(int) * (n_queries + 1), cudaMemcpyHostToDevice, st));
-  if (n_neg) DC_CUDA(cudaMemcpyAsync(d_cols, neg_cols, sizeof(int) * n_neg, cudaMemcpyHostToDevice, st));
+  if ((rc = stage_tables(pl, pos, neg_off, neg_cols, ws, st))) return rc;
   // prologue of dc_predict: operand planes of fp32 prompts and fp32 features (normalised in place when asked); fp16
   // features are normalised in place by dc_ground
-  int rc;
-  const void *t_hi = text, *t_lo = nullptr;
-  if (text_dtype == DC_F32) {
-    const size_t pb = align_up((size_t)n_prompts * dim * 2, 256);
-    if ((rc = launch_row_normalize(const_cast<void*>(text), DC_F32, n_prompts, dim, 0, false, ws + w.t_planes,
-                                   ws + w.t_planes + pb, st)))
-      return rc;
-    t_hi = ws + w.t_planes;
-    t_lo = ws + w.t_planes + pb;
-  }
+  const void *t_hi, *t_lo;
+  if ((rc = prompt_planes(pl, text, text_dtype, dim, ws, &t_hi, &t_lo, st))) return rc;
   const void *x_hi = feats, *x_lo = nullptr;
   if (feat_dtype == DC_F32) {
     const size_t xb = align_up((size_t)n_points * dim * 2, 256);
-    if ((rc = launch_row_normalize(feats, DC_F32, n_points, dim, normalize, true, ws + w.x_planes, ws + w.x_planes + xb, st)))
+    if ((rc = launch_row_normalize(feats, DC_F32, n_points, dim, normalize, true, ws + pl.x_planes, ws + pl.x_planes + xb, st)))
       return rc;
-    x_hi = ws + w.x_planes;
-    x_lo = ws + w.x_planes + xb;
+    x_hi = ws + pl.x_planes;
+    x_lo = ws + pl.x_planes + xb;
   }
   // S = X . T^T once, every distinct prompt a column
-  float* sims = reinterpret_cast<float*>(ws + w.sims);
+  float* sims = reinterpret_cast<float*>(ws + pl.sims);
   if ((rc = dc_ground(x_hi, x_lo, n_points, t_hi, t_lo, n_prompts, dim, DC_GROUND_RAW, softmax_temp,
                       (feat_dtype == DC_F16 && normalize) ? 1 : 0, sims, n_prompts, nullptr, nullptr,
                       minmax + 4 * n_queries, nullptr, 0, stream)))
     return rc;
-  // rows of S per block: as many as fit 48 KB of shared memory, 32 to 256
-  const int ld = n_prompts | 1;
-  int tile_rows = 256;
-  while (tile_rows > 32 && (size_t)tile_rows * ld * sizeof(float) > 48 * 1024) tile_rows >>= 1;
-  const size_t smem = (size_t)tile_rows * ld * sizeof(float);
-  const int64_t n_tiles = dc::ceil_div<int64_t>(n_points, tile_rows);
-  // few tiles (small scenes): split the queries over more blocks, up to 4 blocks per SM in all
-  const int want_chunks = (int)std::min<int64_t>(n_queries, dc::ceil_div<int64_t>(4 * (int64_t)dc::sm_count(), n_tiles));
-  const int q_per_chunk = (n_queries + want_chunks - 1) / want_chunks;
-  const int n_chunks = (n_queries + q_per_chunk - 1) / q_per_chunk;
-  DC_CHECK_ARG(n_tiles * n_chunks < (1ll << 31), "dc_predict_queries: too many blocks");
-  const float inv_temp = 1.0f / softmax_temp;
-  // the attribute belongs to the (function, device) pair: set for the device in use whenever a tile needs > 48 KB
-  const void* fn = mode == DC_GROUND_PAIRED ? (const void*)query_scores_kernel<DC_GROUND_PAIRED>
-                 : mode == DC_GROUND_ARGMAX ? (const void*)query_scores_kernel<DC_GROUND_ARGMAX>
-                                            : (const void*)query_scores_kernel<DC_GROUND_RAW>;
-  if (smem > 48 * 1024) DC_CUDA(cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-  const unsigned grid = (unsigned)(n_tiles * n_chunks);
-#define DC_QUERY_SCORES(M)                                                                                              \
-  query_scores_kernel<M><<<grid, 256, smem, st>>>(sims, n_points, n_prompts, d_pos, d_off, d_cols, n_queries, tile_rows, \
-                                                  q_per_chunk, n_chunks, inv_temp, out, pred, minmax)
-  if (mode == DC_GROUND_PAIRED) DC_QUERY_SCORES(DC_GROUND_PAIRED);
-  else if (mode == DC_GROUND_ARGMAX) DC_QUERY_SCORES(DC_GROUND_ARGMAX);
-  else DC_QUERY_SCORES(DC_GROUND_RAW);
-#undef DC_QUERY_SCORES
+  return score_queries(pl, ws, mode, softmax_temp, threshold, out, pred, st);
+}
+
+size_t dc_predict_many_workspace(int n_scenes, const int64_t* point_off, const int32_t* prompt_off, const int32_t* query_off,
+                                 int64_t n_neg_total, int dim, int feat_dtype, int text_dtype) {
+  if (n_scenes < 0 || (n_scenes > 0 && !(point_off && prompt_off && query_off))) return 0;
+  const int64_t zero64 = 0;
+  const int32_t zero32 = 0;
+  if (n_scenes == 0) return score_plan(0, &zero64, &zero32, &zero32, 0, dim, feat_dtype, text_dtype, true, false).total;
+  return score_plan(n_scenes, point_off, prompt_off, query_off, n_neg_total, dim, feat_dtype, text_dtype, true, false).total;
+}
+
+int dc_predict_many(void* feats, int feat_dtype, const void* text, int text_dtype, int dim, int n_scenes,
+                    const int64_t* point_off, const int32_t* prompt_off, const int32_t* query_off, const int32_t* pos,
+                    const int32_t* neg_off, const int32_t* neg_cols, int mode, float softmax_temp, int normalize,
+                    float threshold, float* out, uint8_t* pred, void* workspace, size_t workspace_bytes,
+                    dc_stream_t stream) {
+  DC_CHECK_ARG(n_scenes >= 0, "dc_predict_many: negative scene count");
+  if (n_scenes == 0) return DC_OK;
+  DC_CHECK_ARG(point_off && prompt_off && query_off && neg_off && workspace, "dc_predict_many: null pointer argument");
+  DC_CHECK_ARG(feat_dtype == DC_F16 || feat_dtype == DC_F32, "dc_predict_many: features must be fp16 or fp32");
+  DC_CHECK_ARG(text_dtype == DC_F16 || text_dtype == DC_F32, "dc_predict_many: prompt embeddings must be fp16 or fp32");
+  DC_CHECK_ARG(mode == DC_GROUND_RAW || mode == DC_GROUND_PAIRED || mode == DC_GROUND_ARGMAX, "dc_predict_many: bad mode");
+  DC_CHECK_ARG(dim > 0 && dim % 64 == 0, "dc_predict_many: feature dim must be a multiple of 64 (got %d)", dim);
+  DC_CHECK_ARG(((uintptr_t)workspace & 255) == 0, "dc_predict_many: workspace must be 256-byte aligned");
+  DC_CHECK_ARG(point_off[0] == 0 && prompt_off[0] == 0 && query_off[0] == 0, "dc_predict_many: offset tables must start at 0");
+  for (int s = 0; s < n_scenes; ++s) {
+    const int64_t ns = point_off[s + 1] - point_off[s];
+    const int ps = prompt_off[s + 1] - prompt_off[s], qs = query_off[s + 1] - query_off[s];
+    DC_CHECK_ARG(ns >= 0 && ps >= 0 && qs >= 0, "dc_predict_many: offset tables must not decrease (scene %d)", s);
+    DC_CHECK_ARG(ps <= kQueryMaxPrompts, "dc_predict_many: scene %d: 0..%d prompts (got %d)", s, kQueryMaxPrompts, ps);
+    DC_CHECK_ARG(qs == 0 || ps >= 1, "dc_predict_many: scene %d has queries but no prompts", s);
+  }
+  const int64_t n_rows = point_off[n_scenes];
+  const int n_queries = query_off[n_scenes];
+  DC_CHECK_ARG(n_rows < (1ll << 31), "dc_predict_many: too many points for one call (%lld)", (long long)n_rows);
+  DC_CHECK_ARG(n_queries <= 65535, "dc_predict_many: at most 65535 queries in all (got %d)", n_queries);
+  DC_CHECK_ARG(n_rows == 0 || feats, "dc_predict_many: null pointer argument");
+  DC_CHECK_ARG(prompt_off[n_scenes] == 0 || text, "dc_predict_many: null pointer argument");
+  int64_t n_cells = 0;
+  for (int s = 0; s < n_scenes; ++s)
+    n_cells += (int64_t)(query_off[s + 1] - query_off[s]) * (point_off[s + 1] - point_off[s]);
+  DC_CHECK_ARG(n_cells == 0 || (out && pred), "dc_predict_many: null pointer argument");
+  DC_CHECK_ARG(n_queries == 0 || pos, "dc_predict_many: null pointer argument");
+  int rc;
+  if ((rc = check_columns("dc_predict_many", n_scenes, prompt_off, query_off, pos, neg_off, neg_cols, mode))) return rc;
+  if (n_queries == 0) return DC_OK;
+  cudaStream_t st = dc::as_stream(stream);
+  const ScorePlan pl = score_plan(n_scenes, point_off, prompt_off, query_off, neg_off[n_queries], dim, feat_dtype,
+                                  text_dtype, true, feat_dtype == DC_F16 && normalize);
+  if (workspace_bytes < pl.total)
+    return dc::fail(DC_ERR_WORKSPACE, "dc_predict_many: workspace %zu < %zu", workspace_bytes, pl.total);
+  uint8_t* ws = static_cast<uint8_t*>(workspace);
+  float* minmax = reinterpret_cast<float*>(ws + pl.minmax);
+  init_query_minmax_kernel<<<1, 256, 0, st>>>(minmax, pl.minmax_slots);
   DC_LAUNCH_CHECK();
-  // per-query min-max (+ threshold), every query in one launch (blockIdx.y = query)
-  const int64_t blocks = dc::ceil_div<int64_t>(n_points, 256);
-  const int64_t per_query = std::max<int64_t>(1, dc::ceil_div<int64_t>((int64_t)dc::sm_count() * 8, n_queries));
-  minmax_threshold_kernel<<<dim3((unsigned)std::min(blocks, per_query), (unsigned)n_queries), 256, 0, st>>>(
-      out, n_points, minmax, mode == DC_GROUND_ARGMAX ? 1 : 0, threshold, mode == DC_GROUND_ARGMAX ? 0 : 1, pred);
-  DC_LAUNCH_CHECK();
-  return DC_OK;
+  if (pl.blocks.empty()) return DC_OK;  // every scene with queries is empty
+  if ((rc = stage_tables(pl, pos, neg_off, neg_cols, ws, st))) return rc;
+  const void *t_hi, *t_lo;
+  if ((rc = prompt_planes(pl, text, text_dtype, dim, ws, &t_hi, &t_lo, st))) return rc;
+  // the features of the scenes with queries, normalised in place (when asked) as dc_predict_queries does: fp32 rows
+  // also get their operand planes. One launch per run of consecutive such scenes (one launch when every scene has
+  // queries); the rows of a scene without queries stay untouched.
+  const size_t xb = align_up((size_t)n_rows * dim * 2, 256);
+  const size_t row_bytes = (size_t)dim * (feat_dtype == DC_F32 ? 4 : 2);
+  const void *x_hi = feats, *x_lo = nullptr;
+  if (feat_dtype == DC_F32) {
+    x_hi = ws + pl.x_planes;
+    x_lo = ws + pl.x_planes + xb;
+  }
+  if (feat_dtype == DC_F32 || normalize) {
+    for (int s = 0; s < n_scenes;) {
+      if (query_off[s + 1] == query_off[s]) { ++s; continue; }
+      int e = s + 1;
+      while (e < n_scenes && query_off[e + 1] > query_off[e]) ++e;
+      const int64_t r0 = point_off[s], rows = point_off[e] - r0;
+      uint8_t* hi = feat_dtype == DC_F32 ? ws + pl.x_planes + (size_t)r0 * dim * 2 : nullptr;
+      uint8_t* lo = feat_dtype == DC_F32 ? hi + xb : nullptr;
+      if ((rc = launch_row_normalize(static_cast<uint8_t*>(feats) + (size_t)r0 * row_bytes, feat_dtype, rows, dim, normalize,
+                                     true, hi, lo, st)))
+        return rc;
+      s = e;
+    }
+  }
+  // S = X . T^T of every scene with its own prompts: one tcgen05 GEMM per block of 256 prompt columns over the tile list
+  // (a tile = 128 rows of one scene x that scene's columns of the block), written once at the row stride s_ld
+  const int n_terms = x_lo ? 3 : (t_lo ? 2 : 1);
+  const uint8_t* tb = ws + pl.tables;
+  float* sims = reinterpret_cast<float*>(ws + pl.sims);
+  for (size_t cb = 0; cb < pl.tile_count.size(); ++cb) {
+    if (pl.tile_count[cb] == 0) continue;
+    Params p{reinterpret_cast<const int4*>(tb + pl.t_tiles) + pl.tile_start[cb],
+             reinterpret_cast<const int*>(tb + pl.t_counts) + cb, n_rows, 0, dim, n_terms, 0};
+    EpiStore epi{sims + 256 * cb, pl.s_ld};
+    if ((rc = launch_bn(pl.tile_bn[cb], x_hi, x_lo, n_rows, t_hi, t_lo, pl.n_text_rows, p, epi,
+                        pl.tile_count[cb], st)))
+      return rc;
+  }
+  return score_queries(pl, ws, mode, softmax_temp, threshold, out, pred, st);
 }
 
 int dc_minmax_threshold(float* values, int64_t n, const float* minmax, int use_raw_extrema_for_test, float threshold,

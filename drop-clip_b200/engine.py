@@ -968,6 +968,64 @@ class FusionEngine:
             self.launches += 1
         return score, pred
 
+    def predict_many(self, feats: torch.Tensor, counts, text: torch.Tensor, prompt_counts, pos, neg_lists, mode: int,
+                     softmax_temp: float, normalize: bool, threshold: float):
+        """`predict_queries` for every scene of a batch in one library call. feats (sum N, C) holds the scenes' rows in
+        scene order, counts[s] = N_s; text (sum P, C) the scenes' prompt blocks (already normalised rows),
+        prompt_counts[s] = P_s; pos[s] / neg_lists[s] (None: no negatives, RAW) index scene s's prompt block as in
+        predict_queries. Every index, count and mode rule is checked before anything reaches the device. Returns one
+        (score (Q_s, N_s) fp32, pred (Q_s, N_s) uint8) pair per scene, views into one score and one pred buffer; each
+        equals predict_queries(rows of scene s, text block of scene s, pos[s], neg_lists[s], ...)."""
+        counts = [int(c) for c in counts]
+        prompt_counts = [int(p) for p in prompt_counts]
+        s_n = len(counts)
+        if len(prompt_counts) != s_n or len(pos) != s_n or (neg_lists is not None and len(neg_lists) != s_n):
+            raise ValueError(f"{s_n} scenes but {len(prompt_counts)} prompt counts, {len(pos)} positive lists"
+                             + ("" if neg_lists is None else f", {len(neg_lists)} negative lists"))
+        if any(c < 0 for c in counts) or sum(counts) != feats.shape[0]:
+            raise ValueError(f"point counts {counts} do not sum to the {feats.shape[0]} feature rows")
+        if any(p < 0 for p in prompt_counts) or sum(prompt_counts) != text.shape[0]:
+            raise ValueError(f"prompt counts {prompt_counts} do not sum to the {text.shape[0]} prompt rows")
+        tables = [query_csr(pos[s], None if neg_lists is None else neg_lists[s], prompt_counts[s]) for s in range(s_n)]
+        for _, off, cols in tables:
+            raw = mode == _lib.DC_GROUND_RAW
+            if off.size > 1 and (raw != (cols.size == 0) or (not raw and (np.diff(off) == 0).any())):
+                raise ValueError("raw mode takes no negatives; paired and argmax need negatives for every query")
+        q_counts = [int(t[0].size) for t in tables]
+        dev = feats.device
+        cells = [q * n for q, n in zip(q_counts, counts)]
+        res = torch.empty(max(sum(cells), 1) * 5 + 256, dtype=torch.uint8, device=dev)  # score fp32 + pred u8 in one allocation
+        pred_base = 4 * max(sum(cells), 1)
+        out, at = [], 0
+        for q, n, c in zip(q_counts, counts, cells):
+            out.append((res[4 * at:4 * (at + c)].view(torch.float32).view(q, n), res[pred_base + at:pred_base + at + c].view(q, n)))
+            at += c
+        if s_n == 0 or sum(q_counts) == 0:
+            return out
+        n_total, dim = feats.shape
+        text = text.contiguous()
+        if text.dtype not in (torch.float16, torch.float32):
+            text = text.float()
+        point_off = _prefix(counts).astype(np.int64)
+        prompt_off = _prefix(prompt_counts).astype(np.int32)
+        query_off = _prefix(q_counts).astype(np.int32)
+        pos_a = np.concatenate([t[0] for t in tables]).astype(np.int32)
+        cols = np.concatenate([t[2] for t in tables]).astype(np.int32)
+        off = _prefix([int(t[1][-1]) for t in tables])
+        neg_off = np.concatenate([[0]] + [t[1][1:] + off[s] for s, t in enumerate(tables)]).astype(np.int32)
+        fcode, tcode = _lib.torch_dtype_code(feats.dtype), _lib.torch_dtype_code(text.dtype)
+        c_p = lambda a: a.ctypes.data_as(ctypes.c_void_p)  # noqa: E731
+        ws_bytes = self.lib.dc_predict_many_workspace(s_n, c_p(point_off), c_p(prompt_off), c_p(query_off), int(cols.size),
+                                                      dim, fcode, tcode)
+        ws = torch.empty(ws_bytes + 256, dtype=torch.uint8, device=dev)
+        shift = (-ws.data_ptr()) % 256
+        check(self.lib.dc_predict_many(
+            ptr(feats) if n_total else None, fcode, ptr(text) if text.shape[0] else None, tcode, dim, s_n, c_p(point_off),
+            c_p(prompt_off), c_p(query_off), c_p(pos_a), c_p(neg_off), c_p(cols) if cols.size else None, mode,
+            float(softmax_temp), int(bool(normalize)), float(threshold), ctypes.c_void_p(res.data_ptr()),
+            ctypes.c_void_p(res.data_ptr() + pred_base), ctypes.c_void_p(ws.data_ptr() + shift), ws_bytes, current_stream()))
+        return out
+
     def minmax_threshold(self, values, minmax, use_raw: bool, threshold: float, want_pred: bool):
         pred = torch.empty(values.numel(), dtype=torch.uint8, device=values.device) if want_pred else None
         check(self.lib.dc_minmax_threshold(ptr(values), values.numel(), ptr(minmax), int(use_raw), float(threshold),

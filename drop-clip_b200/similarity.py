@@ -47,6 +47,27 @@ def query_columns(queries, qneg, generic):
     return texts, pos, [[column(x) for x in negs] for negs in per_query]
 
 
+def batch_query_columns(scene_queries, qneg, generic):
+    """The prompt tables of ClipSimilarity.predict_many: (texts, gather, prompt_counts, pos, neg_lists). Scene s gets
+    the table query_columns(scene_queries[s], qneg, generic) = (texts_s, pos[s], neg_lists[s]), with pos[s] and
+    neg_lists[s] local to it; `texts` holds every distinct text of the batch once, in order of appearance, and the
+    scene tables one after the other are texts[gather[j]] (scene s: prompt_counts[s] = len(texts_s) entries). So one
+    encode_text of `texts` and one index_select with `gather` give every scene its prompt rows."""
+    texts, col = [], {}
+    gather, prompt_counts, pos, neg_lists = [], [], [], []
+    for queries in scene_queries:
+        texts_s, pos_s, negs_s = query_columns(list(queries), qneg, generic)
+        for t in texts_s:
+            if t not in col:
+                col[t] = len(texts)
+                texts.append(t)
+        gather += [col[t] for t in texts_s]
+        prompt_counts.append(len(texts_s))
+        pos.append(pos_s)
+        neg_lists.append(negs_s)
+    return texts, gather, prompt_counts, pos, neg_lists
+
+
 
 def _load_clip(model_name, device):
     """The reference imports its vendored CLIP (`models.features.clip`); use it when importable."""
@@ -184,6 +205,49 @@ class ClipSimilarity(object):
         score, pred = self._eng().predict_queries(vis_feats, text.to(vis_feats.device), pos, negs, mode, self.SOFTMAX_TEMP,
                                                   bool(norm_vis_feat), threshold)
         return pred.view(torch.bool), score
+
+    @torch.no_grad()
+    def predict_many(self, vis_feats, counts, queries, qneg="scene", norm_vis_feat=None, method=None, threshold=None):
+        """`predict_queries` for every scene of a batch in one library call. vis_feats (sum N, C) holds the scenes' rows
+        in scene order (a collated sparse batch), counts[s] = N_s, queries[s] the query texts of scene s; qneg applies to
+        every scene as in predict_queries. Returns one entry per scene: what predict_queries(rows of scene s,
+        queries[s], qneg, norm_vis_feat, method, threshold) returns, a (pred (Q_s, N_s) bool, sims (Q_s, N_s) fp32) pair
+        (views into one score and one pred buffer) or None for a method predict does not know.
+        Every distinct text of the batch is encoded in one encode_text call. The rows of the scenes with queries are
+        normalised in place once (a scene without queries is left as it is, as predict_queries leaves it).
+        Unlike a loop of predict_queries, which would have normalised the scenes before the failing one, every error
+        is raised before any row changes: IndexError when method == "argmax" and a scene with queries has one point,
+        RuntimeError for CPU or non-contiguous features, ValueError when counts do not sum to the rows."""
+        method = method or self.method
+        threshold = threshold or self.threshold
+        norm_vis_feat = norm_vis_feat or self.norm_vis_feat
+        self._check_feats(vis_feats)
+        counts = [int(c) for c in counts]
+        scene_queries = [list(q) for q in queries]
+        if len(scene_queries) != len(counts):
+            raise ValueError(f"{len(counts)} point counts but {len(scene_queries)} query lists")
+        if any(c < 0 for c in counts) or sum(counts) != vis_feats.shape[0]:
+            raise ValueError(f"point counts {counts} do not sum to the {vis_feats.shape[0]} feature rows")
+        texts, gather, prompt_counts, pos, negs = batch_query_columns(scene_queries, qneg, self.NEGATIVE_PROMPT_GENERIC)
+        if qneg is None:
+            mode = _lib.DC_GROUND_RAW
+        elif method == "paired":
+            mode = _lib.DC_GROUND_PAIRED
+        elif method == "argmax":
+            mode = _lib.DC_GROUND_ARGMAX
+        else:
+            return [None] * len(counts)  # predict falls off the end of its if/elif chain
+        if mode == _lib.DC_GROUND_ARGMAX and any(n == 1 and q for n, q in zip(counts, scene_queries)):
+            raise IndexError("too many indices for tensor of dimension 1")  # predict's behaviour (q18)
+        if texts:
+            emb = self.model.encode_text(self._tok(texts).to(self.device))
+            emb /= emb.norm(dim=-1, keepdim=True)
+            text = emb.index_select(0, torch.tensor(gather, dtype=torch.long, device=emb.device)).to(vis_feats.device)
+        else:
+            text = vis_feats.new_empty((0, vis_feats.shape[1]))
+        res = self._eng().predict_many(vis_feats, counts, text, prompt_counts, pos, None if qneg is None else negs, mode,
+                                       self.SOFTMAX_TEMP, bool(norm_vis_feat), threshold)
+        return [(pred.view(torch.bool), score) for score, pred in res]
 
 
 # ---------------------------------------------------------------------- a18

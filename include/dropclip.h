@@ -387,6 +387,29 @@ DC_API int dc_predict_queries(void* feats, int feat_dtype, int64_t n_points, con
                               int dim, const int32_t* pos, const int32_t* neg_off, const int32_t* neg_cols, int n_queries,
                               int mode, float softmax_temp, int normalize, float threshold, float* out, uint8_t* pred,
                               void* workspace, size_t workspace_bytes, dc_stream_t stream);
+/* dc_predict_queries for every scene of a batch in ONE call. Scene s owns the feature rows [point_off[s], point_off[s+1]),
+ * the prompt rows [prompt_off[s], prompt_off[s+1]) and the queries [query_off[s], query_off[s+1]); its (Q_s, N_s) block of
+ * the result equals what dc_predict_queries returns for that scene alone, bit for bit (same operands, same K order, same
+ * epilogue arithmetic).
+ *   feats [sum N, dim] fp16/fp32, the rows of the scenes with queries normalised in place when `normalize` (the rows of a
+ *   scene without queries are left untouched); text [sum P, dim] fp16/fp32 rows already L2-normalised; P_s <= 1536.
+ *   point_off (int64), prompt_off and query_off (int32) [n_scenes + 1] in HOST memory, starting at 0; sum N < 2^31,
+ *   sum Q <= 65535.
+ *   pos [sum Q], neg_off [sum Q + 1], neg_cols [neg_off[sum Q]] int32 in HOST memory: the columns of query q of scene s,
+ *   LOCAL to the scene's prompt block ([0, P_s)). Checked on the host like dc_predict_queries' table, then copied into
+ *   the workspace by cudaMemcpyAsync, with the GEMM's tile list and the scoring tables.
+ *   out fp32 / pred uint8: scene s's (Q_s, N_s) block starts at sum_{s' < s} Q_s' * N_s'.
+ *   One tcgen05 GEMM per block of 256 prompt columns over a tile list (128 rows of one scene x that scene's prompts)
+ *   writes S = X . T^T once, at a row stride of ld = max P_s rounded up to 4.
+ *   workspace: 256-byte aligned, dc_predict_many_workspace() bytes. S alone is 4 * sum N * ld bytes, so one scene with
+ *   many prompts widens S for the whole batch. */
+DC_API size_t dc_predict_many_workspace(int n_scenes, const int64_t* point_off, const int32_t* prompt_off,
+                                        const int32_t* query_off, int64_t n_neg_total, int dim, int feat_dtype, int text_dtype);
+DC_API int dc_predict_many(void* feats, int feat_dtype, const void* text, int text_dtype, int dim, int n_scenes,
+                           const int64_t* point_off, const int32_t* prompt_off, const int32_t* query_off, const int32_t* pos,
+                           const int32_t* neg_off, const int32_t* neg_cols, int mode, float softmax_temp, int normalize,
+                           float threshold, float* out, uint8_t* pred, void* workspace, size_t workspace_bytes,
+                           dc_stream_t stream);
 
 /* Global min-max normalisation + threshold (models/similarity.py:83-88, :95-98):
  * values <- (v - min)/(max - min) (or v / max when the raw extrema coincide), pred = values > thr
