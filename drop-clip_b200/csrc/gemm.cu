@@ -928,7 +928,8 @@ int dc_view_score(const void* feats, int feat_dtype, int64_t total_rows, int dim
   int* tile_count = reinterpret_cast<int*>(ws + w.tile_count);
   build_score_tiles_kernel<<<1, 1024, 0, st>>>(feat_off, view_off, query_off, n_scenes, tiles, tile_count, w.max_tiles);
   DC_LAUNCH_CHECK();
-  Params p{tiles, tile_count, total_rows, bn, dim, feat_dtype == DC_F32 ? 3 : 2};
+  Params p{tiles, tile_count, total_rows, bn, dim};
+  dc::gemm::set_terms(p, a_lo, q_lo);
   EpiStore epi{sims, sims_ld};
   return launch_bn(bn, a_hi, a_lo, total_rows, q_hi, q_lo, total_queries, p, epi, w.max_tiles, st);
 }
@@ -1028,7 +1029,6 @@ int dc_ground(const void* x_hi, const void* x_lo, int64_t n_points, const void* 
   const size_t need = dc_ground_workspace(n_points, n_prompts, mode);
   if (need > 0 && (!workspace || workspace_bytes < need))
     return dc::fail(DC_ERR_WORKSPACE, "dc_ground: %zu workspace bytes needed for %d prompts, got %zu", need, n_prompts, workspace_bytes);
-  const int n_terms = x_lo ? 3 : (t_lo ? 2 : 1);
   const int max_tiles = (int)dc::ceil_div<int64_t>(n_points, dc::gemm::kBlockM);
   // the prompt axis in blocks of <= 256 columns (the widest UMMA N): partial sums / maxima of the paired softmax,
   // the mean of the negatives and the arg max combine across blocks through `carry` (models/similarity.py:47-61
@@ -1036,7 +1036,8 @@ int dc_ground(const void* x_hi, const void* x_lo, int64_t n_points, const void* 
   for (int c0 = 0; c0 < n_prompts; c0 += 256) {
     const int cols = n_prompts - c0 < 256 ? n_prompts - c0 : 256;
     const int bn = pick_bn(cols);
-    Params p{nullptr, nullptr, n_points, cols, dim, n_terms};
+    Params p{nullptr, nullptr, n_points, cols, dim};
+    dc::gemm::set_terms(p, x_lo, t_lo);
     // after the separate normalisation pass the rows written last are still in L2 (126 MB): walk the tiles backwards
     p.reverse = (normalize_fp16_rows && c0 == 0) ? 1 : 0;
     EpiGround epi{};
@@ -1462,13 +1463,13 @@ int dc_predict_many(void* feats, int feat_dtype, const void* text, int text_dtyp
   }
   // S = X . T^T of every scene with its own prompts: one tcgen05 GEMM per block of 256 prompt columns over the tile list
   // (a tile = 128 rows of one scene x that scene's columns of the block), written once at the row stride s_ld
-  const int n_terms = x_lo ? 3 : (t_lo ? 2 : 1);
   const uint8_t* tb = ws + pl.tables;
   float* sims = reinterpret_cast<float*>(ws + pl.sims);
   for (size_t cb = 0; cb < pl.tile_count.size(); ++cb) {
     if (pl.tile_count[cb] == 0) continue;
     Params p{reinterpret_cast<const int4*>(tb + pl.t_tiles) + pl.tile_start[cb],
-             reinterpret_cast<const int*>(tb + pl.t_counts) + cb, n_rows, 0, dim, n_terms, 0};
+             reinterpret_cast<const int*>(tb + pl.t_counts) + cb, n_rows, 0, dim};
+    dc::gemm::set_terms(p, x_lo, t_lo);
     EpiStore epi{sims + 256 * cb, pl.s_ld};
     if ((rc = launch_bn(pl.tile_bn[cb], x_hi, x_lo, n_rows, t_hi, t_lo, pl.n_text_rows, p, epi,
                         pl.tile_count[cb], st)))

@@ -3,7 +3,8 @@
 // A and B are fp16 K-major planes in global memory. fp32 inputs are represented by two planes
 // (hi = fp16(x), lo = fp16(x - hi)); the kernel then runs the three products hi.hi + hi.lo +
 // lo.hi into the same accumulator, which restores ~22 bits of operand precision while staying on
-// the full-rate kind::f16 tensor path.
+// the full-rate kind::f16 tensor path. With one fp32 operand only its lo product is added: hi.lo
+// (fp32 B) or lo.hi (fp32 A, Params::a_lo_only).
 //
 // Warp roles (320 threads): warp 0 = TMA producer, warp 1 = TMEM allocator + MMA issuer,
 // warps 2..9 = epilogue (TMEM -> registers -> global). Three pipelines: smem full/empty ring
@@ -45,7 +46,14 @@ struct Params {
   int k;                  // inner dimension (multiple of 64)
   int n_terms;            // 1: hi.hi   2: + hi.lo   3: + lo.hi
   int reverse;            // dense tiling: walk the row tiles last to first (the rows a preceding pass wrote last are still in L2)
+  int a_lo_only;          // A has a lo plane and B has none (fp32 features, fp16 prompts): n_terms == 2 and term 1 is lo.hi
 };
+
+// The products whose planes exist: hi.hi, + hi.lo when B has a lo plane, + lo.hi when A has one.
+inline void set_terms(Params& p, const void* a_lo, const void* b_lo) {
+  p.n_terms = 1 + (a_lo ? 1 : 0) + (b_lo ? 1 : 0);
+  p.a_lo_only = (a_lo && !b_lo) ? 1 : 0;
+}
 
 template <int BN>
 struct Config {
@@ -106,8 +114,8 @@ gemm_kernel(const __grid_constant__ CUtensorMap tm_a_hi, const __grid_constant__
   if (warp == 0 && lane == 0) {
     umma::prefetch_tmap(&tm_a_hi);
     umma::prefetch_tmap(&tm_b_hi);
-    if (p.n_terms > 1) umma::prefetch_tmap(&tm_b_lo);
-    if (p.n_terms > 2) umma::prefetch_tmap(&tm_a_lo);
+    if (p.n_terms > 1 && !p.a_lo_only) umma::prefetch_tmap(&tm_b_lo);
+    if (p.n_terms > 2 || p.a_lo_only) umma::prefetch_tmap(&tm_a_lo);
     for (int s = 0; s < Cfg::kStages; ++s) {
       umma::mbar_init(full + s, 1);
       umma::mbar_init(empty + s, 1);
@@ -135,8 +143,9 @@ gemm_kernel(const __grid_constant__ CUtensorMap tm_a_hi, const __grid_constant__
       for (int t = blockIdx.x; t < n_tiles; t += gridDim.x) {
         const Tile tile = fetch_tile(p, t);
         for (int term = 0; term < p.n_terms; ++term) {
-          const CUtensorMap* ta = (term == 2) ? &tm_a_lo : &tm_a_hi;
-          const CUtensorMap* tb = (term == 1) ? &tm_b_lo : &tm_b_hi;
+          const bool a_lo = term == 2 || (term == 1 && p.a_lo_only);
+          const CUtensorMap* ta = a_lo ? &tm_a_lo : &tm_a_hi;
+          const CUtensorMap* tb = (term == 1 && !p.a_lo_only) ? &tm_b_lo : &tm_b_hi;
           for (int kb = 0; kb < k_blocks; ++kb) {
             umma::mbar_wait(empty + stage, phase ^ 1);
             umma::mbar_expect_tx(full + stage, Cfg::kStageBytes);

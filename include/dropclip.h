@@ -336,7 +336,8 @@ DC_API int dc_row_normalize(void* x, int dtype, int64_t n_rows, int dim, int nor
 
 /* sims = X . T^T followed by the mode's epilogue, one tcgen05 GEMM per block of 256 prompts.
  *   x_hi/x_lo  [n_points, dim] fp16 planes (x_lo NULL for fp16 features)
- *   t_hi/t_lo  [n_prompts, dim] fp16 planes, any n_prompts >= 1, prompt 0 is the positive one
+ *   t_hi/t_lo  [n_prompts, dim] fp16 planes (t_lo NULL for fp16 prompts), any n_prompts >= 1, prompt 0 is the positive
+ *              one. Either lo plane may be NULL while the other is set; the GEMM adds the lo product of each plane given.
  *   DC_GROUND_RAW:    out [n_points, out_ld] fp32 raw similarities
  *   DC_GROUND_PAIRED: out [n_points] fp32
  *   DC_GROUND_ARGMAX: out [n_points] fp32 (pos - mean(neg)), pred [n_points] uint8 (argmax == 0)
