@@ -5,6 +5,7 @@
 #include <algorithm>
 #include <cstring>
 #include <mutex>
+#include <type_traits>
 #include <vector>
 
 #include "gemm.cuh"
@@ -714,13 +715,42 @@ __global__ void init_minmax_kernel(float* m) {
   if (threadIdx.x == 0) { m[0] = INFINITY; m[1] = -INFINITY; m[2] = INFINITY; m[3] = -INFINITY; }
 }
 
+// The ground-truth tables of a counting launch of minmax_threshold_kernel (dc_predict_many_iou). Query q's points carry
+// the labels labels[point_row[q] + i]; its object ids are gt_ids[gt_off[q] .. gt_off[q+1]), sorted and unique.
+struct IouCount {
+  const void* labels;
+  const int64_t* point_row;
+  const int* gt_off;
+  const int64_t* gt_ids;
+  unsigned long long* inter;
+  unsigned long long* uni;
+};
+
+// Whether `label` is one of ids[0 .. n) (ascending): a binary search through the read-only cache.
+__device__ __forceinline__ bool id_listed(int64_t label, const int64_t* __restrict__ ids, int n) {
+  const int64_t* end = ids + n;
+  while (n > 0) {  // lower bound
+    const int half = n >> 1;
+    if (__ldg(ids + half) < label) { ids += half + 1; n -= half + 1; }
+    else n = half;
+  }
+  return ids < end && __ldg(ids) == label;
+}
+
 // A single-row launch (gridDim.y == 1, no row table) normalises v [n] with the extrema mm [4]. With `row_off`, blockIdx.y
 // selects query row y = v [row_off[y], row_off[y + 1]) with its own extrema mm [4 * y] (dc_predict_queries,
 // dc_predict_many); `n` is then unused.
+// Label != void (int32_t / int64_t, with a row table): count instead of writing. Point i of query y is predicted when
+// the normalised score x > thr (or, when !pred_from_thr, its argmax byte pred[i] is set) and is ground truth when its
+// label is one of the query's ids; the block adds |pred & gt| and |pred | gt| to cnt.inter[y] and cnt.uni[y]. Neither v
+// nor pred is written.
+template <class Label>
 __global__ void __launch_bounds__(256) minmax_threshold_kernel(float* __restrict__ v, int64_t n, const float* __restrict__ mm,
                                                                int use_raw, float thr, int pred_from_thr,
                                                                uint8_t* __restrict__ pred,
-                                                               const int64_t* __restrict__ row_off = nullptr) {
+                                                               const int64_t* __restrict__ row_off = nullptr,
+                                                               IouCount cnt = {}) {
+  constexpr bool kCount = !std::is_void<Label>::value;
   if (row_off) {
     const int64_t o = row_off[blockIdx.y];
     n = row_off[blockIdx.y + 1] - o;
@@ -731,11 +761,49 @@ __global__ void __launch_bounds__(256) minmax_threshold_kernel(float* __restrict
   const float mn = mm[0], mx = mm[1];
   const bool differ = use_raw ? (mm[3] != mm[2]) : (mx != mn);
   const float range = mx - mn;
-  for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (int64_t)gridDim.x * blockDim.x) {
-    float x = v[i];
-    x = differ ? (x - mn) / range : x / mx;
-    v[i] = x;
-    if (pred_from_thr) pred[i] = x > thr ? 1 : 0;
+  if constexpr (!kCount) {
+    for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (int64_t)gridDim.x * blockDim.x) {
+      float x = v[i];
+      x = differ ? (x - mn) / range : x / mx;
+      v[i] = x;
+      if (pred_from_thr) pred[i] = x > thr ? 1 : 0;
+    }
+  } else {
+    const Label* __restrict__ labels = static_cast<const Label*>(cnt.labels) + cnt.point_row[blockIdx.y];
+    const int g0 = cnt.gt_off[blockIdx.y], n_ids = cnt.gt_off[blockIdx.y + 1] - g0;
+    const int64_t* __restrict__ ids = cnt.gt_ids + g0;
+    unsigned both = 0, either = 0;  // < 2^31 points per query
+    for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (int64_t)gridDim.x * blockDim.x) {
+      bool p;
+      if (pred_from_thr) {
+        float x = v[i];
+        x = differ ? (x - mn) / range : x / mx;
+        p = x > thr;
+      } else {
+        p = pred[i] != 0;
+      }
+      const bool g = id_listed((int64_t)__ldg(labels + i), ids, n_ids);
+      both += (p && g) ? 1u : 0u;
+      either += (p || g) ? 1u : 0u;
+    }
+    __shared__ unsigned s_both[8], s_either[8];
+    both = __reduce_add_sync(0xffffffffu, both);
+    either = __reduce_add_sync(0xffffffffu, either);
+    if ((threadIdx.x & 31) == 0) {
+      s_both[threadIdx.x >> 5] = both;
+      s_either[threadIdx.x >> 5] = either;
+    }
+    __syncthreads();
+    if (threadIdx.x == 0) {
+      both = 0;
+      either = 0;
+      for (int w = 0; w < (int)(blockDim.x >> 5); ++w) {
+        both += s_both[w];
+        either += s_either[w];
+      }
+      if (both) atomicAdd(cnt.inter + blockIdx.y, (unsigned long long)both);
+      if (either) atomicAdd(cnt.uni + blockIdx.y, (unsigned long long)either);
+    }
   }
 }
 
@@ -1121,12 +1189,17 @@ namespace {
 // and the device tables - query rows, column CSR, scenes, score blocks and (dc_predict_many) the GEMM's tile lists -
 // staged in one host buffer and copied into the workspace by one cudaMemcpyAsync. A scene without queries gets no
 // blocks, no tiles and no normalisation.
+// dc_predict_many_iou also stages its ground-truth tables (query q's first feature row, gt_off, gt_ids) in the table
+// region, and keeps the scores and the argmax bytes in the workspace (`v`, `pred`).
 struct ScorePlan {
-  size_t minmax, tables, t_planes, x_planes, sims, total;                          // workspace byte offsets
-  size_t t_qrow, t_pos, t_off, t_cols, t_scenes, t_blocks, t_counts, t_tiles, t_bytes;  // inside the table region
+  size_t minmax, tables, t_planes, x_planes, sims, v, pred, total;                 // workspace byte offsets
+  size_t t_qrow, t_pos, t_off, t_cols, t_scenes, t_blocks, t_counts, t_tiles;      // inside the table region
+  size_t t_qpoint, t_gt_off, t_gt_ids, t_bytes;
   int n_queries = 0, minmax_slots = 0, max_prompts = 1, s_ld = 0, tile_rows = 0;  // max_prompts: over the scenes with queries
   int64_t n_rows = 0, n_text_rows = 0, n_neg = 0, max_points = 0;  // max_points: over the scenes with queries
+  int64_t n_gt = -1;              // dc_predict_many_iou: the number of ground-truth ids; -1: no counting
   std::vector<int64_t> qrow_off;  // [n_queries + 1]: query q's row of v / pred
+  std::vector<int64_t> qpoint;    // counting: [n_queries], the feature row of query q's first point
   std::vector<ScoreScene> scenes;
   std::vector<ScoreBlock> blocks;
   std::vector<int4> tiles;                            // the column blocks' tile lists, one after the other
@@ -1135,14 +1208,18 @@ struct ScorePlan {
 
 // tile_list: dc_predict_many's GEMM (explicit tiles, S row stride = the widest scene rounded up to 4); otherwise
 // dc_ground writes S [n_points, n_prompts] of the one scene densely. reverse: list the first column block's tiles last
-// to first (the rows normalised last are still in L2, as in dc_ground).
+// to first (the rows normalised last are still in L2, as in dc_ground). n_gt >= 0: the plan of dc_predict_many_iou with
+// n_gt ground-truth ids.
 ScorePlan score_plan(int n_scenes, const int64_t* point_off, const int32_t* prompt_off, const int32_t* query_off,
-                     int64_t n_neg, int dim, int feat_dtype, int text_dtype, bool tile_list, bool reverse) {
+                     int64_t n_neg, int dim, int feat_dtype, int text_dtype, bool tile_list, bool reverse,
+                     int64_t n_gt = -1) {
   ScorePlan pl;
   pl.n_rows = point_off[n_scenes];
   pl.n_text_rows = prompt_off[n_scenes];
   pl.n_queries = query_off[n_scenes];
   pl.n_neg = n_neg;
+  pl.n_gt = n_gt;
+  const bool count = n_gt >= 0;
   int& max_prompts = pl.max_prompts;
   int64_t out_off = 0;
   for (int s = 0; s < n_scenes; ++s) {
@@ -1150,6 +1227,7 @@ ScorePlan score_plan(int n_scenes, const int64_t* point_off, const int32_t* prom
     const int ps = prompt_off[s + 1] - prompt_off[s], qs = query_off[s + 1] - query_off[s];
     pl.scenes.push_back(ScoreScene{point_off[s], out_off, (int)ns, ps, query_off[s], 0});
     for (int q = 0; q < qs; ++q) pl.qrow_off.push_back(out_off + q * ns);
+    if (count) pl.qpoint.insert(pl.qpoint.end(), qs, point_off[s]);
     out_off += qs * ns;
     if (qs > 0) {
       max_prompts = std::max(max_prompts, ps);
@@ -1204,7 +1282,10 @@ ScorePlan score_plan(int n_scenes, const int64_t* point_off, const int32_t* prom
   pl.t_scenes = t; t += align_up(sizeof(ScoreScene) * pl.scenes.size(), 16);
   pl.t_blocks = t; t += align_up(sizeof(ScoreBlock) * pl.blocks.size(), 16);
   pl.t_counts = t; t += align_up(sizeof(int) * pl.tile_count.size(), 16);
-  pl.t_tiles = t; t += sizeof(int4) * pl.tiles.size();
+  pl.t_tiles = t; t += align_up(sizeof(int4) * pl.tiles.size(), 16);
+  pl.t_qpoint = t; if (count) t += align_up(sizeof(int64_t) * q, 16);
+  pl.t_gt_off = t; if (count) t += align_up(sizeof(int) * (q + 1), 16);
+  pl.t_gt_ids = t; if (count) t += sizeof(int64_t) * (size_t)n_gt;
   pl.t_bytes = t;
   pl.minmax_slots = pl.n_queries + (tile_list ? 0 : 1);  // + dc_ground's extrema, unused
   size_t off = 0;
@@ -1213,6 +1294,8 @@ ScorePlan score_plan(int n_scenes, const int64_t* point_off, const int32_t* prom
   pl.t_planes = off; if (text_dtype == DC_F32) off += 2 * align_up((size_t)pl.n_text_rows * dim * 2, 256);
   pl.x_planes = off; if (feat_dtype == DC_F32) off += 2 * align_up((size_t)(pl.n_rows > 0 ? pl.n_rows : 1) * dim * 2, 256);
   pl.sims = off; off += align_up((size_t)(pl.n_rows > 0 ? pl.n_rows : 1) * pl.s_ld * sizeof(float), 256);
+  pl.v = off; if (count) off += align_up(sizeof(float) * (size_t)out_off, 256);
+  pl.pred = off; if (count) off += align_up((size_t)out_off, 256);
   pl.total = off;
   return pl;
 }
@@ -1244,7 +1327,7 @@ int check_columns(const char* fn, int n_scenes, const int32_t* prompt_off, const
 }
 
 int stage_tables(const ScorePlan& pl, const int32_t* pos, const int32_t* neg_off, const int32_t* neg_cols, uint8_t* ws,
-                 cudaStream_t st) {
+                 cudaStream_t st, const int32_t* gt_off = nullptr, const int64_t* gt_ids = nullptr) {
   std::vector<uint8_t> h(pl.t_bytes);
   auto put = [&](size_t at, const void* src, size_t bytes) {
     if (bytes) memcpy(h.data() + at, src, bytes);
@@ -1258,14 +1341,20 @@ int stage_tables(const ScorePlan& pl, const int32_t* pos, const int32_t* neg_off
   put(pl.t_blocks, pl.blocks.data(), sizeof(ScoreBlock) * pl.blocks.size());
   put(pl.t_counts, pl.tile_count.data(), sizeof(int) * pl.tile_count.size());
   put(pl.t_tiles, pl.tiles.data(), sizeof(int4) * pl.tiles.size());
+  if (pl.n_gt >= 0) {
+    put(pl.t_qpoint, pl.qpoint.data(), sizeof(int64_t) * q);
+    put(pl.t_gt_off, gt_off, sizeof(int) * (q + 1));
+    put(pl.t_gt_ids, gt_ids, sizeof(int64_t) * (size_t)pl.n_gt);
+  }
   // pageable source: cudaMemcpyAsync returns once it has staged the bytes, so `h` may go out of scope
   DC_CUDA(cudaMemcpyAsync(ws + pl.tables, h.data(), pl.t_bytes, cudaMemcpyHostToDevice, st));
   return DC_OK;
 }
 
-// Every query scored from its columns of S [n_rows, s_ld], then its min-max and threshold (one launch each).
+// Every query scored from its columns of S [n_rows, s_ld], then its min-max and threshold (one launch each). With `cnt`
+// (dc_predict_many_iou) the second launch counts against the labels of dtype label_dtype instead of writing v and pred.
 int score_queries(const ScorePlan& pl, uint8_t* ws, int mode, float softmax_temp, float threshold, float* out,
-                  uint8_t* pred, cudaStream_t st) {
+                  uint8_t* pred, cudaStream_t st, const IouCount* cnt = nullptr, int label_dtype = DC_I64) {
   if (pl.blocks.empty()) return DC_OK;
   DC_CHECK_ARG(pl.blocks.size() < (1ull << 31), "too many score blocks for one launch");
   const uint8_t* tb = ws + pl.tables;
@@ -1296,8 +1385,16 @@ int score_queries(const ScorePlan& pl, uint8_t* ws, int mode, float softmax_temp
   // per-query min-max (+ threshold), every query in one launch (blockIdx.y = query, its row from the table)
   const int64_t blocks_x = dc::ceil_div<int64_t>(pl.max_points, 256);
   const int64_t per_query = std::max<int64_t>(1, dc::ceil_div<int64_t>((int64_t)dc::sm_count() * 8, pl.n_queries));
-  minmax_threshold_kernel<<<dim3((unsigned)std::min(blocks_x, per_query), (unsigned)pl.n_queries), 256, 0, st>>>(
-      out, 0, minmax, mode == DC_GROUND_ARGMAX ? 1 : 0, threshold, mode == DC_GROUND_ARGMAX ? 0 : 1, pred, qrow);
+  const dim3 mm_grid((unsigned)std::min(blocks_x, per_query), (unsigned)pl.n_queries);
+  const int use_raw = mode == DC_GROUND_ARGMAX ? 1 : 0, pred_from_thr = mode == DC_GROUND_ARGMAX ? 0 : 1;
+  if (!cnt)
+    minmax_threshold_kernel<void><<<mm_grid, 256, 0, st>>>(out, 0, minmax, use_raw, threshold, pred_from_thr, pred, qrow);
+  else if (label_dtype == DC_I32)
+    minmax_threshold_kernel<int32_t><<<mm_grid, 256, 0, st>>>(out, 0, minmax, use_raw, threshold, pred_from_thr, pred, qrow,
+                                                              *cnt);
+  else
+    minmax_threshold_kernel<int64_t><<<mm_grid, 256, 0, st>>>(out, 0, minmax, use_raw, threshold, pred_from_thr, pred, qrow,
+                                                              *cnt);
   DC_LAUNCH_CHECK();
   return DC_OK;
 }
@@ -1380,61 +1477,110 @@ int dc_predict_queries(void* feats, int feat_dtype, int64_t n_points, const void
   return score_queries(pl, ws, mode, softmax_temp, threshold, out, pred, st);
 }
 
-size_t dc_predict_many_workspace(int n_scenes, const int64_t* point_off, const int32_t* prompt_off, const int32_t* query_off,
-                                 int64_t n_neg_total, int dim, int feat_dtype, int text_dtype) {
+}  // extern "C"
+
+namespace {
+
+// The ground-truth side of dc_predict_many_iou.
+struct IouArgs {
+  const void* labels;
+  int label_dtype;
+  const int32_t* gt_off;
+  const int64_t* gt_ids;
+  int64_t* inter;
+  int64_t* uni;
+};
+
+size_t predict_many_workspace(int n_scenes, const int64_t* point_off, const int32_t* prompt_off, const int32_t* query_off,
+                              int64_t n_neg_total, int dim, int feat_dtype, int text_dtype, int64_t n_gt) {
   if (n_scenes < 0 || (n_scenes > 0 && !(point_off && prompt_off && query_off))) return 0;
   const int64_t zero64 = 0;
   const int32_t zero32 = 0;
-  if (n_scenes == 0) return score_plan(0, &zero64, &zero32, &zero32, 0, dim, feat_dtype, text_dtype, true, false).total;
-  return score_plan(n_scenes, point_off, prompt_off, query_off, n_neg_total, dim, feat_dtype, text_dtype, true, false).total;
+  if (n_scenes == 0)
+    return score_plan(0, &zero64, &zero32, &zero32, 0, dim, feat_dtype, text_dtype, true, false, n_gt >= 0 ? 0 : -1).total;
+  return score_plan(n_scenes, point_off, prompt_off, query_off, n_neg_total, dim, feat_dtype, text_dtype, true, false,
+                    n_gt).total;
 }
 
-int dc_predict_many(void* feats, int feat_dtype, const void* text, int text_dtype, int dim, int n_scenes,
-                    const int64_t* point_off, const int32_t* prompt_off, const int32_t* query_off, const int32_t* pos,
-                    const int32_t* neg_off, const int32_t* neg_cols, int mode, float softmax_temp, int normalize,
-                    float threshold, float* out, uint8_t* pred, void* workspace, size_t workspace_bytes,
-                    dc_stream_t stream) {
-  DC_CHECK_ARG(n_scenes >= 0, "dc_predict_many: negative scene count");
+// dc_predict_many (iou == nullptr: the scores and predictions go to out / pred) and dc_predict_many_iou (the scores and
+// the argmax bytes stay in the workspace; the threshold pass counts against the ground truth instead). `fn` names the
+// entry point in the error messages.
+int predict_many(const char* fn, void* feats, int feat_dtype, const void* text, int text_dtype, int dim, int n_scenes,
+                 const int64_t* point_off, const int32_t* prompt_off, const int32_t* query_off, const int32_t* pos,
+                 const int32_t* neg_off, const int32_t* neg_cols, int mode, float softmax_temp, int normalize,
+                 float threshold, float* out, uint8_t* pred, const IouArgs* iou, void* workspace, size_t workspace_bytes,
+                 dc_stream_t stream) {
+  DC_CHECK_ARG(n_scenes >= 0, "%s: negative scene count", fn);
   if (n_scenes == 0) return DC_OK;
-  DC_CHECK_ARG(point_off && prompt_off && query_off && neg_off && workspace, "dc_predict_many: null pointer argument");
-  DC_CHECK_ARG(feat_dtype == DC_F16 || feat_dtype == DC_F32, "dc_predict_many: features must be fp16 or fp32");
-  DC_CHECK_ARG(text_dtype == DC_F16 || text_dtype == DC_F32, "dc_predict_many: prompt embeddings must be fp16 or fp32");
-  DC_CHECK_ARG(mode == DC_GROUND_RAW || mode == DC_GROUND_PAIRED || mode == DC_GROUND_ARGMAX, "dc_predict_many: bad mode");
-  DC_CHECK_ARG(dim > 0 && dim % 64 == 0, "dc_predict_many: feature dim must be a multiple of 64 (got %d)", dim);
-  DC_CHECK_ARG(((uintptr_t)workspace & 255) == 0, "dc_predict_many: workspace must be 256-byte aligned");
-  DC_CHECK_ARG(point_off[0] == 0 && prompt_off[0] == 0 && query_off[0] == 0, "dc_predict_many: offset tables must start at 0");
+  DC_CHECK_ARG(point_off && prompt_off && query_off && neg_off && workspace, "%s: null pointer argument", fn);
+  DC_CHECK_ARG(feat_dtype == DC_F16 || feat_dtype == DC_F32, "%s: features must be fp16 or fp32", fn);
+  DC_CHECK_ARG(text_dtype == DC_F16 || text_dtype == DC_F32, "%s: prompt embeddings must be fp16 or fp32", fn);
+  DC_CHECK_ARG(mode == DC_GROUND_RAW || mode == DC_GROUND_PAIRED || mode == DC_GROUND_ARGMAX, "%s: bad mode", fn);
+  DC_CHECK_ARG(dim > 0 && dim % 64 == 0, "%s: feature dim must be a multiple of 64 (got %d)", fn, dim);
+  DC_CHECK_ARG(((uintptr_t)workspace & 255) == 0, "%s: workspace must be 256-byte aligned", fn);
+  DC_CHECK_ARG(point_off[0] == 0 && prompt_off[0] == 0 && query_off[0] == 0, "%s: offset tables must start at 0", fn);
   for (int s = 0; s < n_scenes; ++s) {
     const int64_t ns = point_off[s + 1] - point_off[s];
     const int ps = prompt_off[s + 1] - prompt_off[s], qs = query_off[s + 1] - query_off[s];
-    DC_CHECK_ARG(ns >= 0 && ps >= 0 && qs >= 0, "dc_predict_many: offset tables must not decrease (scene %d)", s);
-    DC_CHECK_ARG(ps <= kQueryMaxPrompts, "dc_predict_many: scene %d: 0..%d prompts (got %d)", s, kQueryMaxPrompts, ps);
-    DC_CHECK_ARG(qs == 0 || ps >= 1, "dc_predict_many: scene %d has queries but no prompts", s);
+    DC_CHECK_ARG(ns >= 0 && ps >= 0 && qs >= 0, "%s: offset tables must not decrease (scene %d)", fn, s);
+    DC_CHECK_ARG(ps <= kQueryMaxPrompts, "%s: scene %d: 0..%d prompts (got %d)", fn, s, kQueryMaxPrompts, ps);
+    DC_CHECK_ARG(qs == 0 || ps >= 1, "%s: scene %d has queries but no prompts", fn, s);
   }
   const int64_t n_rows = point_off[n_scenes];
   const int n_queries = query_off[n_scenes];
-  DC_CHECK_ARG(n_rows < (1ll << 31), "dc_predict_many: too many points for one call (%lld)", (long long)n_rows);
-  DC_CHECK_ARG(n_queries <= 65535, "dc_predict_many: at most 65535 queries in all (got %d)", n_queries);
-  DC_CHECK_ARG(n_rows == 0 || feats, "dc_predict_many: null pointer argument");
-  DC_CHECK_ARG(prompt_off[n_scenes] == 0 || text, "dc_predict_many: null pointer argument");
+  DC_CHECK_ARG(n_rows < (1ll << 31), "%s: too many points for one call (%lld)", fn, (long long)n_rows);
+  DC_CHECK_ARG(n_queries <= 65535, "%s: at most 65535 queries in all (got %d)", fn, n_queries);
+  DC_CHECK_ARG(n_rows == 0 || feats, "%s: null pointer argument", fn);
+  DC_CHECK_ARG(prompt_off[n_scenes] == 0 || text, "%s: null pointer argument", fn);
   int64_t n_cells = 0;
   for (int s = 0; s < n_scenes; ++s)
     n_cells += (int64_t)(query_off[s + 1] - query_off[s]) * (point_off[s + 1] - point_off[s]);
-  DC_CHECK_ARG(n_cells == 0 || (out && pred), "dc_predict_many: null pointer argument");
-  DC_CHECK_ARG(n_queries == 0 || pos, "dc_predict_many: null pointer argument");
+  DC_CHECK_ARG(iou || n_cells == 0 || (out && pred), "%s: null pointer argument", fn);
+  DC_CHECK_ARG(n_queries == 0 || pos, "%s: null pointer argument", fn);
   int rc;
-  if ((rc = check_columns("dc_predict_many", n_scenes, prompt_off, query_off, pos, neg_off, neg_cols, mode))) return rc;
+  if ((rc = check_columns(fn, n_scenes, prompt_off, query_off, pos, neg_off, neg_cols, mode))) return rc;
+  int64_t n_gt = -1;
+  if (iou) {
+    DC_CHECK_ARG(iou->label_dtype == DC_I32 || iou->label_dtype == DC_I64, "%s: labels must be int32 or int64", fn);
+    DC_CHECK_ARG(n_queries == 0 || (iou->gt_off && iou->inter && iou->uni), "%s: null pointer argument", fn);
+    DC_CHECK_ARG(n_cells == 0 || iou->labels, "%s: null pointer argument", fn);
+    if (n_queries > 0) {
+      const int32_t* g = iou->gt_off;
+      DC_CHECK_ARG(g[0] == 0, "%s: gt_off[0] must be 0", fn);
+      for (int q = 0; q < n_queries; ++q) {
+        DC_CHECK_ARG(g[q + 1] >= g[q], "%s: gt_off must not decrease (query %d)", fn, q);
+        for (int j = g[q] + 1; j < g[q + 1]; ++j)
+          DC_CHECK_ARG(iou->gt_ids[j] > iou->gt_ids[j - 1], "%s: query %d: ground-truth ids must be strictly ascending", fn,
+                       q);
+      }
+      n_gt = g[n_queries];
+      DC_CHECK_ARG(n_gt == 0 || iou->gt_ids, "%s: null pointer argument", fn);
+    }
+  }
   if (n_queries == 0) return DC_OK;
   cudaStream_t st = dc::as_stream(stream);
   const ScorePlan pl = score_plan(n_scenes, point_off, prompt_off, query_off, neg_off[n_queries], dim, feat_dtype,
-                                  text_dtype, true, feat_dtype == DC_F16 && normalize);
-  if (workspace_bytes < pl.total)
-    return dc::fail(DC_ERR_WORKSPACE, "dc_predict_many: workspace %zu < %zu", workspace_bytes, pl.total);
+                                  text_dtype, true, feat_dtype == DC_F16 && normalize, n_gt);
+  if (workspace_bytes < pl.total) return dc::fail(DC_ERR_WORKSPACE, "%s: workspace %zu < %zu", fn, workspace_bytes, pl.total);
   uint8_t* ws = static_cast<uint8_t*>(workspace);
+  IouCount cnt{};
+  if (iou) {
+    // every query reports 0 / 0 until its blocks add to it (a query of an empty scene gets none)
+    DC_CUDA(cudaMemsetAsync(iou->inter, 0, sizeof(int64_t) * n_queries, st));
+    DC_CUDA(cudaMemsetAsync(iou->uni, 0, sizeof(int64_t) * n_queries, st));
+    out = reinterpret_cast<float*>(ws + pl.v);
+    pred = ws + pl.pred;
+    const uint8_t* tb = ws + pl.tables;
+    cnt = IouCount{iou->labels, reinterpret_cast<const int64_t*>(tb + pl.t_qpoint), reinterpret_cast<const int*>(tb + pl.t_gt_off),
+                   reinterpret_cast<const int64_t*>(tb + pl.t_gt_ids), reinterpret_cast<unsigned long long*>(iou->inter),
+                   reinterpret_cast<unsigned long long*>(iou->uni)};
+  }
   float* minmax = reinterpret_cast<float*>(ws + pl.minmax);
   init_query_minmax_kernel<<<1, 256, 0, st>>>(minmax, pl.minmax_slots);
   DC_LAUNCH_CHECK();
   if (pl.blocks.empty()) return DC_OK;  // every scene with queries is empty
-  if ((rc = stage_tables(pl, pos, neg_off, neg_cols, ws, st))) return rc;
+  if ((rc = stage_tables(pl, pos, neg_off, neg_cols, ws, st, iou ? iou->gt_off : nullptr, iou ? iou->gt_ids : nullptr)))
+    return rc;
   const void *t_hi, *t_lo;
   if ((rc = prompt_planes(pl, text, text_dtype, dim, ws, &t_hi, &t_lo, st))) return rc;
   // the features of the scenes with queries, normalised in place (when asked) as dc_predict_queries does: fp32 rows
@@ -1475,7 +1621,46 @@ int dc_predict_many(void* feats, int feat_dtype, const void* text, int text_dtyp
                         pl.tile_count[cb], st)))
       return rc;
   }
-  return score_queries(pl, ws, mode, softmax_temp, threshold, out, pred, st);
+  return score_queries(pl, ws, mode, softmax_temp, threshold, out, pred, st, iou ? &cnt : nullptr,
+                       iou ? iou->label_dtype : DC_I64);
+}
+
+}  // namespace
+
+extern "C" {
+
+size_t dc_predict_many_workspace(int n_scenes, const int64_t* point_off, const int32_t* prompt_off, const int32_t* query_off,
+                                 int64_t n_neg_total, int dim, int feat_dtype, int text_dtype) {
+  return predict_many_workspace(n_scenes, point_off, prompt_off, query_off, n_neg_total, dim, feat_dtype, text_dtype, -1);
+}
+
+int dc_predict_many(void* feats, int feat_dtype, const void* text, int text_dtype, int dim, int n_scenes,
+                    const int64_t* point_off, const int32_t* prompt_off, const int32_t* query_off, const int32_t* pos,
+                    const int32_t* neg_off, const int32_t* neg_cols, int mode, float softmax_temp, int normalize,
+                    float threshold, float* out, uint8_t* pred, void* workspace, size_t workspace_bytes,
+                    dc_stream_t stream) {
+  return predict_many("dc_predict_many", feats, feat_dtype, text, text_dtype, dim, n_scenes, point_off, prompt_off,
+                      query_off, pos, neg_off, neg_cols, mode, softmax_temp, normalize, threshold, out, pred, nullptr,
+                      workspace, workspace_bytes, stream);
+}
+
+size_t dc_predict_many_iou_workspace(int n_scenes, const int64_t* point_off, const int32_t* prompt_off,
+                                     const int32_t* query_off, int64_t n_neg_total, int64_t n_gt_total, int dim,
+                                     int feat_dtype, int text_dtype) {
+  return predict_many_workspace(n_scenes, point_off, prompt_off, query_off, n_neg_total, dim, feat_dtype, text_dtype,
+                                n_gt_total > 0 ? n_gt_total : 0);
+}
+
+int dc_predict_many_iou(void* feats, int feat_dtype, const void* text, int text_dtype, int dim, int n_scenes,
+                        const int64_t* point_off, const int32_t* prompt_off, const int32_t* query_off, const int32_t* pos,
+                        const int32_t* neg_off, const int32_t* neg_cols, const void* labels, int label_dtype,
+                        const int32_t* gt_off, const int64_t* gt_ids, int mode, float softmax_temp, int normalize,
+                        float threshold, int64_t* inter, int64_t* uni, void* workspace, size_t workspace_bytes,
+                        dc_stream_t stream) {
+  const IouArgs iou{labels, label_dtype, gt_off, gt_ids, inter, uni};
+  return predict_many("dc_predict_many_iou", feats, feat_dtype, text, text_dtype, dim, n_scenes, point_off, prompt_off,
+                      query_off, pos, neg_off, neg_cols, mode, softmax_temp, normalize, threshold, nullptr, nullptr, &iou,
+                      workspace, workspace_bytes, stream);
 }
 
 int dc_minmax_threshold(float* values, int64_t n, const float* minmax, int use_raw_extrema_for_test, float threshold,
@@ -1485,7 +1670,7 @@ int dc_minmax_threshold(float* values, int64_t n, const float* minmax, int use_r
   if (n <= 0) return DC_OK;
   const int64_t blocks = dc::ceil_div<int64_t>(n, 256);
   const unsigned grid = (unsigned)(blocks < (int64_t)dc::sm_count() * 8 ? blocks : (int64_t)dc::sm_count() * 8);
-  minmax_threshold_kernel<<<grid, 256, 0, dc::as_stream(stream)>>>(values, n, minmax, use_raw_extrema_for_test, threshold,
+  minmax_threshold_kernel<void><<<grid, 256, 0, dc::as_stream(stream)>>>(values, n, minmax, use_raw_extrema_for_test, threshold,
                                                                   pred_from_threshold, pred);
   DC_LAUNCH_CHECK();
   return DC_OK;

@@ -13,6 +13,7 @@ from dataclasses import dataclass, field
 from typing import Dict, List, Optional, Sequence
 
 import ctypes
+import operator
 import os
 
 import numpy as np
@@ -77,6 +78,31 @@ def query_csr(pos, neg_lists, n_prompts: int):
     if off[-1] >= 2 ** 31:
         raise ValueError("too many negative columns for one call")
     return pos_a.astype(np.int32), off.astype(np.int32), cols.astype(np.int32)
+
+
+def gt_csr(gt_ids, q_counts, label_dtype):
+    """Host ground-truth table of FusionEngine.predict_many_iou: (gt_off int32 [sum Q + 1], ids int64) from gt_ids[s][q],
+    any iterable of ints per query q of scene s (q_counts[s] queries), each list sorted and deduplicated. ValueError when
+    a scene's number of id lists differs from its query count, or an id lies outside the range of label_dtype (the
+    dtype of the labels it is compared with: torch.int32 or torch.int64)."""
+    lo, hi = (-2 ** 31, 2 ** 31 - 1) if label_dtype == torch.int32 else (-2 ** 63, 2 ** 63 - 1)
+    if len(gt_ids) != len(q_counts):
+        raise ValueError(f"{len(q_counts)} scenes but {len(gt_ids)} ground-truth lists")
+    lists = []
+    for s, (scene, q) in enumerate(zip(gt_ids, q_counts)):
+        scene = list(scene)
+        if len(scene) != q:
+            raise ValueError(f"scene {s} has {q} queries but {len(scene)} ground-truth id lists")
+        for ids in scene:
+            ids = sorted({operator.index(i) for i in ids})
+            if ids and (ids[0] < lo or ids[-1] > hi):
+                raise ValueError(f"object id {ids[0] if ids[0] < lo else ids[-1]} outside the range of {label_dtype} labels")
+            lists.append(ids)
+    off = _prefix([len(x) for x in lists])
+    if off[-1] >= 2 ** 31:
+        raise ValueError("too many ground-truth ids for one call")
+    ids = np.array([i for x in lists for i in x], dtype=np.int64)
+    return off.astype(np.int32), ids
 
 
 def intrinsic_matrix(intr: Dict[str, float]) -> np.ndarray:
@@ -968,14 +994,11 @@ class FusionEngine:
             self.launches += 1
         return score, pred
 
-    def predict_many(self, feats: torch.Tensor, counts, text: torch.Tensor, prompt_counts, pos, neg_lists, mode: int,
-                     softmax_temp: float, normalize: bool, threshold: float):
-        """`predict_queries` for every scene of a batch in one library call. feats (sum N, C) holds the scenes' rows in
-        scene order, counts[s] = N_s; text (sum P, C) the scenes' prompt blocks (already normalised rows),
-        prompt_counts[s] = P_s; pos[s] / neg_lists[s] (None: no negatives, RAW) index scene s's prompt block as in
-        predict_queries. Every index, count and mode rule is checked before anything reaches the device. Returns one
-        (score (Q_s, N_s) fp32, pred (Q_s, N_s) uint8) pair per scene, views into one score and one pred buffer; each
-        equals predict_queries(rows of scene s, text block of scene s, pos[s], neg_lists[s], ...)."""
+    @staticmethod
+    def _batch_tables(feats: torch.Tensor, counts, text: torch.Tensor, prompt_counts, pos, neg_lists, mode: int):
+        """The host tables of predict_many / predict_many_iou, every index, count and mode rule checked: a dict of
+        point_off int64, prompt_off / query_off int32 [S + 1], q_counts, pos int32 [sum Q], neg_off int32 [sum Q + 1] and
+        neg_cols int32 (global CSR of the scene-local columns)."""
         counts = [int(c) for c in counts]
         prompt_counts = [int(p) for p in prompt_counts]
         s_n = len(counts)
@@ -992,6 +1015,25 @@ class FusionEngine:
             if off.size > 1 and (raw != (cols.size == 0) or (not raw and (np.diff(off) == 0).any())):
                 raise ValueError("raw mode takes no negatives; paired and argmax need negatives for every query")
         q_counts = [int(t[0].size) for t in tables]
+        none = [np.zeros(0, dtype=np.int32)]
+        off = _prefix([int(t[1][-1]) for t in tables])
+        return {"counts": counts, "q_counts": q_counts, "point_off": _prefix(counts).astype(np.int64),
+                "prompt_off": _prefix(prompt_counts).astype(np.int32), "query_off": _prefix(q_counts).astype(np.int32),
+                "pos": np.concatenate(none + [t[0] for t in tables]).astype(np.int32),
+                "neg_off": np.concatenate([[0]] + [t[1][1:] + off[s] for s, t in enumerate(tables)]).astype(np.int32),
+                "neg_cols": np.concatenate(none + [t[2] for t in tables]).astype(np.int32)}
+
+    def predict_many(self, feats: torch.Tensor, counts, text: torch.Tensor, prompt_counts, pos, neg_lists, mode: int,
+                     softmax_temp: float, normalize: bool, threshold: float):
+        """`predict_queries` for every scene of a batch in one library call. feats (sum N, C) holds the scenes' rows in
+        scene order, counts[s] = N_s; text (sum P, C) the scenes' prompt blocks (already normalised rows),
+        prompt_counts[s] = P_s; pos[s] / neg_lists[s] (None: no negatives, RAW) index scene s's prompt block as in
+        predict_queries. Every index, count and mode rule is checked before anything reaches the device. Returns one
+        (score (Q_s, N_s) fp32, pred (Q_s, N_s) uint8) pair per scene, views into one score and one pred buffer; each
+        equals predict_queries(rows of scene s, text block of scene s, pos[s], neg_lists[s], ...)."""
+        tb = self._batch_tables(feats, counts, text, prompt_counts, pos, neg_lists, mode)
+        counts, q_counts = tb["counts"], tb["q_counts"]
+        s_n = len(counts)
         dev = feats.device
         cells = [q * n for q, n in zip(q_counts, counts)]
         res = torch.empty(max(sum(cells), 1) * 5 + 256, dtype=torch.uint8, device=dev)  # score fp32 + pred u8 in one allocation
@@ -1006,25 +1048,61 @@ class FusionEngine:
         text = text.contiguous()
         if text.dtype not in (torch.float16, torch.float32):
             text = text.float()
-        point_off = _prefix(counts).astype(np.int64)
-        prompt_off = _prefix(prompt_counts).astype(np.int32)
-        query_off = _prefix(q_counts).astype(np.int32)
-        pos_a = np.concatenate([t[0] for t in tables]).astype(np.int32)
-        cols = np.concatenate([t[2] for t in tables]).astype(np.int32)
-        off = _prefix([int(t[1][-1]) for t in tables])
-        neg_off = np.concatenate([[0]] + [t[1][1:] + off[s] for s, t in enumerate(tables)]).astype(np.int32)
         fcode, tcode = _lib.torch_dtype_code(feats.dtype), _lib.torch_dtype_code(text.dtype)
         c_p = lambda a: a.ctypes.data_as(ctypes.c_void_p)  # noqa: E731
-        ws_bytes = self.lib.dc_predict_many_workspace(s_n, c_p(point_off), c_p(prompt_off), c_p(query_off), int(cols.size),
-                                                      dim, fcode, tcode)
+        cols = tb["neg_cols"]
+        ws_bytes = self.lib.dc_predict_many_workspace(s_n, c_p(tb["point_off"]), c_p(tb["prompt_off"]), c_p(tb["query_off"]),
+                                                      int(cols.size), dim, fcode, tcode)
         ws = torch.empty(ws_bytes + 256, dtype=torch.uint8, device=dev)
         shift = (-ws.data_ptr()) % 256
         check(self.lib.dc_predict_many(
-            ptr(feats) if n_total else None, fcode, ptr(text) if text.shape[0] else None, tcode, dim, s_n, c_p(point_off),
-            c_p(prompt_off), c_p(query_off), c_p(pos_a), c_p(neg_off), c_p(cols) if cols.size else None, mode,
-            float(softmax_temp), int(bool(normalize)), float(threshold), ctypes.c_void_p(res.data_ptr()),
+            ptr(feats) if n_total else None, fcode, ptr(text) if text.shape[0] else None, tcode, dim, s_n, c_p(tb["point_off"]),
+            c_p(tb["prompt_off"]), c_p(tb["query_off"]), c_p(tb["pos"]), c_p(tb["neg_off"]), c_p(cols) if cols.size else None,
+            mode, float(softmax_temp), int(bool(normalize)), float(threshold), ctypes.c_void_p(res.data_ptr()),
             ctypes.c_void_p(res.data_ptr() + pred_base), ctypes.c_void_p(ws.data_ptr() + shift), ws_bytes, current_stream()))
         return out
+
+    def predict_many_iou(self, feats: torch.Tensor, counts, text: torch.Tensor, prompt_counts, pos, neg_lists, labels,
+                         gt_ids, mode: int, softmax_temp: float, normalize: bool, threshold: float):
+        """predict_many scored against point labels in one library call, without returning the scores or predictions:
+        (inter, union) int64 CUDA tensors of shape (sum Q,), in query order. For query q of scene s, inter = |pred & gt|
+        and union = |pred | gt| where pred is row q of predict_many's scene-s prediction and gt = isin(labels of scene s,
+        gt_ids[s][q]). labels (sum N,) int32 / int64 CUDA tensor in feature-row order; gt_ids[s][q] any iterable of ints
+        (sorted and deduplicated here). Every index, count, mode, label and id rule is checked before anything reaches
+        the device; an id outside the label dtype's range raises ValueError."""
+        tb = self._batch_tables(feats, counts, text, prompt_counts, pos, neg_lists, mode)
+        counts, q_counts = tb["counts"], tb["q_counts"]
+        if not isinstance(labels, torch.Tensor) or labels.dtype not in (torch.int32, torch.int64):
+            raise ValueError("labels must be an int32 or int64 tensor")
+        if labels.numel() != feats.shape[0]:
+            raise ValueError(f"{labels.numel()} labels for {feats.shape[0]} feature rows")
+        if labels.device != feats.device:
+            raise RuntimeError(f"labels on {labels.device}, features on {feats.device}")
+        gt_off, ids = gt_csr(gt_ids, q_counts, labels.dtype)
+        s_n, n_q = len(counts), sum(q_counts)
+        dev = feats.device
+        res = torch.empty((2, n_q), dtype=torch.int64, device=dev)
+        if n_q == 0:
+            return res[0], res[1]
+        labels = labels.reshape(-1).contiguous()
+        n_total, dim = feats.shape
+        text = text.contiguous()
+        if text.dtype not in (torch.float16, torch.float32):
+            text = text.float()
+        fcode, tcode = _lib.torch_dtype_code(feats.dtype), _lib.torch_dtype_code(text.dtype)
+        c_p = lambda a: a.ctypes.data_as(ctypes.c_void_p)  # noqa: E731
+        cols = tb["neg_cols"]
+        ws_bytes = self.lib.dc_predict_many_iou_workspace(s_n, c_p(tb["point_off"]), c_p(tb["prompt_off"]),
+                                                          c_p(tb["query_off"]), int(cols.size), int(ids.size), dim, fcode, tcode)
+        ws = torch.empty(ws_bytes + 256, dtype=torch.uint8, device=dev)
+        shift = (-ws.data_ptr()) % 256
+        check(self.lib.dc_predict_many_iou(
+            ptr(feats) if n_total else None, fcode, ptr(text) if text.shape[0] else None, tcode, dim, s_n, c_p(tb["point_off"]),
+            c_p(tb["prompt_off"]), c_p(tb["query_off"]), c_p(tb["pos"]), c_p(tb["neg_off"]), c_p(cols) if cols.size else None,
+            ptr(labels) if n_total else None, _lib.torch_dtype_code(labels.dtype), c_p(gt_off), c_p(ids) if ids.size else None,
+            mode, float(softmax_temp), int(bool(normalize)), float(threshold), ptr(res[0]), ptr(res[1]),
+            ctypes.c_void_p(ws.data_ptr() + shift), ws_bytes, current_stream()))
+        return res[0], res[1]
 
     def minmax_threshold(self, values, minmax, use_raw: bool, threshold: float, want_pred: bool):
         pred = torch.empty(values.numel(), dtype=torch.uint8, device=values.device) if want_pred else None

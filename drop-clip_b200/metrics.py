@@ -15,7 +15,7 @@ import torch
 from . import _lib
 from ._lib import check, current_stream, ptr
 
-__all__ = ["trainMetricPC", "intersectionAndUnionGPU", "binary_iou_counts"]
+__all__ = ["trainMetricPC", "intersectionAndUnionGPU", "binary_iou_counts", "grounding_scores"]
 
 
 def _require_cuda(t: torch.Tensor, what: str):
@@ -64,10 +64,18 @@ def binary_iou_counts(preds: Sequence[torch.Tensor], gts: Sequence[torch.Tensor]
 @torch.no_grad()
 def trainMetricPC(output, target, threshold=0.35, pr_ious=[0.25, 0.5, 0.75], sigmoid=False):
     assert len(output) == len(target)
-    count = 1e-6 + len(output)
-    if len(output) == 0:  # the reference's accumulators stay python floats
+    if len(output) == 0:
+        return grounding_scores((), (), pr_ious)
+    return grounding_scores(*binary_iou_counts(list(output), list(target), threshold, sigmoid), pr_ious)
+
+
+@torch.no_grad()
+def grounding_scores(inter, union, pr_ious=[0.25, 0.5, 0.75]):
+    """trainMetricPC's mIoU and Pr@k (percent) from per-instance |pred & gt| and |pred | gt| counts, e.g. the
+    (inter, union) of binary_iou_counts or of ClipSimilarity.predict_many_iou."""
+    count = 1e-6 + len(inter)
+    if len(inter) == 0:  # the reference's accumulators stay python floats
         return 100. * (0.0 / (count + 1e-6)), [100. * (0.0 / count) for _ in pr_ious]
-    inter, union = binary_iou_counts(list(output), list(target), threshold, sigmoid)
     iou = inter / (union + 1e-6)  # int64 / fp32 -> fp32, as in the reference
     mean_iou = iou.sum()          # (the reference adds the instances one by one in fp32)
     mean_prec: List[torch.Tensor] = [(iou > pr_iou).float().sum() for pr_iou in pr_ious]

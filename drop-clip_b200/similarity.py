@@ -221,6 +221,43 @@ class ClipSimilarity(object):
         method = method or self.method
         threshold = threshold or self.threshold
         norm_vis_feat = norm_vis_feat or self.norm_vis_feat
+        batch = self._batch_prompts(vis_feats, counts, queries, qneg, method)
+        if batch is None:
+            return [None] * len(counts)  # predict falls off the end of its if/elif chain
+        counts, mode, text, prompt_counts, pos, negs = batch
+        res = self._eng().predict_many(vis_feats, counts, text, prompt_counts, pos, negs, mode, self.SOFTMAX_TEMP,
+                                       bool(norm_vis_feat), threshold)
+        return [(pred.view(torch.bool), score) for score, pred in res]
+
+    @torch.no_grad()
+    def predict_many_iou(self, vis_feats, counts, labels, obj_queries, qneg="scene", norm_vis_feat=None, method=None,
+                         threshold=None):
+        """predict_many scored against the point labels in one library call, for the grounding evaluation loops
+        (engine/distil.py:436-493, tools/validate_upper_bound.py:200-221): returns (inter, union), int64 CUDA tensors of
+        shape (sum Q,). obj_queries[s] maps each text query of scene s to its object ids (the reference's mapping);
+        the queries of a scene are its keys in order, scene after scene. For query q with ids `ids` of scene s,
+        inter = |pred & gt| and union = |pred | gt|, where pred is the row predict_many(vis_feats, counts, [list(o) for o in
+        obj_queries], qneg, ...) returns for the query and gt = isin(labels of scene s, ids): what trainMetricPC counts
+        for that query, at any of its thresholds in (0, 1] without sigmoid. metrics.grounding_scores(inter, union) then
+        gives trainMetricPC's mIoU and Pr@k. Neither the scores nor the predictions are returned.
+        labels (sum N,) int32 / int64 CUDA tensor in feature-row order. Defaults, the in-place normalisation and the
+        errors follow predict_many, and every error is raised before any row changes; ValueError also for labels of
+        another dtype or count, and for an id outside the labels' dtype. None for a method predict does not know."""
+        method = method or self.method
+        threshold = threshold or self.threshold
+        norm_vis_feat = norm_vis_feat or self.norm_vis_feat
+        obj_queries = [dict(o) for o in obj_queries]
+        batch = self._batch_prompts(vis_feats, counts, [list(o) for o in obj_queries], qneg, method)
+        if batch is None:
+            return None  # predict falls off the end of its if/elif chain
+        counts, mode, text, prompt_counts, pos, negs = batch
+        gt_ids = [[list(ids) for ids in o.values()] for o in obj_queries]
+        return self._eng().predict_many_iou(vis_feats, counts, text, prompt_counts, pos, negs, labels, gt_ids, mode,
+                                            self.SOFTMAX_TEMP, bool(norm_vis_feat), threshold)
+
+    def _batch_prompts(self, vis_feats, counts, queries, qneg, method):
+        """The checks and the prompt tables of predict_many: (counts, mode, text, prompt_counts, pos, negs), or None for a
+        method predict does not know. Every distinct text of the batch is encoded in one encode_text call."""
         self._check_feats(vis_feats)
         counts = [int(c) for c in counts]
         scene_queries = [list(q) for q in queries]
@@ -236,7 +273,7 @@ class ClipSimilarity(object):
         elif method == "argmax":
             mode = _lib.DC_GROUND_ARGMAX
         else:
-            return [None] * len(counts)  # predict falls off the end of its if/elif chain
+            return None
         if mode == _lib.DC_GROUND_ARGMAX and any(n == 1 and q for n, q in zip(counts, scene_queries)):
             raise IndexError("too many indices for tensor of dimension 1")  # predict's behaviour (q18)
         if texts:
@@ -245,9 +282,7 @@ class ClipSimilarity(object):
             text = emb.index_select(0, torch.tensor(gather, dtype=torch.long, device=emb.device)).to(vis_feats.device)
         else:
             text = vis_feats.new_empty((0, vis_feats.shape[1]))
-        res = self._eng().predict_many(vis_feats, counts, text, prompt_counts, pos, None if qneg is None else negs, mode,
-                                       self.SOFTMAX_TEMP, bool(norm_vis_feat), threshold)
-        return [(pred.view(torch.bool), score) for score, pred in res]
+        return counts, mode, text, prompt_counts, pos, None if qneg is None else negs
 
 
 # ---------------------------------------------------------------------- a18

@@ -411,6 +411,30 @@ DC_API int dc_predict_many(void* feats, int feat_dtype, const void* text, int te
                            const int32_t* neg_off, const int32_t* neg_cols, int mode, float softmax_temp, int normalize,
                            float threshold, float* out, uint8_t* pred, void* workspace, size_t workspace_bytes,
                            dc_stream_t stream);
+/* dc_predict_many scored against per-point ground truth in ONE call, for the grounding evaluation (trainMetricPC
+ * utils/misc.py:21-50 after the query loop): the same launches up to the threshold pass, which counts instead of writing
+ * the predictions. For query q, inter[q] = |pred_q & gt_q| and uni[q] = |pred_q | gt_q|, where pred_q is row q of
+ * dc_predict_many's pred (the same bits) and gt_q[i] = (labels[i] is one of the query's ids) over the query's scene.
+ * Neither the scores nor the predictions are returned: they stay in the workspace.
+ *   feats, text, the offset tables, pos / neg_off / neg_cols, mode, softmax_temp, normalize, threshold: as in
+ *   dc_predict_many, with the same rules and limits (the rows of the scenes with queries are normalised in place).
+ *   labels [sum N] int32 (DC_I32) or int64 (DC_I64), device memory, in feature-row order; compared as int64.
+ *   gt_off [sum Q + 1] int32 and gt_ids [gt_off[sum Q]] int64 in HOST memory: query q's object ids are
+ *   gt_ids[gt_off[q] .. gt_off[q+1]), strictly ascending (an empty list: no point is ground truth). Checked on the host
+ *   before any launch (gt_off[0] == 0, gt_off does not decrease, ids ascend), then staged with the other tables.
+ *   inter / uni [sum Q] int64, device memory: zeroed first, so a query of an empty scene reports 0 / 0.
+ *   workspace: 256-byte aligned, dc_predict_many_iou_workspace() bytes, n_gt_total = gt_off[sum Q]. It holds
+ *   dc_predict_many's workspace plus the (sum Q_s * N_s) scores and argmax bytes.
+ * The call does not synchronise. */
+DC_API size_t dc_predict_many_iou_workspace(int n_scenes, const int64_t* point_off, const int32_t* prompt_off,
+                                            const int32_t* query_off, int64_t n_neg_total, int64_t n_gt_total, int dim,
+                                            int feat_dtype, int text_dtype);
+DC_API int dc_predict_many_iou(void* feats, int feat_dtype, const void* text, int text_dtype, int dim, int n_scenes,
+                               const int64_t* point_off, const int32_t* prompt_off, const int32_t* query_off,
+                               const int32_t* pos, const int32_t* neg_off, const int32_t* neg_cols, const void* labels,
+                               int label_dtype, const int32_t* gt_off, const int64_t* gt_ids, int mode, float softmax_temp,
+                               int normalize, float threshold, int64_t* inter, int64_t* uni, void* workspace,
+                               size_t workspace_bytes, dc_stream_t stream);
 
 /* Global min-max normalisation + threshold (models/similarity.py:83-88, :95-98):
  * values <- (v - min)/(max - min) (or v / max when the raw extrema coincide), pred = values > thr
