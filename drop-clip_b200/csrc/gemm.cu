@@ -807,6 +807,115 @@ __global__ void __launch_bounds__(256) minmax_threshold_kernel(float* __restrict
   }
 }
 
+constexpr int kSweepMaxThresholds = 1024;  // dc_predict_many_iou_sweep: two block histograms of <= 1025 bins, 8.2 KB
+
+// The threshold pass of dc_predict_many_iou_sweep: query row y = v [row_off[y], row_off[y + 1]) with its extrema and
+// ground truth as in the counting instances of minmax_threshold_kernel, and the same normalised score x. Instead of one
+// threshold, the U ascending distinct levels u[0 .. U): point i falls into bin k = #{j : x > u_j} (0 for a NaN x;
+// argmax: U when its byte is set, else 0), so x > u_r exactly when k > r. The block counts its points per (g, k) in
+// shared memory, with one shared atomic per group of lanes of a warp that share the bin (most points of a query fall
+// into one or two bins), and adds its non-zero bins to hist [n_queries][2][U + 1] (g = 0: not ground truth, 1: ground
+// truth; 32 bits, < 2^31 points per query).
+template <class Label>
+__global__ void __launch_bounds__(256) threshold_sweep_kernel(const float* __restrict__ v, const float* __restrict__ mm,
+                                                              int use_raw, int pred_from_thr,
+                                                              const uint8_t* __restrict__ pred,
+                                                              const int64_t* __restrict__ row_off,
+                                                              const float* __restrict__ levels, int n_levels, IouCount cnt,
+                                                              unsigned* __restrict__ hist) {
+  extern __shared__ unsigned s_sweep[];
+  const int bins = n_levels + 1;
+  unsigned* s_hist = s_sweep;                                  // [2][bins]
+  float* s_lv = reinterpret_cast<float*>(s_sweep + 2 * bins);  // [n_levels]
+  for (int j = threadIdx.x; j < 2 * bins; j += blockDim.x) s_hist[j] = 0;
+  for (int j = threadIdx.x; j < n_levels; j += blockDim.x) s_lv[j] = levels[j];
+  __syncthreads();
+  const int64_t o = row_off[blockIdx.y];
+  const int64_t n = row_off[blockIdx.y + 1] - o;
+  v += o;
+  pred += o;
+  mm += 4 * blockIdx.y;
+  const float mn = mm[0], mx = mm[1];
+  const bool differ = use_raw ? (mm[3] != mm[2]) : (mx != mn);
+  const float range = mx - mn;
+  const Label* __restrict__ labels = static_cast<const Label*>(cnt.labels) + cnt.point_row[blockIdx.y];
+  const int g0 = cnt.gt_off[blockIdx.y], n_ids = cnt.gt_off[blockIdx.y + 1] - g0;
+  const int64_t* __restrict__ ids = cnt.gt_ids + g0;
+  const int lane = threadIdx.x & 31;
+  // the loop runs warp-uniformly (lanes past the end take no bin), so every lane can join __match_any_sync
+  for (int64_t base = (int64_t)blockIdx.x * blockDim.x + (threadIdx.x - lane); base < n;
+       base += (int64_t)gridDim.x * blockDim.x) {
+    const int64_t i = base + lane;
+    int bin = -1;
+    if (i < n) {
+      int k;
+      if (pred_from_thr) {
+        float x = v[i];
+        x = differ ? (x - mn) / range : x / mx;
+        int lo = 0, hi = n_levels;  // k = #{j : u_j < x}: the comparison x > u_j, false for every u_j when x is NaN
+        while (lo < hi) {
+          const int mid = (lo + hi) >> 1;
+          if (s_lv[mid] < x) lo = mid + 1;
+          else hi = mid;
+        }
+        k = lo;
+      } else {
+        k = pred[i] != 0 ? n_levels : 0;
+      }
+      bin = id_listed((int64_t)__ldg(labels + i), ids, n_ids) ? bins + k : k;
+    }
+    const unsigned same = __match_any_sync(0xffffffffu, bin);
+    if (bin >= 0 && lane == __ffs(same) - 1) atomicAdd(s_hist + bin, (unsigned)__popc(same));
+  }
+  __syncthreads();
+  unsigned* h = hist + (int64_t)blockIdx.y * 2 * bins;
+  for (int j = threadIdx.x; j < 2 * bins; j += blockDim.x)
+    if (s_hist[j]) atomicAdd(h + j, s_hist[j]);
+}
+
+// The counts of dc_predict_many_iou_sweep from the histograms of threshold_sweep_kernel, one block per query q: with
+// r = rank[t], inter[t][q] = sum_{k > r} hist[q][1][k] and uni[t][q] = |gt_q| + sum_{k > r} hist[q][0][k], where
+// |gt_q| = sum_k hist[q][1][k]. One warp takes the suffix sums (each lane a run of bins), then the block writes T rows.
+__global__ void __launch_bounds__(256) sweep_counts_kernel(const unsigned* __restrict__ hist, int n_levels,
+                                                           const int* __restrict__ rank, int n_thr, int n_queries,
+                                                           int64_t* __restrict__ inter, int64_t* __restrict__ uni) {
+  extern __shared__ unsigned s_suffix[];  // [2][bins]: sum_{j >= k} hist[q][g][j]
+  const int bins = n_levels + 1;
+  const unsigned* h = hist + (int64_t)blockIdx.x * 2 * bins;
+  if (threadIdx.x < 32) {
+    const int lane = threadIdx.x;
+    const int run = (bins + 31) / 32;
+    const int j0 = min(bins, lane * run), j1 = min(bins, j0 + run);
+    unsigned sn = 0, sg = 0;
+    for (int j = j0; j < j1; ++j) {
+      sn += h[j];
+      sg += h[bins + j];
+    }
+    for (int d = 1; d < 32; d <<= 1) {  // inclusive suffix sums over the lanes
+      const unsigned an = __shfl_down_sync(0xffffffffu, sn, d), ag = __shfl_down_sync(0xffffffffu, sg, d);
+      if (lane + d < 32) {
+        sn += an;
+        sg += ag;
+      }
+    }
+    unsigned rn = __shfl_down_sync(0xffffffffu, sn, 1), rg = __shfl_down_sync(0xffffffffu, sg, 1);
+    if (lane == 31) rn = rg = 0;
+    for (int j = j1 - 1; j >= j0; --j) {
+      rn += h[j];
+      rg += h[bins + j];
+      s_suffix[j] = rn;
+      s_suffix[bins + j] = rg;
+    }
+  }
+  __syncthreads();
+  const unsigned gt = s_suffix[bins];
+  for (int t = threadIdx.x; t < n_thr; t += blockDim.x) {
+    const int k = rank[t] + 1;  // in [1, U]
+    inter[(int64_t)t * n_queries + blockIdx.x] = s_suffix[bins + k];
+    uni[(int64_t)t * n_queries + blockIdx.x] = gt + s_suffix[k];
+  }
+}
+
 __global__ void init_query_minmax_kernel(float* m, int n_slots) {
   for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < 4 * n_slots; i += gridDim.x * blockDim.x)
     m[i] = (i & 1) ? -INFINITY : INFINITY;
@@ -1190,14 +1299,18 @@ namespace {
 // staged in one host buffer and copied into the workspace by one cudaMemcpyAsync. A scene without queries gets no
 // blocks, no tiles and no normalisation.
 // dc_predict_many_iou also stages its ground-truth tables (query q's first feature row, gt_off, gt_ids) in the table
-// region, and keeps the scores and the argmax bytes in the workspace (`v`, `pred`).
+// region, and keeps the scores and the argmax bytes in the workspace (`v`, `pred`). dc_predict_many_iou_sweep adds its
+// threshold levels and ranks to the table region (room for n_thr each) and its histograms to the workspace (`hist`).
 struct ScorePlan {
-  size_t minmax, tables, t_planes, x_planes, sims, v, pred, total;                 // workspace byte offsets
+  size_t minmax, tables, t_planes, x_planes, sims, v, pred, hist, total;           // workspace byte offsets
   size_t t_qrow, t_pos, t_off, t_cols, t_scenes, t_blocks, t_counts, t_tiles;      // inside the table region
-  size_t t_qpoint, t_gt_off, t_gt_ids, t_bytes;
+  size_t t_qpoint, t_gt_off, t_gt_ids, t_levels, t_rank, t_bytes;
   int n_queries = 0, minmax_slots = 0, max_prompts = 1, s_ld = 0, tile_rows = 0;  // max_prompts: over the scenes with queries
   int64_t n_rows = 0, n_text_rows = 0, n_neg = 0, max_points = 0;  // max_points: over the scenes with queries
   int64_t n_gt = -1;              // dc_predict_many_iou: the number of ground-truth ids; -1: no counting
+  int n_thr = 0;                  // dc_predict_many_iou_sweep: the number of thresholds; 0: one threshold
+  std::vector<float> levels;      // sweep: the distinct threshold levels, ascending (threshold_levels)
+  std::vector<int> rank;          // sweep: [n_thr], threshold t's index in `levels`
   std::vector<int64_t> qrow_off;  // [n_queries + 1]: query q's row of v / pred
   std::vector<int64_t> qpoint;    // counting: [n_queries], the feature row of query q's first point
   std::vector<ScoreScene> scenes;
@@ -1209,16 +1322,17 @@ struct ScorePlan {
 // tile_list: dc_predict_many's GEMM (explicit tiles, S row stride = the widest scene rounded up to 4); otherwise
 // dc_ground writes S [n_points, n_prompts] of the one scene densely. reverse: list the first column block's tiles last
 // to first (the rows normalised last are still in L2, as in dc_ground). n_gt >= 0: the plan of dc_predict_many_iou with
-// n_gt ground-truth ids.
+// n_gt ground-truth ids; with n_thr > 0 as well, the plan of dc_predict_many_iou_sweep with n_thr thresholds.
 ScorePlan score_plan(int n_scenes, const int64_t* point_off, const int32_t* prompt_off, const int32_t* query_off,
                      int64_t n_neg, int dim, int feat_dtype, int text_dtype, bool tile_list, bool reverse,
-                     int64_t n_gt = -1) {
+                     int64_t n_gt = -1, int n_thr = 0) {
   ScorePlan pl;
   pl.n_rows = point_off[n_scenes];
   pl.n_text_rows = prompt_off[n_scenes];
   pl.n_queries = query_off[n_scenes];
   pl.n_neg = n_neg;
   pl.n_gt = n_gt;
+  pl.n_thr = n_thr;
   const bool count = n_gt >= 0;
   int& max_prompts = pl.max_prompts;
   int64_t out_off = 0;
@@ -1286,6 +1400,9 @@ ScorePlan score_plan(int n_scenes, const int64_t* point_off, const int32_t* prom
   pl.t_qpoint = t; if (count) t += align_up(sizeof(int64_t) * q, 16);
   pl.t_gt_off = t; if (count) t += align_up(sizeof(int) * (q + 1), 16);
   pl.t_gt_ids = t; if (count) t += sizeof(int64_t) * (size_t)n_gt;
+  if (n_thr > 0) t = align_up(t, 16);
+  pl.t_levels = t; t += sizeof(float) * (size_t)n_thr;
+  pl.t_rank = t; t += sizeof(int) * (size_t)n_thr;
   pl.t_bytes = t;
   pl.minmax_slots = pl.n_queries + (tile_list ? 0 : 1);  // + dc_ground's extrema, unused
   size_t off = 0;
@@ -1296,6 +1413,7 @@ ScorePlan score_plan(int n_scenes, const int64_t* point_off, const int32_t* prom
   pl.sims = off; off += align_up((size_t)(pl.n_rows > 0 ? pl.n_rows : 1) * pl.s_ld * sizeof(float), 256);
   pl.v = off; if (count) off += align_up(sizeof(float) * (size_t)out_off, 256);
   pl.pred = off; if (count) off += align_up((size_t)out_off, 256);
+  pl.hist = off; off += align_up(sizeof(unsigned) * 2 * (size_t)(n_thr > 0 ? n_thr + 1 : 0) * q, 256);
   pl.total = off;
   return pl;
 }
@@ -1346,13 +1464,17 @@ int stage_tables(const ScorePlan& pl, const int32_t* pos, const int32_t* neg_off
     put(pl.t_gt_off, gt_off, sizeof(int) * (q + 1));
     put(pl.t_gt_ids, gt_ids, sizeof(int64_t) * (size_t)pl.n_gt);
   }
+  put(pl.t_levels, pl.levels.data(), sizeof(float) * pl.levels.size());
+  put(pl.t_rank, pl.rank.data(), sizeof(int) * pl.rank.size());
   // pageable source: cudaMemcpyAsync returns once it has staged the bytes, so `h` may go out of scope
   DC_CUDA(cudaMemcpyAsync(ws + pl.tables, h.data(), pl.t_bytes, cudaMemcpyHostToDevice, st));
   return DC_OK;
 }
 
 // Every query scored from its columns of S [n_rows, s_ld], then its min-max and threshold (one launch each). With `cnt`
-// (dc_predict_many_iou) the second launch counts against the labels of dtype label_dtype instead of writing v and pred.
+// (dc_predict_many_iou) the second launch counts against the labels of dtype label_dtype instead of writing v and pred;
+// a sweep plan (dc_predict_many_iou_sweep) replaces it with threshold_sweep_kernel into the zeroed histograms, then
+// sweep_counts_kernel writes cnt.inter / cnt.uni [n_thr][n_queries].
 int score_queries(const ScorePlan& pl, uint8_t* ws, int mode, float softmax_temp, float threshold, float* out,
                   uint8_t* pred, cudaStream_t st, const IouCount* cnt = nullptr, int label_dtype = DC_I64) {
   if (pl.blocks.empty()) return DC_OK;
@@ -1387,7 +1509,22 @@ int score_queries(const ScorePlan& pl, uint8_t* ws, int mode, float softmax_temp
   const int64_t per_query = std::max<int64_t>(1, dc::ceil_div<int64_t>((int64_t)dc::sm_count() * 8, pl.n_queries));
   const dim3 mm_grid((unsigned)std::min(blocks_x, per_query), (unsigned)pl.n_queries);
   const int use_raw = mode == DC_GROUND_ARGMAX ? 1 : 0, pred_from_thr = mode == DC_GROUND_ARGMAX ? 0 : 1;
-  if (!cnt)
+  if (pl.n_thr > 0) {
+    const int n_levels = (int)pl.levels.size();
+    const float* levels = reinterpret_cast<const float*>(tb + pl.t_levels);
+    unsigned* hist = reinterpret_cast<unsigned*>(ws + pl.hist);
+    const size_t sweep_smem = sizeof(unsigned) * 2 * (n_levels + 1) + sizeof(float) * n_levels;
+    if (label_dtype == DC_I32)
+      threshold_sweep_kernel<int32_t><<<mm_grid, 256, sweep_smem, st>>>(out, minmax, use_raw, pred_from_thr, pred, qrow,
+                                                                        levels, n_levels, *cnt, hist);
+    else
+      threshold_sweep_kernel<int64_t><<<mm_grid, 256, sweep_smem, st>>>(out, minmax, use_raw, pred_from_thr, pred, qrow,
+                                                                        levels, n_levels, *cnt, hist);
+    DC_LAUNCH_CHECK();
+    sweep_counts_kernel<<<(unsigned)pl.n_queries, 256, sizeof(unsigned) * 2 * (n_levels + 1), st>>>(
+        hist, n_levels, reinterpret_cast<const int*>(tb + pl.t_rank), pl.n_thr, pl.n_queries,
+        reinterpret_cast<int64_t*>(cnt->inter), reinterpret_cast<int64_t*>(cnt->uni));
+  } else if (!cnt)
     minmax_threshold_kernel<void><<<mm_grid, 256, 0, st>>>(out, 0, minmax, use_raw, threshold, pred_from_thr, pred, qrow);
   else if (label_dtype == DC_I32)
     minmax_threshold_kernel<int32_t><<<mm_grid, 256, 0, st>>>(out, 0, minmax, use_raw, threshold, pred_from_thr, pred, qrow,
@@ -1481,7 +1618,8 @@ int dc_predict_queries(void* feats, int feat_dtype, int64_t n_points, const void
 
 namespace {
 
-// The ground-truth side of dc_predict_many_iou.
+// The ground-truth side of dc_predict_many_iou; with n_thresholds > 0, of dc_predict_many_iou_sweep (inter / uni are
+// then [n_thresholds][sum Q]).
 struct IouArgs {
   const void* labels;
   int label_dtype;
@@ -1489,17 +1627,39 @@ struct IouArgs {
   const int64_t* gt_ids;
   int64_t* inter;
   int64_t* uni;
+  const float* thresholds;
+  int n_thresholds;
 };
 
 size_t predict_many_workspace(int n_scenes, const int64_t* point_off, const int32_t* prompt_off, const int32_t* query_off,
-                              int64_t n_neg_total, int dim, int feat_dtype, int text_dtype, int64_t n_gt) {
+                              int64_t n_neg_total, int dim, int feat_dtype, int text_dtype, int64_t n_gt, int n_thr = 0) {
   if (n_scenes < 0 || (n_scenes > 0 && !(point_off && prompt_off && query_off))) return 0;
   const int64_t zero64 = 0;
   const int32_t zero32 = 0;
   if (n_scenes == 0)
-    return score_plan(0, &zero64, &zero32, &zero32, 0, dim, feat_dtype, text_dtype, true, false, n_gt >= 0 ? 0 : -1).total;
+    return score_plan(0, &zero64, &zero32, &zero32, 0, dim, feat_dtype, text_dtype, true, false, n_gt >= 0 ? 0 : -1,
+                      n_thr).total;
   return score_plan(n_scenes, point_off, prompt_off, query_off, n_neg_total, dim, feat_dtype, text_dtype, true, false,
-                    n_gt).total;
+                    n_gt, n_thr).total;
+}
+
+int check_thresholds(const char* fn, const float* thresholds, int n_thresholds) {
+  DC_CHECK_ARG(n_thresholds >= 1 && n_thresholds <= kSweepMaxThresholds, "%s: 1..%d thresholds (got %d)", fn,
+               kSweepMaxThresholds, n_thresholds);
+  DC_CHECK_ARG(thresholds, "%s: null pointer argument", fn);
+  return DC_OK;
+}
+
+// The sweep's threshold tables: the distinct values of thresholds[0 .. n) ascending, a NaN as +inf (x > NaN and
+// x > +inf are false for every x), and rank[t] = the index of entry t's value among them. -0 and +0 are one level.
+void threshold_levels(const float* thresholds, int n, std::vector<float>& levels, std::vector<int>& rank) {
+  std::vector<float> vals(n);
+  for (int t = 0; t < n; ++t) vals[t] = thresholds[t] != thresholds[t] ? INFINITY : thresholds[t];
+  levels = vals;
+  std::sort(levels.begin(), levels.end());
+  levels.erase(std::unique(levels.begin(), levels.end()), levels.end());
+  rank.resize(n);
+  for (int t = 0; t < n; ++t) rank[t] = (int)(std::lower_bound(levels.begin(), levels.end(), vals[t]) - levels.begin());
 }
 
 // dc_predict_many (iou == nullptr: the scores and predictions go to out / pred) and dc_predict_many_iou (the scores and
@@ -1559,15 +1719,19 @@ int predict_many(const char* fn, void* feats, int feat_dtype, const void* text, 
   }
   if (n_queries == 0) return DC_OK;
   cudaStream_t st = dc::as_stream(stream);
-  const ScorePlan pl = score_plan(n_scenes, point_off, prompt_off, query_off, neg_off[n_queries], dim, feat_dtype,
-                                  text_dtype, true, feat_dtype == DC_F16 && normalize, n_gt);
+  const int n_thr = iou ? iou->n_thresholds : 0;
+  ScorePlan pl = score_plan(n_scenes, point_off, prompt_off, query_off, neg_off[n_queries], dim, feat_dtype, text_dtype,
+                            true, feat_dtype == DC_F16 && normalize, n_gt, n_thr);
   if (workspace_bytes < pl.total) return dc::fail(DC_ERR_WORKSPACE, "%s: workspace %zu < %zu", fn, workspace_bytes, pl.total);
+  if (n_thr > 0) threshold_levels(iou->thresholds, n_thr, pl.levels, pl.rank);
   uint8_t* ws = static_cast<uint8_t*>(workspace);
   IouCount cnt{};
   if (iou) {
     // every query reports 0 / 0 until its blocks add to it (a query of an empty scene gets none)
-    DC_CUDA(cudaMemsetAsync(iou->inter, 0, sizeof(int64_t) * n_queries, st));
-    DC_CUDA(cudaMemsetAsync(iou->uni, 0, sizeof(int64_t) * n_queries, st));
+    const size_t rows = (size_t)std::max(n_thr, 1) * n_queries;
+    DC_CUDA(cudaMemsetAsync(iou->inter, 0, sizeof(int64_t) * rows, st));
+    DC_CUDA(cudaMemsetAsync(iou->uni, 0, sizeof(int64_t) * rows, st));
+    if (n_thr > 0) DC_CUDA(cudaMemsetAsync(ws + pl.hist, 0, sizeof(unsigned) * 2 * (pl.levels.size() + 1) * n_queries, st));
     out = reinterpret_cast<float*>(ws + pl.v);
     pred = ws + pl.pred;
     const uint8_t* tb = ws + pl.tables;
@@ -1661,6 +1825,41 @@ int dc_predict_many_iou(void* feats, int feat_dtype, const void* text, int text_
   return predict_many("dc_predict_many_iou", feats, feat_dtype, text, text_dtype, dim, n_scenes, point_off, prompt_off,
                       query_off, pos, neg_off, neg_cols, mode, softmax_temp, normalize, threshold, nullptr, nullptr, &iou,
                       workspace, workspace_bytes, stream);
+}
+
+size_t dc_predict_many_iou_sweep_workspace(int n_scenes, const int64_t* point_off, const int32_t* prompt_off,
+                                           const int32_t* query_off, int64_t n_neg_total, int64_t n_gt_total,
+                                           int n_thresholds, int dim, int feat_dtype, int text_dtype) {
+  if (n_thresholds < 1 || n_thresholds > kSweepMaxThresholds) return 0;
+  return predict_many_workspace(n_scenes, point_off, prompt_off, query_off, n_neg_total, dim, feat_dtype, text_dtype,
+                                n_gt_total > 0 ? n_gt_total : 0, n_thresholds);
+}
+
+int dc_predict_many_iou_sweep(void* feats, int feat_dtype, const void* text, int text_dtype, int dim, int n_scenes,
+                              const int64_t* point_off, const int32_t* prompt_off, const int32_t* query_off,
+                              const int32_t* pos, const int32_t* neg_off, const int32_t* neg_cols, const void* labels,
+                              int label_dtype, const int32_t* gt_off, const int64_t* gt_ids, int mode, float softmax_temp,
+                              int normalize, const float* thresholds, int n_thresholds, int64_t* inter, int64_t* uni,
+                              void* workspace, size_t workspace_bytes, dc_stream_t stream) {
+  int rc;
+  if ((rc = check_thresholds("dc_predict_many_iou_sweep", thresholds, n_thresholds))) return rc;
+  const IouArgs iou{labels, label_dtype, gt_off, gt_ids, inter, uni, thresholds, n_thresholds};
+  return predict_many("dc_predict_many_iou_sweep", feats, feat_dtype, text, text_dtype, dim, n_scenes, point_off,
+                      prompt_off, query_off, pos, neg_off, neg_cols, mode, softmax_temp, normalize, 0.f, nullptr, nullptr,
+                      &iou, workspace, workspace_bytes, stream);
+}
+
+int dc_sweep_levels(const float* thresholds, int n_thresholds, float* levels, int32_t* rank, int* n_levels) {
+  int rc;
+  if ((rc = check_thresholds("dc_sweep_levels", thresholds, n_thresholds))) return rc;
+  DC_CHECK_ARG(levels && rank && n_levels, "dc_sweep_levels: null pointer argument");
+  std::vector<float> lv;
+  std::vector<int> rk;
+  threshold_levels(thresholds, n_thresholds, lv, rk);
+  std::copy(lv.begin(), lv.end(), levels);
+  std::copy(rk.begin(), rk.end(), rank);
+  *n_levels = (int)lv.size();
+  return DC_OK;
 }
 
 int dc_minmax_threshold(float* values, int64_t n, const float* minmax, int use_raw_extrema_for_test, float threshold,

@@ -105,6 +105,24 @@ def gt_csr(gt_ids, q_counts, label_dtype):
     return off.astype(np.int32), ids
 
 
+SWEEP_MAX_THRESHOLDS = 1024  # dc_predict_many_iou_sweep's limit
+_NO_DEFAULT = object()
+
+
+def threshold_table(thresholds, default=_NO_DEFAULT):
+    """Host threshold table of FusionEngine.predict_many_iou_sweep: fp32 [T] in the caller's order, each entry rounded
+    to fp32 as a threshold argument of the scalar calls is (the kernels compare in fp32). With `default` given, a falsy
+    entry (0, 0.0, None) stands for it, as `threshold or self.threshold` does in ClipSimilarity. ValueError for no
+    entries or more than SWEEP_MAX_THRESHOLDS."""
+    thresholds = list(thresholds)
+    if not 1 <= len(thresholds) <= SWEEP_MAX_THRESHOLDS:
+        raise ValueError(f"1..{SWEEP_MAX_THRESHOLDS} thresholds (got {len(thresholds)})")
+    if default is not _NO_DEFAULT:
+        thresholds = [t or default for t in thresholds]
+    with np.errstate(over="ignore"):  # beyond fp32: +-inf, as ctypes.c_float rounds it
+        return np.array([float(t) for t in thresholds], dtype=np.float64).astype(np.float32)
+
+
 def intrinsic_matrix(intr: Dict[str, float]) -> np.ndarray:
     """utils/feature_fusion.py:35-40, always promoted to fp64 (K @ fp64 points is fp64 anyway)."""
     return np.asarray([[intr["fx"], 0, intr["cx"]], [0, intr["fy"], intr["cy"]], [0, 0, 1]], dtype=np.float64)
@@ -1070,6 +1088,23 @@ class FusionEngine:
         gt_ids[s][q]). labels (sum N,) int32 / int64 CUDA tensor in feature-row order; gt_ids[s][q] any iterable of ints
         (sorted and deduplicated here). Every index, count, mode, label and id rule is checked before anything reaches
         the device; an id outside the label dtype's range raises ValueError."""
+        return self._many_iou(feats, counts, text, prompt_counts, pos, neg_lists, labels, gt_ids, mode, softmax_temp,
+                              normalize, threshold, None)
+
+    def predict_many_iou_sweep(self, feats: torch.Tensor, counts, text: torch.Tensor, prompt_counts, pos, neg_lists,
+                               labels, gt_ids, mode: int, softmax_temp: float, normalize: bool, thresholds):
+        """predict_many_iou at every threshold of `thresholds` in one library call: (inter, union) int64 CUDA tensors of
+        shape (T, sum Q), row t equal to predict_many_iou(feats.clone(), ..., threshold=thresholds[t]) on the features
+        as passed. thresholds: 1..SWEEP_MAX_THRESHOLDS numbers in any order (threshold_table: fp32, duplicates, +-inf and
+        NaN allowed). The features are normalised in place once, as by one predict_many_iou call. Every check, the
+        threshold table's included, runs before anything reaches the device."""
+        thr = threshold_table(thresholds)
+        return self._many_iou(feats, counts, text, prompt_counts, pos, neg_lists, labels, gt_ids, mode, softmax_temp,
+                              normalize, None, thr)
+
+    def _many_iou(self, feats, counts, text, prompt_counts, pos, neg_lists, labels, gt_ids, mode, softmax_temp, normalize,
+                  threshold, thr):
+        """predict_many_iou (thr None: one threshold) or predict_many_iou_sweep (thr: fp32 [T])."""
         tb = self._batch_tables(feats, counts, text, prompt_counts, pos, neg_lists, mode)
         counts, q_counts = tb["counts"], tb["q_counts"]
         if not isinstance(labels, torch.Tensor) or labels.dtype not in (torch.int32, torch.int64):
@@ -1081,7 +1116,7 @@ class FusionEngine:
         gt_off, ids = gt_csr(gt_ids, q_counts, labels.dtype)
         s_n, n_q = len(counts), sum(q_counts)
         dev = feats.device
-        res = torch.empty((2, n_q), dtype=torch.int64, device=dev)
+        res = torch.empty((2, n_q) if thr is None else (2, thr.size, n_q), dtype=torch.int64, device=dev)
         if n_q == 0:
             return res[0], res[1]
         labels = labels.reshape(-1).contiguous()
@@ -1092,16 +1127,22 @@ class FusionEngine:
         fcode, tcode = _lib.torch_dtype_code(feats.dtype), _lib.torch_dtype_code(text.dtype)
         c_p = lambda a: a.ctypes.data_as(ctypes.c_void_p)  # noqa: E731
         cols = tb["neg_cols"]
-        ws_bytes = self.lib.dc_predict_many_iou_workspace(s_n, c_p(tb["point_off"]), c_p(tb["prompt_off"]),
-                                                          c_p(tb["query_off"]), int(cols.size), int(ids.size), dim, fcode, tcode)
+        tables = (s_n, c_p(tb["point_off"]), c_p(tb["prompt_off"]), c_p(tb["query_off"]), int(cols.size), int(ids.size))
+        if thr is None:
+            ws_bytes = self.lib.dc_predict_many_iou_workspace(*tables, dim, fcode, tcode)
+        else:
+            ws_bytes = self.lib.dc_predict_many_iou_sweep_workspace(*tables, thr.size, dim, fcode, tcode)
         ws = torch.empty(ws_bytes + 256, dtype=torch.uint8, device=dev)
         shift = (-ws.data_ptr()) % 256
-        check(self.lib.dc_predict_many_iou(
-            ptr(feats) if n_total else None, fcode, ptr(text) if text.shape[0] else None, tcode, dim, s_n, c_p(tb["point_off"]),
-            c_p(tb["prompt_off"]), c_p(tb["query_off"]), c_p(tb["pos"]), c_p(tb["neg_off"]), c_p(cols) if cols.size else None,
-            ptr(labels) if n_total else None, _lib.torch_dtype_code(labels.dtype), c_p(gt_off), c_p(ids) if ids.size else None,
-            mode, float(softmax_temp), int(bool(normalize)), float(threshold), ptr(res[0]), ptr(res[1]),
-            ctypes.c_void_p(ws.data_ptr() + shift), ws_bytes, current_stream()))
+        args = (ptr(feats) if n_total else None, fcode, ptr(text) if text.shape[0] else None, tcode, dim, s_n,
+                c_p(tb["point_off"]), c_p(tb["prompt_off"]), c_p(tb["query_off"]), c_p(tb["pos"]), c_p(tb["neg_off"]),
+                c_p(cols) if cols.size else None, ptr(labels) if n_total else None, _lib.torch_dtype_code(labels.dtype),
+                c_p(gt_off), c_p(ids) if ids.size else None, mode, float(softmax_temp), int(bool(normalize)))
+        tail = (ptr(res[0]), ptr(res[1]), ctypes.c_void_p(ws.data_ptr() + shift), ws_bytes, current_stream())
+        if thr is None:
+            check(self.lib.dc_predict_many_iou(*args, float(threshold), *tail))
+        else:
+            check(self.lib.dc_predict_many_iou_sweep(*args, c_p(thr), thr.size, *tail))
         return res[0], res[1]
 
     def minmax_threshold(self, values, minmax, use_raw: bool, threshold: float, want_pred: bool):

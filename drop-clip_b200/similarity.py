@@ -14,7 +14,7 @@ from __future__ import annotations
 import torch
 
 from . import _lib
-from .engine import FusionEngine
+from .engine import FusionEngine, threshold_table
 
 DEVICE = torch.device("cuda")  # the reference's expression always evaluates to 'cuda' (quirk q20)
 
@@ -243,8 +243,29 @@ class ClipSimilarity(object):
         labels (sum N,) int32 / int64 CUDA tensor in feature-row order. Defaults, the in-place normalisation and the
         errors follow predict_many, and every error is raised before any row changes; ValueError also for labels of
         another dtype or count, and for an id outside the labels' dtype. None for a method predict does not know."""
+        return self._many_iou("predict_many_iou", vis_feats, counts, labels, obj_queries, qneg, norm_vis_feat, method,
+                              threshold or self.threshold)
+
+    @torch.no_grad()
+    def predict_many_iou_sweep(self, vis_feats, counts, labels, obj_queries, thresholds, qneg="scene", norm_vis_feat=None,
+                               method=None):
+        """predict_many_iou at many thresholds in one library call, to choose the threshold on a validation set or to
+        report mIoU / Pr@k against it: returns (inter, union), int64 CUDA tensors of shape (T, sum Q). Row t equals
+        predict_many_iou(vis_feats.clone(), counts, labels, obj_queries, qneg, norm_vis_feat, method,
+        threshold=thresholds[t]) on the rows as passed, and metrics.grounding_scores(inter[t], union[t]) gives that
+        call's mIoU and Pr@k. Everything before the threshold comparison (normalisation, GEMM, scoring, min-max) runs
+        once. thresholds: 1..1024 numbers in the caller's order, duplicates allowed; a falsy entry (0, 0.0, None) means
+        self.threshold, as for the single call, and each entry is rounded to fp32 as the single call rounds it. A NaN or
+        +inf entry predicts no point (inter 0, union |gt|); -inf every point whose score is not NaN. With method
+        "argmax" every row is the same. Defaults, the in-place normalisation (done once), empty scenes and the errors
+        follow predict_many_iou; ValueError also for no thresholds or more than 1024, raised before any row changes."""
+        return self._many_iou("predict_many_iou_sweep", vis_feats, counts, labels, obj_queries, qneg, norm_vis_feat,
+                              method, threshold_table(thresholds, self.threshold))
+
+    def _many_iou(self, fn, vis_feats, counts, labels, obj_queries, qneg, norm_vis_feat, method, threshold):
+        """FusionEngine.predict_many_iou / predict_many_iou_sweep (`fn`) at `threshold` (one or a table) from the
+        reference's text -> ids mappings; None for a method predict does not know."""
         method = method or self.method
-        threshold = threshold or self.threshold
         norm_vis_feat = norm_vis_feat or self.norm_vis_feat
         obj_queries = [dict(o) for o in obj_queries]
         batch = self._batch_prompts(vis_feats, counts, [list(o) for o in obj_queries], qneg, method)
@@ -252,8 +273,8 @@ class ClipSimilarity(object):
             return None  # predict falls off the end of its if/elif chain
         counts, mode, text, prompt_counts, pos, negs = batch
         gt_ids = [[list(ids) for ids in o.values()] for o in obj_queries]
-        return self._eng().predict_many_iou(vis_feats, counts, text, prompt_counts, pos, negs, labels, gt_ids, mode,
-                                            self.SOFTMAX_TEMP, bool(norm_vis_feat), threshold)
+        return getattr(self._eng(), fn)(vis_feats, counts, text, prompt_counts, pos, negs, labels, gt_ids, mode,
+                                        self.SOFTMAX_TEMP, bool(norm_vis_feat), threshold)
 
     def _batch_prompts(self, vis_feats, counts, queries, qneg, method):
         """The checks and the prompt tables of predict_many: (counts, mode, text, prompt_counts, pos, negs), or None for a

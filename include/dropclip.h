@@ -435,6 +435,33 @@ DC_API int dc_predict_many_iou(void* feats, int feat_dtype, const void* text, in
                                int label_dtype, const int32_t* gt_off, const int64_t* gt_ids, int mode, float softmax_temp,
                                int normalize, float threshold, int64_t* inter, int64_t* uni, void* workspace,
                                size_t workspace_bytes, dc_stream_t stream);
+/* dc_predict_many_iou at many thresholds in ONE call, for choosing the threshold or reporting mIoU / Pr@k against it:
+ * everything up to the threshold pass runs once. Row t of inter / uni equals, bit for bit, what dc_predict_many_iou
+ * returns with threshold = thresholds[t] on the same (unnormalised) inputs. The pass bins each point by how many of the
+ * distinct thresholds its normalised score exceeds, so its cost per point does not grow with n_thresholds.
+ *   Every argument as in dc_predict_many_iou, with the same rules and limits, except:
+ *   thresholds [n_thresholds] fp32 in HOST memory, 1 <= n_thresholds <= 1024, in any order; duplicates, +-inf and NaN
+ *   allowed (x > NaN is false: a NaN threshold predicts no point, like +inf). Argmax ignores them: every row is equal.
+ *   inter / uni [n_thresholds * sum Q] int64, device memory, row-major by threshold (row t = thresholds[t]), zeroed by
+ *   the call.
+ *   workspace: 256-byte aligned, dc_predict_many_iou_sweep_workspace() bytes (0 for n_thresholds outside 1..1024):
+ *   dc_predict_many_iou's workspace plus two tables of n_thresholds 4-byte entries and 8 * (n_thresholds + 1) bytes
+ *   of histograms per query, each region rounded up to 256 bytes.
+ * Host-side checks happen before any launch. The call does not synchronise. */
+DC_API size_t dc_predict_many_iou_sweep_workspace(int n_scenes, const int64_t* point_off, const int32_t* prompt_off,
+                                                  const int32_t* query_off, int64_t n_neg_total, int64_t n_gt_total,
+                                                  int n_thresholds, int dim, int feat_dtype, int text_dtype);
+DC_API int dc_predict_many_iou_sweep(void* feats, int feat_dtype, const void* text, int text_dtype, int dim, int n_scenes,
+                                     const int64_t* point_off, const int32_t* prompt_off, const int32_t* query_off,
+                                     const int32_t* pos, const int32_t* neg_off, const int32_t* neg_cols,
+                                     const void* labels, int label_dtype, const int32_t* gt_off, const int64_t* gt_ids,
+                                     int mode, float softmax_temp, int normalize, const float* thresholds,
+                                     int n_thresholds, int64_t* inter, int64_t* uni, void* workspace,
+                                     size_t workspace_bytes, dc_stream_t stream);
+/* The host table dc_predict_many_iou_sweep stages (pure host code, no device needed): levels[0 .. *n_levels) are the
+ * distinct values of thresholds[0 .. n_thresholds) ascending, with NaN taken as +inf and -0 and +0 one level, and rank[t]
+ * is the index of entry t's level. levels and rank have room for n_thresholds entries; 1 <= n_thresholds <= 1024. */
+DC_API int dc_sweep_levels(const float* thresholds, int n_thresholds, float* levels, int32_t* rank, int* n_levels);
 
 /* Global min-max normalisation + threshold (models/similarity.py:83-88, :95-98):
  * values <- (v - min)/(max - min) (or v / max when the raw extrema coincide), pred = values > thr
