@@ -742,6 +742,17 @@ class FusionEngine:
         """Drops never-visible points. Returns (new_index, kept_off (device), kept_off (host), mask offsets
         (host), compacted mask, compacted rows). `out_dtype=torch.int64` widens a uint8 mask while
         compacting (the reference's visibility mask is int64)."""
+        new_index, kept_off = self.compact_scan(b, any_vis)
+        kept_host = kept_off.cpu().numpy()  # sizes of the outputs: one small D2H, like the reference's .cpu() at :278
+        n_kept = np.diff(kept_host)
+        out_off_host = _prefix([v * k for v, k in zip(b.n_views, n_kept)])
+        out_off = torch.from_numpy(out_off_host).to(b.device)
+        cmask = self._compact_mask(b, mask, any_vis, new_index, kept_off, out_off, int(out_off_host[-1]), out_dtype)
+        rows_out = [self.compact_rows(t, any_vis, new_index, int(kept_host[-1])) for t in extra_rows]
+        return new_index, kept_off, kept_host, out_off_host, cmask, rows_out
+
+    def compact_scan(self, b: SceneBatch, any_vis):
+        """The scan every compaction starts with: (new_index [sum N] i64, kept_off [S+1] i64), both on the device."""
         n = b.total_points
         new_index = torch.empty(max(n, 1), dtype=torch.int64, device=b.device)
         kept_off = torch.empty(b.n_scenes + 1, dtype=torch.int64, device=b.device)
@@ -750,30 +761,35 @@ class FusionEngine:
         check(self.lib.dc_compact_scan(ptr(any_vis), n, ptr(b.off["point"]), b.n_scenes, ptr(new_index), ptr(kept_off),
                                        ptr(ws), ws_bytes, current_stream()))
         self.launches += 4
-        kept_host = kept_off.cpu().numpy()  # sizes of the outputs: one small D2H, like the reference's .cpu() at :278
-        n_kept = np.diff(kept_host)
-        out_off_host = _prefix([v * k for v, k in zip(b.n_views, n_kept)])
-        out_off = torch.from_numpy(out_off_host).to(b.device)
+        return new_index, kept_off
+
+    def _compact_mask(self, b: SceneBatch, mask, any_vis, new_index, kept_off, out_off, n_out: int, out_dtype=None):
+        """Mask-layout array (elements of 1, 4 or 8 bytes) compacted into `n_out` elements at the device offsets
+        `out_off`; `out_dtype=torch.int64` widens a uint8 mask."""
         widen = out_dtype is not None and out_dtype != mask.dtype
         if widen and not (mask.dtype == torch.uint8 and out_dtype == torch.int64):
             raise ValueError("compact: only uint8 -> int64 widening is supported")
-        n_mask = int(out_off_host[-1])
-        cmask_buf = torch.empty(max(n_mask, 1), dtype=out_dtype if widen else mask.dtype, device=b.device)
+        out_buf = torch.empty(max(n_out, 1), dtype=out_dtype if widen else mask.dtype, device=b.device)
         check(self.lib.dc_compact_mask(ptr(mask), 18 if widen else mask.element_size(), ptr(b.off["mask"]), ptr(b.off["point"]),
                                        ptr(b.off["view"]), ptr(any_vis), ptr(new_index), ptr(kept_off), ptr(out_off),
-                                       b.n_scenes, max(b.n_points, default=0), max(b.n_views, default=0), ptr(cmask_buf),
+                                       b.n_scenes, max(b.n_points, default=0), max(b.n_views, default=0), ptr(out_buf),
                                        current_stream()))
         self.launches += 1
-        cmask = cmask_buf[:n_mask]
-        rows_out = []
-        for t in extra_rows:
-            t2 = t.reshape(n, -1)
-            o_buf = torch.empty((max(int(kept_host[-1]), 1), t2.shape[1]), dtype=t.dtype, device=b.device)
-            check(self.lib.dc_compact_rows(ptr(t2), t2.shape[1] * t2.element_size(), ptr(any_vis), ptr(new_index), n,
-                                           ptr(o_buf), current_stream()))
-            self.launches += 1
-            rows_out.append(o_buf[:int(kept_host[-1])])
-        return new_index, kept_off, kept_host, out_off_host, cmask, rows_out
+        return out_buf[:n_out]
+
+    def compact_unsized(self, b: SceneBatch, any_vis, masks: Sequence[tuple] = (), rows: Sequence[torch.Tensor] = ()):
+        """`compact` without reading anything back: every output is allocated for all points kept and laid out from the
+        device's kept counts, so once kept_off is on the host, scene s's (V_s, K_s) mask block starts at
+        sum_{t<s} V_t K_t and its rows at kept_off[s]. `masks` holds (mask, out_dtype) pairs, out_dtype as in `compact`.
+        Returns (kept_off (device), compacted masks, compacted rows)."""
+        new_index, kept_off = self.compact_scan(b, any_vis)
+        out_off = torch.empty(b.n_scenes + 1, dtype=torch.int64, device=b.device)
+        check(self.lib.dc_compact_mask_offsets(ptr(kept_off), ptr(b.off["view"]), b.n_scenes, ptr(out_off), current_stream()))
+        self.launches += 1
+        n_mask = int(b.off_host["mask"][-1])
+        masks_out = [self._compact_mask(b, m, any_vis, new_index, kept_off, out_off, n_mask, dt) for m, dt in masks]
+        rows_out = [self.compact_rows(t, any_vis, new_index, b.total_points) for t in rows]
+        return kept_off, masks_out, rows_out
 
     # ------------------------------------------------------------------ whole object-level pass
     def fuse_object_level(self, b: SceneBatch, threshold=0.05, use_visibility=False, use_similarity=True,

@@ -144,44 +144,78 @@ class MultiviewFeatureFusion:
         eng = self._eng(device)
         if self.use_similarity:
             assert query_embeddings is not None, "Must provide query embeddings for using similarity."
-        out = self._aggregate(eng, points, depths, seg_masks, camera_poses, mv_features, query_embeddings)
+        b = self._pixel_batch(eng, self._staging, points, depths, seg_masks, camera_poses, mv_features, query_embeddings)
+        mask, _, _ = eng.visibility(b, self.visibility_threshold, torch.uint8)
+        sums, weight = eng.pixel_fuse(b, mask, self._sim_kernel(), self.norm_feat)
         n_views, n_pts = len(depths), points.shape[0]
-        vis = out["mask"].view(n_views, n_pts).to(torch.int64)
-        simw = out["weight"].view(n_views, n_pts) if self.use_similarity else None
-        return out["sum"], vis, simw
+        vis = mask.view(n_views, n_pts).to(torch.int64)
+        simw = weight.view(n_views, n_pts) if self.use_similarity else None
+        return sums, vis, simw
 
-    def _aggregate(self, eng, points, depths, seg_masks, camera_poses, mv_features, query_embeddings, normalize=False):
+    def _pixel_batch(self, eng, staging, points, depths, seg_masks, camera_poses, mv_features, query_embeddings):
+        """Host -> device upload of one scene with its patch maps (pinned staging, async H2D on the current stream).
+        The reference normalises its own upsampled copy of the maps under norm_feat, so nothing is written back."""
         segs = [s.cpu().numpy() if isinstance(s, torch.Tensor) else s for s in seg_masks]
         feats = [f.float() for f in mv_features]
         assert feats[0].shape[-1] == self.feature_size
         q = query_embeddings if self.use_similarity else None
-        b = SceneBatch.from_host([self._scene(points, depths, camera_poses, None, segs, feats, q)], eng.device,
-                                 pixel_features=True, staging=self._staging)
+        return SceneBatch.from_host([self._scene(points, depths, camera_poses, None, segs, feats, q)], eng.device,
+                                    pixel_features=True, staging=staging)
+
+    def _stage_pix(self, eng, staging, points, colors, labels, depths, seg_masks, camera_poses, mv_features, query_embeddings):
+        """Staging half of fuse_points: the scene and the rows it hands back, uploaded on the current stream."""
+        b = self._pixel_batch(eng, staging, points, depths, seg_masks, camera_poses, mv_features, query_embeddings)
+        self._stage_rows(b, staging, points, colors, labels)
+        return b
+
+    def _finish_pix(self, eng, b, points, colors, labels):
+        """Finishing half of fuse_points on the current stream. Every compaction is enqueued at its upper bound (all
+        points kept) and laid out from the kept count on the device, so the one host wait, for that count, also covers
+        the read-back of the returned rows."""
+        n_views = b.total_views
+        kern = self._sim_kernel()
+        host_rows = {"points": points, "colors": colors, "labels": labels}
+        if b.total_points == 0:  # an empty cloud: the projection and fusion launches need at least one point
+            feats = torch.empty((0, int(b.feats.shape[-1])), dtype=torch.float32, device=b.device)
+            vis = torch.empty((n_views, 0), dtype=torch.int64, device=b.device)
+            simw = torch.empty((n_views, 0), dtype=torch.float32, device=b.device) if kern is not None else None
+            keep = np.zeros(0, dtype=bool)
+            return (feats, vis, simw), tuple(arr[keep] for arr in host_rows.values())
         mask, any_vis, _ = eng.visibility(b, self.visibility_threshold, torch.uint8)
-        sums, weight = eng.pixel_fuse(b, mask, self._sim_kernel(), self.norm_feat, normalize=normalize)
-        if self.norm_feat:
-            # the reference normalises the caller's upsampled copy, not mv_features itself: nothing to write back
-            pass
-        return {"batch": b, "mask": mask, "any": any_vis, "sum": sums, "weight": weight}
+        # the division by sum_v visibility / sum_v similarity (:266-268) is fused into the fusion kernel
+        sums, weight = eng.pixel_fuse(b, mask, kern, self.norm_feat, normalize=True)
+        masks = [(mask, torch.int64)] + ([(weight.view(torch.int32), None)] if weight is not None else [])
+        dev_rows = b.row_sources
+        names = list(dev_rows)
+        kept_off, masks_out, rows_out = eng.compact_unsized(b, any_vis, masks, [sums] + [dev_rows[k] for k in names])
+        kept_host = self._pinned_like(kept_off)
+        kept_host.copy_(kept_off, non_blocking=True)
+        outs = {}
+        for k, t in zip(names, rows_out[1:]):
+            outs[k] = self._pinned_like(t)
+            outs[k].copy_(t, non_blocking=True)
+        keep_host = None
+        if len(names) < 3:  # some array could not travel as raw rows: filter it on the host like the reference
+            keep_host = self._pinned_like(any_vis)
+            keep_host.copy_(any_vis, non_blocking=True)
+        torch.cuda.current_stream().synchronize()
+        n_kept = int(kept_host[-1])
+        vis = masks_out[0][: n_views * n_kept].view(n_views, n_kept)
+        simw = masks_out[1][: n_views * n_kept].view(torch.float32).view(n_views, n_kept) if weight is not None else None
+        final = []
+        for name, arr in host_rows.items():
+            if name in outs:
+                final.append(outs[name].numpy()[:n_kept].view(arr.dtype).reshape((n_kept,) + tuple(np.shape(arr)[1:])))
+            else:
+                final.append(arr[keep_host.numpy().astype(bool)])
+        return (rows_out[0][:n_kept], vis, simw), tuple(final)
 
     def fuse_points(self, points, colors, labels, depths, seg_masks, camera_poses, mv_features, query_embeddings, device=None):
         device = device or self.device
         eng = self._eng(device)
-        # the division by sum_v visibility / sum_v similarity (:266-268) is fused into the fusion kernel
-        out = self._aggregate(eng, points, depths, seg_masks, camera_poses, mv_features, query_embeddings, normalize=True)
-        b = out["batch"]
-        n_views = len(depths)
-        rows = [out["sum"]]
-        new_index, kept_off, kept_host, out_off_host, cmask, rows_out = eng.compact(b, out["any"], out["mask"], rows)
-        n_kept = int(kept_host[-1])
-        keep = out["any"].cpu().numpy().astype(bool)
-        points, colors, labels = points[keep], colors[keep], labels[keep]
-        vis = cmask.view(n_views, n_kept).to(torch.int64)
-        simw = None
-        if self.use_similarity:
-            _, _, _, _, cw, _ = eng.compact(b, out["any"], out["weight"].view(torch.int32))
-            simw = cw.view(torch.float32).view(n_views, n_kept)
-        return (rows_out[0], vis, simw), (points, colors, labels)
+        b = self._stage_pix(eng, self._staging, points, colors, labels, depths, seg_masks, camera_poses, mv_features,
+                            query_embeddings)
+        return self._finish_pix(eng, b, points, colors, labels)
 
     # ------------------------------------------------------------------ a4 (object level)
     def _stage_obj(self, eng, staging, points, labels, depths, seg_masks, camera_poses, mv_features, query_embeddings,
@@ -194,21 +228,25 @@ class MultiviewFeatureFusion:
         segs = [s.cpu().numpy() if isinstance(s, torch.Tensor) else s for s in seg_masks]
         b = SceneBatch.from_host([self._scene(points, depths, camera_poses, labels, segs, feats, query_embeddings)],
                                  eng.device, staging=staging)
-        # rows that are only filtered and handed back (points[keep], colors[keep], labels[keep]) travel as raw
-        # bytes so that the filtering can run on the device
+        self._stage_rows(b, staging, points, colors, labels)
+        return b
+
+    @staticmethod
+    def _stage_rows(b, staging, points, colors, labels):
+        """Rows that are only filtered and handed back (points[keep], colors[keep], labels[keep]) travel as raw bytes, so
+        that the filtering can run on the device: b.row_sources maps each array that can to its (N, row) device tensor."""
         n_pts = b.total_points
         b.row_sources = {}
         for name, arr in (("points", points), ("colors", colors), ("labels", labels)):
             if name == "points" and isinstance(arr, np.ndarray) and arr.dtype == np.float64:
                 b.row_sources[name] = b.points
-            elif name == "labels" and isinstance(arr, np.ndarray) and arr.dtype == np.int64:
+            elif name == "labels" and b.labels is not None and isinstance(arr, np.ndarray) and arr.dtype == np.int64:
                 b.row_sources[name] = b.labels.view(-1, 1)
             elif isinstance(arr, np.ndarray) and arr.ndim >= 1 and arr.shape[0] == n_pts and n_pts > 0 and \
                     arr.dtype.kind in "fiub" and arr.size > 0:
                 # any fixed-width dtype travels as raw bytes (uint8 colours, int32 / uint8 labels, fp16 points ...)
                 b.row_sources[name] = staging.upload(np.ascontiguousarray(arr).reshape(n_pts, -1).view(np.uint8))
         staging.end()
-        return b
 
     @staticmethod
     def _pinned_like(t: torch.Tensor) -> torch.Tensor:
@@ -286,14 +324,14 @@ class MultiviewFeatureFusion:
 
     @torch.no_grad()
     def fuse_many(self, scenes, return_obj=True, device=None):
-        """Throughput form of `fuse` for the object-level path: `scenes` is an iterable of argument
-        tuples (points, colors, labels, depths, seg_masks, camera_poses, mv_features, query_embeddings);
-        yields exactly what `fuse(*args, return_obj=...)` returns, in order. The host->device staging of
-        scene i+1 runs on a side stream in a helper thread while scene i is fused and read back, so
-        the loop runs at the speed of the slower of the two (PCIe/host-copy bound at MV-TOD sizes).
-        This is what the reference's scene loop (tools/preprocess_data.py:188-297) becomes."""
-        if not self.use_obj_prior:
-            raise NotImplementedError("fuse_many covers the object-level path (use_obj_prior=1)")
+        """Throughput form of `fuse`: `scenes` is an iterable of argument tuples (points, colors, labels, depths,
+        seg_masks, camera_poses, mv_features, query_embeddings); yields exactly what `fuse(*args, device=device)`
+        returns, in order. The host->device staging of scene i+1 runs on a side stream in a helper thread while scene i
+        is fused and read back, so the loop runs at the speed of the slower of the two (PCIe/host-copy bound at MV-TOD
+        sizes). Both levels are covered. At object level `return_obj` is passed to each `fuse`; at pixel level
+        (use_obj_prior=0) it has no meaning, as `fuse_points` has no such argument, and is ignored. A scene that fails
+        raises when the loop reaches it, after every earlier scene was yielded, with the exception `fuse` raises for it.
+        This is what the reference's scene loops (tools/preprocess_data.py:188-297, scripts/run_eval.py:205-220) become."""
         from concurrent.futures import ThreadPoolExecutor
         device = device or self.device
         eng = self._eng(device)
@@ -308,15 +346,25 @@ class MultiviewFeatureFusion:
             self._many_stream = torch.cuda.Stream(device=dev)
         side = self._many_stream
 
-        def stage(k, args):
+        def stage(k, args, ready):
             torch.cuda.set_device(dev_index)
             points, colors, labels, depths, seg_masks, camera_poses, mv_features, query = args
             with torch.cuda.stream(side):
-                b = self._stage_obj(eng, stagings[k % 2], points, labels, depths, seg_masks, camera_poses, mv_features, query,
-                                    colors)
+                side.wait_event(ready)  # device inputs the caller produced before handing the scene over
+                if self.use_obj_prior:
+                    b = self._stage_obj(eng, stagings[k % 2], points, labels, depths, seg_masks, camera_poses, mv_features,
+                                        query, colors)
+                else:
+                    b = self._stage_pix(eng, stagings[k % 2], points, colors, labels, depths, seg_masks, camera_poses,
+                                        mv_features, query)
                 ev = torch.cuda.Event()
                 ev.record(side)
             return b, ev
+
+        def submit(k, args):
+            ready = torch.cuda.Event()
+            ready.record()
+            return pool.submit(stage, k, args, ready)
 
         it = iter(scenes)
         with ThreadPoolExecutor(max_workers=1) as pool:
@@ -325,17 +373,21 @@ class MultiviewFeatureFusion:
                 cur_args = next(it)
             except StopIteration:
                 return
-            fut = pool.submit(stage, k, cur_args)
+            fut = submit(k, cur_args)
             while True:
                 b, ev = fut.result()
                 try:
                     nxt_args = next(it)
-                    fut = pool.submit(stage, k + 1, nxt_args)
+                    fut = submit(k + 1, nxt_args)
                 except StopIteration:
                     nxt_args, fut = None, None
                 torch.cuda.current_stream().wait_event(ev)
                 points, colors, labels, depths, seg_masks, camera_poses, mv_features, query = cur_args
-                yield self._finish_obj(eng, stagings[k % 2], b, points, colors, labels, depths, mv_features, query, return_obj)
+                if self.use_obj_prior:
+                    yield self._finish_obj(eng, stagings[k % 2], b, points, colors, labels, depths, mv_features, query,
+                                           return_obj)
+                else:
+                    yield self._finish_pix(eng, b, points, colors, labels)
                 if fut is None:
                     return
                 cur_args, k = nxt_args, k + 1
