@@ -86,7 +86,11 @@ SIGNATURES = {
     "dc_sort_workspace": (c_size_t, [c_int64]),
     "dc_unique_max_pool": (c_int, [P, P, c_int, c_int, c_int64, P, P, P, P, c_size_t, P]),
     "dc_voxel_down_mean": (c_int, [P, c_int64, c_double, P, P, P, P, c_size_t, P]),
+    "dc_voxel_down_trace_workspace": (c_size_t, [c_int64]),
     "dc_voxel_down_trace": (c_int, [P, P, P, c_int64, c_double, P, P, P, P, P, P, P, c_size_t, P]),
+    "dc_aggregate_views_workspace": (c_size_t, [c_int, c_int, c_int64, c_int]),
+    "dc_aggregate_views": (c_int, [P, P, c_int, P, c_int, P, P, P, P, P, c_float, P, c_int, c_int, c_int, P, P, P, P, P, P, P, P, P,
+                                   P, c_size_t, P]),
     "dc_nearest_index": (c_int, [P, c_int64, P, c_int64, P, P, P]),
     "dc_binary_iou_counts": (c_int, [P, P, c_int, P, c_int, c_int64, c_float, c_int, c_int, P, P, P]),
     "dc_class_iou_workspace": (c_size_t, [c_int]),
@@ -96,6 +100,7 @@ SIGNATURES = {
                                  P, P, P, P, P]),
     "dc_host_gather_copy": (c_int, [P, c_int64, c_int64, P, c_int]),
     "dc_host_gather_narrow_i64_u8": (c_int, [P, c_int64, c_int64, P, c_int, POINTER(c_int)]),
+    "dc_host_masks_to_seg": (c_int, [P, P, P, c_int, P, P, c_int, P, c_int, POINTER(c_int)]),
 }
 
 _lib = None

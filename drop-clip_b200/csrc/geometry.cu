@@ -6,7 +6,7 @@
 // _cvt_regrad_coord :89-92 / _cvt_blender_coord :95-97, transform_pointcloud_to_world_frame
 // utils/transforms.py:43-49 (np.dot(pose, [p;1]) -> k-ascending FMA chain, pose promoted from
 // fp32), pointcloud_to_pixel utils/projections.py:59-64.
-#include "common.cuh"
+#include "geometry_math.cuh"
 
 namespace {
 
@@ -20,35 +20,11 @@ __global__ void __launch_bounds__(256) backproject_kernel(const float* __restric
     const int v = (int)(t / hw);
     const int64_t pix = t - (int64_t)v * hw;
     const int y = (int)(pix / width), x = (int)(pix - (int64_t)y * width);
-    const double z = (double)depths[t];
-    // ((u - cx) / fx) * z : subtraction, division, multiplication are separate roundings in numpy
-    double px, py;
-    if (flip_y & 2) {  // Open3D create_from_rgbd_image: (u - cx) * z / fx
-      px = __ddiv_rn(__dmul_rn(__dsub_rn((double)x, cx), z), fx);
-      py = __ddiv_rn(__dmul_rn(__dsub_rn((double)y, cy), z), fy);
-    } else {           // utils/projections.py:75-81: ((u - cx) / fx) * z
-      px = __dmul_rn(__ddiv_rn(__dsub_rn((double)x, cx), fx), z);
-      py = __dmul_rn(__ddiv_rn(__dsub_rn((double)y, cy), fy), z);
-    }
-    double pz = z;
-    if (flip_y & 1) py = -py;
-    if (flip_z) pz = -pz;
-    if (poses) {
-      const double* m = poses + (int64_t)v * 16;  // fp64 on the device; an fp32 pose upcasts exactly like np.dot does
-      double w[3];
-#pragma unroll
-      for (int r = 0; r < 3; ++r) {
-        double acc = __dmul_rn(m[4 * r], px);
-        acc = __fma_rn(m[4 * r + 1], py, acc);
-        acc = __fma_rn(m[4 * r + 2], pz, acc);
-        acc = __dadd_rn(m[4 * r + 3], acc);
-        w[r] = acc;
-      }
-      px = w[0]; py = w[1]; pz = w[2];
-    }
-    out[3 * t] = px;
-    out[3 * t + 1] = py;
-    out[3 * t + 2] = pz;
+    double w[3];
+    dc::backproject_pixel(x, y, (double)depths[t], fx, fy, cx, cy, flip_y, flip_z, poses ? poses + (int64_t)v * 16 : nullptr, w);
+    out[3 * t] = w[0];
+    out[3 * t + 1] = w[1];
+    out[3 * t + 2] = w[2];
   }
 }
 

@@ -14,6 +14,7 @@
 // of the fusion arithmetic is evaluated here.
 #include <emmintrin.h>  // SSE2 streaming stores (baseline x86-64)
 #include <stdint.h>
+#include <stdlib.h>
 #include <string.h>
 
 #include <unistd.h>
@@ -185,6 +186,54 @@ int dc_host_gather_narrow_i64_u8(const int64_t* const* srcs, int64_t n_items, in
     if (acc & ~(uint64_t)0xff) seen.fetch_or(acc, std::memory_order_relaxed);
   });
   *out_of_range = (seen.load() & ~(uint64_t)0xff) ? 1 : 0;
+  return DC_OK;
+}
+
+int dc_host_masks_to_seg(const uint8_t* const* masks, const int64_t* ids, const int64_t* mask_off, int n_views,
+                         const int64_t* view_pixels, const int64_t* pix_off, int out_dtype, void* dst, int n_threads,
+                         int* out_of_range) {
+  DC_CHECK_ARG(masks && ids && mask_off && view_pixels && pix_off && dst && out_of_range && n_views >= 0,
+               "dc_host_masks_to_seg: bad argument");
+  DC_CHECK_ARG(out_dtype == DC_U8 || out_dtype == DC_I64, "dc_host_masks_to_seg: out_dtype must be DC_U8 or DC_I64");
+  for (int v = 0; v < n_views; ++v)
+    DC_CHECK_ARG(mask_off[v + 1] > mask_off[v] && view_pixels[v] >= 0, "dc_host_masks_to_seg: view %d has no mask", v);
+  // work items: slices of a view's pixels, small enough that the running maxima stay in L1 across the K masks
+  const int64_t slice = 4096;
+  int64_t n_items = 0;
+  for (int v = 0; v < n_views; ++v) n_items += (view_pixels[v] + slice - 1) / slice;
+  std::atomic<int> bad(0);
+  int64_t* item_view = static_cast<int64_t*>(malloc(sizeof(int64_t) * (size_t)(n_views + 1)));  // first item of each view
+  if (!item_view) return ::dc::fail(DC_ERR_INVALID, "dc_host_masks_to_seg: out of host memory");
+  item_view[0] = 0;
+  for (int v = 0; v < n_views; ++v) item_view[v + 1] = item_view[v] + (view_pixels[v] + slice - 1) / slice;
+  parallel_items(n_items, n_threads, [&](int64_t t) {
+    const int v = (int)(std::upper_bound(item_view, item_view + n_views + 1, t) - item_view) - 1;
+    const int64_t s = (t - item_view[v]) * slice;
+    const int64_t len = std::min(slice, view_pixels[v] - s);
+    int64_t acc[slice];
+    for (int64_t k = mask_off[v]; k < mask_off[v + 1]; ++k) {
+      const uint8_t* __restrict__ m = masks[k] + s;
+      const uint64_t id = (uint64_t)ids[k];
+      if (k == mask_off[v]) {
+        for (int64_t j = 0; j < len; ++j) acc[j] = (int64_t)(m[j] * id);  // numpy's int64 product wraps
+      } else {
+        for (int64_t j = 0; j < len; ++j) acc[j] = std::max(acc[j], (int64_t)(m[j] * id));
+      }
+    }
+    if (out_dtype == DC_U8) {
+      uint8_t* __restrict__ o = static_cast<uint8_t*>(dst) + pix_off[v] + s;
+      uint64_t seen = 0;
+      for (int64_t j = 0; j < len; ++j) {
+        seen |= (uint64_t)acc[j];
+        o[j] = (uint8_t)acc[j];
+      }
+      if (seen & ~(uint64_t)0xff) bad.store(1, std::memory_order_relaxed);
+    } else {
+      memcpy(static_cast<int64_t*>(dst) + pix_off[v] + s, acc, sizeof(int64_t) * (size_t)len);
+    }
+  });
+  free(item_view);
+  *out_of_range = bad.load();
   return DC_OK;
 }
 

@@ -2,13 +2,14 @@
 //   * lexicographic sort of (N,3) fp64 rows + unique + segmented max  -> pool_multiview_features
 //     (utils/projections.py:245-261: np.unique(axis=0) + np.maximum.reduceat)
 //   * voxel-grid down-sampling with per-voxel mean in point order     -> pc_voxel_down
-//     (utils/geometry.py:350-352 -> Open3D voxel_down_sample, parity unpinned: Open3D absent)
+//     (utils/geometry.py:350-352 -> Open3D voxel_down_sample, parity unpinned: Open3D absent);
+//     the traced variant with the label vote lives in aggregate.cu
 //   * exact nearest neighbour (fp64, brute force, tiled through smem) -> find_closest_indices
 //     (utils/geometry.py:390-401 -> scipy cKDTree.query, k = 1)
 // The sort is a bitonic network over an index array (power-of-two padded with sentinels); steps
 // whose partner distance fits a CTA run in shared memory, the rest in global memory. Keys are
 // fetched through the index (gather) so that any key type can be sorted by the same kernels.
-#include "common.cuh"
+#include "geometry_math.cuh"
 
 namespace {
 
@@ -218,30 +219,21 @@ __global__ void __launch_bounds__(256) min_bound_kernel(const double* __restrict
   }
   if ((threadIdx.x & 31) == 0) {
     const double v[3] = {lx, ly, lz};
-    for (int a = 0; a < 3; ++a) {
-      unsigned long long b = (unsigned long long)__double_as_longlong(v[a]);
-      b = (b & 0x8000000000000000ull) ? ~b : (b | 0x8000000000000000ull);
-      atomicMin(mn + a, b);
-    }
+    for (int a = 0; a < 3; ++a) atomicMin(mn + a, dc::double_to_ordered(v[a]));
   }
-}
-
-__device__ __forceinline__ double ordered_to_double(unsigned long long b) {
-  b = (b & 0x8000000000000000ull) ? (b & 0x7fffffffffffffffull) : ~b;
-  return __longlong_as_double((long long)b);
 }
 
 __global__ void __launch_bounds__(256) voxel_keys_kernel(const double* __restrict__ pts, int64_t n, double voxel,
                                                          const unsigned long long* __restrict__ mn, unsigned long long* __restrict__ keys,
                                                          int* __restrict__ error) {
-  const double bx = ordered_to_double(mn[0]) - voxel * 0.5, by = ordered_to_double(mn[1]) - voxel * 0.5,
-               bz = ordered_to_double(mn[2]) - voxel * 0.5;
+  const double bx = dc::ordered_to_double(mn[0]) - voxel * 0.5, by = dc::ordered_to_double(mn[1]) - voxel * 0.5,
+               bz = dc::ordered_to_double(mn[2]) - voxel * 0.5;
   for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (int64_t)gridDim.x * blockDim.x) {
     // Open3D: ref_coord = (point - voxel_min_bound) / voxel_size; voxel_index = floor(ref_coord)
-    const double fx = floor(__ddiv_rn(__dsub_rn(pts[3 * i], bx), voxel));
-    const double fy = floor(__ddiv_rn(__dsub_rn(pts[3 * i + 1], by), voxel));
-    const double fz = floor(__ddiv_rn(__dsub_rn(pts[3 * i + 2], bz), voxel));
-    if (!(fx >= 0 && fx < 2097152.0 && fy >= 0 && fy < 2097152.0 && fz >= 0 && fz < 2097152.0)) {
+    const double fx = dc::voxel_coord(pts[3 * i], bx, voxel);
+    const double fy = dc::voxel_coord(pts[3 * i + 1], by, voxel);
+    const double fz = dc::voxel_coord(pts[3 * i + 2], bz, voxel);
+    if (!(dc::voxel_coord_ok(fx) && dc::voxel_coord_ok(fy) && dc::voxel_coord_ok(fz))) {
       atomicExch(error, 1);
       keys[i] = 0;
       continue;
@@ -272,81 +264,6 @@ __global__ void __launch_bounds__(256) voxel_mean_kernel(const double* __restric
     out[3 * u + 1] = sy / (double)c;
     out[3 * u + 2] = sz / (double)c;
     first_index[u] = order[i];
-  }
-}
-
-// voxel_down_sample_and_trace + the majority vote of aggregate_views_blender_new (utils/geometry.py:186-201):
-// per voxel the mean position and colour (members summed in ascending point index, like Open3D's
-// AccumulatedPointForTrace) and `Counter(labels).most_common()[0][0]`: the most frequent label, ties
-// going to the label met first in point order. One thread per voxel; up to kSlots distinct labels are
-// counted in registers in one pass, voxels with more fall back to a quadratic scan.
-__global__ void __launch_bounds__(256) voxel_trace_kernel(const double* __restrict__ pts, const double* __restrict__ cols,
-                                                          const long long* __restrict__ labels, const int* __restrict__ order,
-                                                          const uint8_t* __restrict__ head, const int64_t* __restrict__ seg,
-                                                          int64_t n, double* __restrict__ out_pts, double* __restrict__ out_cols,
-                                                          long long* __restrict__ out_labels, int64_t* __restrict__ first_index,
-                                                          int64_t* __restrict__ counts) {
-  constexpr int kSlots = 8;
-  for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (int64_t)gridDim.x * blockDim.x) {
-    if (!head[i]) continue;
-    double sx = 0, sy = 0, sz = 0, cr = 0, cg = 0, cb = 0;
-    long long lab[kSlots];
-    int cnt[kSlots];
-    int used = 0;
-    bool overflow = false;
-    int64_t c = 0, k = i;
-    do {
-      const int64_t j = order[k];
-      sx += pts[3 * j];
-      sy += pts[3 * j + 1];
-      sz += pts[3 * j + 2];
-      if (cols) {
-        cr += cols[3 * j];
-        cg += cols[3 * j + 1];
-        cb += cols[3 * j + 2];
-      }
-      if (labels && !overflow) {
-        const long long l = labels[j];
-        int s = 0;
-        while (s < used && lab[s] != l) ++s;
-        if (s < used) ++cnt[s];
-        else if (used < kSlots) { lab[used] = l; cnt[used] = 1; ++used; }
-        else overflow = true;
-      }
-      ++c;
-      ++k;
-    } while (k < n && !head[k]);
-    const int64_t u = seg[i];
-    const double dc_ = (double)c;
-    out_pts[3 * u] = sx / dc_;
-    out_pts[3 * u + 1] = sy / dc_;
-    out_pts[3 * u + 2] = sz / dc_;
-    if (cols) {
-      out_cols[3 * u] = cr / dc_;
-      out_cols[3 * u + 1] = cg / dc_;
-      out_cols[3 * u + 2] = cb / dc_;
-    }
-    if (first_index) first_index[u] = order[i];
-    if (counts) counts[u] = c;
-    if (labels) {
-      long long best = 0;
-      int64_t best_n = -1;
-      if (!overflow) {
-        for (int s = 0; s < used; ++s)  // slots are in first-seen order: strict > keeps the earliest on ties
-          if (cnt[s] > best_n) { best_n = cnt[s]; best = lab[s]; }
-      } else {
-        for (int64_t a = i; a < i + c; ++a) {
-          const long long l = labels[order[a]];
-          bool seen = false;
-          for (int64_t b = i; b < a && !seen; ++b) seen = labels[order[b]] == l;
-          if (seen) continue;
-          int64_t m = 0;
-          for (int64_t b = a; b < i + c; ++b) m += labels[order[b]] == l;
-          if (m > best_n) { best_n = m; best = l; }
-        }
-      }
-      out_labels[u] = best;
-    }
   }
 }
 
@@ -468,35 +385,6 @@ int dc_voxel_down_mean(const double* points, int64_t n, double voxel_size, doubl
   key_heads_kernel<<<grid_for(n), 256, 0, st>>>(w.keys, w.order, n, w.head);
   scan_heads_kernel<<<1, 1024, 0, st>>>(w.head, n, w.seg, n_voxels);
   voxel_mean_kernel<<<grid_for(n), 256, 0, st>>>(points, w.order, w.head, w.seg, n, out_points, first_index);
-  DC_LAUNCH_CHECK();
-  return DC_OK;
-}
-
-int dc_voxel_down_trace(const double* points, const double* colors, const int64_t* labels, int64_t n, double voxel_size,
-                        double* out_points, double* out_colors, int64_t* out_labels, int64_t* first_index, int64_t* counts,
-                        int64_t* n_voxels, void* workspace, size_t workspace_bytes, dc_stream_t stream) {
-  DC_CHECK_ARG(points && out_points && n_voxels && workspace, "dc_voxel_down_trace: null pointer argument");
-  DC_CHECK_ARG((!colors || out_colors) && (!labels || out_labels), "dc_voxel_down_trace: output missing for an optional input");
-  DC_CHECK_ARG(voxel_size > 0.0, "dc_voxel_down_trace: voxel_size must be positive");
-  DC_CHECK_ARG(n < (1ll << 30), "dc_voxel_down_trace: too many points");
-  SortWs w = carve(workspace, n);
-  if (workspace_bytes < w.total) return dc::fail(DC_ERR_WORKSPACE, "dc_voxel_down_trace: workspace %zu < %zu", workspace_bytes, w.total);
-  cudaStream_t st = dc::as_stream(stream);
-  if (n <= 0) {
-    DC_CUDA(cudaMemsetAsync(n_voxels, 0, sizeof(int64_t), st));
-    return DC_OK;
-  }
-  DC_CUDA(cudaMemsetAsync(w.mn, 0xFF, 24, st));
-  DC_CUDA(cudaMemsetAsync(w.error, 0, 4, st));
-  min_bound_kernel<<<grid_for(n), 256, 0, st>>>(points, n, w.mn);
-  voxel_keys_kernel<<<grid_for(n), 256, 0, st>>>(points, n, voxel_size, w.mn, w.keys, w.error);
-  int rc = bitonic_sort(w.order, n, LessKey64{w.keys}, st);
-  if (rc) return rc;
-  key_heads_kernel<<<grid_for(n), 256, 0, st>>>(w.keys, w.order, n, w.head);
-  scan_heads_kernel<<<1, 1024, 0, st>>>(w.head, n, w.seg, n_voxels);
-  voxel_trace_kernel<<<grid_for(n), 256, 0, st>>>(points, colors, reinterpret_cast<const long long*>(labels), w.order, w.head,
-                                                 w.seg, n, out_points, out_colors, reinterpret_cast<long long*>(out_labels),
-                                                 first_index, counts);
   DC_LAUNCH_CHECK();
   return DC_OK;
 }

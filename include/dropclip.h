@@ -490,7 +490,7 @@ DC_API int dc_transform_points(const double* points, int64_t n, const double* ma
 
 /* ------------------------------------------------------------------------------------------
  * Sort-based helpers of the REGRAD-style functions in utils/projections.py.
- * workspace for the three calls below: dc_sort_workspace(n) bytes.
+ * workspace for the two calls below: dc_sort_workspace(n) bytes.
  */
 DC_API size_t dc_sort_workspace(int64_t n);
 /* pool_multiview_features utils/projections.py:245-261: np.unique(points, axis=0) (lexicographic
@@ -508,11 +508,36 @@ DC_API int dc_voxel_down_mean(const double* points, int64_t n, double voxel_size
 /* voxel_down_sample_and_trace + label majority vote of aggregate_views_blender_new utils/geometry.py:186-201
  * (Open3D semantics, parity unpinned): per voxel the mean position, the mean colour (optional) and the most
  * frequent label (optional; ties: the label met first in point order, like Counter.most_common()[0][0]);
- * counts[u] = members of voxel u. Voxels ordered by voxel index. workspace: dc_sort_workspace(n). */
+ * counts[u] = members of voxel u, first_index[u] its smallest point index (both optional). Voxels ordered by
+ * voxel index. The one-scene, one-size case of dc_aggregate_views' trace. workspace:
+ * dc_voxel_down_trace_workspace(n) bytes. */
+DC_API size_t dc_voxel_down_trace_workspace(int64_t n);
 DC_API int dc_voxel_down_trace(const double* points, const double* colors, const int64_t* labels, int64_t n,
                         double voxel_size, double* out_points, double* out_colors, int64_t* out_labels,
                         int64_t* first_index, int64_t* counts, int64_t* n_voxels, void* workspace,
                         size_t workspace_bytes, dc_stream_t stream);
+/* aggregate_views_blender_new utils/geometry.py:120-204 for S scenes at U voxel sizes in one call.
+ * Inputs (device): the views' depth maps (fp32), instance maps (DC_U8 / DC_I64) and RGB images (3 channels,
+ * DC_U8 / DC_F64), concatenated view after view (scene after scene); view v covers pixels
+ * [view_pix_off[v], view_pix_off[v + 1]) as a row-major view_hw[2v] x view_hw[2v + 1] image.
+ * Host tables: view_pix_off[V + 1], view_hw[2V], scene_view_off[S + 1], poses[16V] (fp64 world matrices,
+ * row-major 4x4), fxfycxcy[4], voxel_sizes[U] (each > 0; depth_trunc must not be NaN when U > 0).
+ * Per scene, a pixel is labelled when depth < depth_trunc and kept as a point when 0 < depth < depth_trunc:
+ * points / colors / labels receive scene s's rows at [point_off[s], point_off[s + 1]) / [label_off[s], ...)
+ * (device int64 [S + 1]); a point is the Open3D back-projection flipped by (1, -1, -1) and moved by the view's
+ * world matrix, a colour is rgb / 255.0. Point j of a scene votes with label j of that scene.
+ * Voxel outputs: segment (u, s) = scene s at voxel_sizes[u] is rows [vox_off[u S + s], vox_off[u S + s + 1])
+ * of vox_points / vox_colors / vox_labels (device int64 vox_off[U S + 1]); see dc_voxel_down_trace.
+ * Capacities: n_pixels rows for points / colors / labels, U * n_pixels for the voxel outputs, where
+ * n_pixels = view_pix_off[V] and U * n_pixels < 2^31. workspace: dc_aggregate_views_workspace bytes. */
+DC_API size_t dc_aggregate_views_workspace(int n_scenes, int n_views, int64_t n_pixels, int n_sizes);
+DC_API int dc_aggregate_views(const float* depths, const void* segs, int seg_dtype, const void* rgbs, int rgb_dtype,
+                              const int64_t* view_pix_off, const int32_t* view_hw, const int32_t* scene_view_off,
+                              const double* poses, const double* fxfycxcy, float depth_trunc, const double* voxel_sizes,
+                              int n_scenes, int n_views, int n_sizes, double* points, double* colors, int64_t* labels,
+                              int64_t* point_off, int64_t* label_off, double* vox_points, double* vox_colors,
+                              int64_t* vox_labels, int64_t* vox_off, void* workspace, size_t workspace_bytes,
+                              dc_stream_t stream);
 /* find_closest_indices utils/geometry.py:390-401 (cKDTree.query k=1): exact fp64 nearest neighbour
  * of every query point in `ref` (ties: smallest index); out_dist2 (squared distance) may be NULL. */
 DC_API int dc_nearest_index(const double* query, int64_t m, const double* ref, int64_t n, int64_t* out_index,
@@ -564,6 +589,15 @@ DC_API int dc_sample_gather(const double* xyz, const double* rgb, const int64_t*
 DC_API int dc_host_gather_copy(const void* const* srcs, int64_t n_items, int64_t item_bytes, void* dst, int n_threads);
 DC_API int dc_host_gather_narrow_i64_u8(const int64_t* const* srcs, int64_t n_items, int64_t item_elems, uint8_t* dst,
                                         int n_threads, int* out_of_range);
+/* dc_host_masks_to_seg: binary_masks_to_seg utils/image.py:11-15 for n_views views in one pass over the masks:
+ * view v has masks masks[mask_off[v] .. mask_off[v + 1]) (bool or uint8, view_pixels[v] bytes each, at least one)
+ * with instance ids ids[mask_off[v] ..]; its map, value = max over k of (int64) mask_k * id_k as numpy computes
+ * it (a pixel covered by every mask takes the largest product, without the 0), is written at dst + pix_off[v]
+ * elements. out_dtype DC_U8 or DC_I64; with DC_U8, *out_of_range = 1 when a value lies outside [0, 255] (the
+ * maps are then incomplete; the caller builds them again as DC_I64). */
+DC_API int dc_host_masks_to_seg(const uint8_t* const* masks, const int64_t* ids, const int64_t* mask_off, int n_views,
+                                const int64_t* view_pixels, const int64_t* pix_off, int out_dtype, void* dst,
+                                int n_threads, int* out_of_range);
 
 #ifdef __cplusplus
 }
